@@ -47,7 +47,9 @@ N_CLASSES = 66
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline and e2e regions (the fp32-mode and ViT-B/16 sections time "
+                         "max(3, min(steps, 10)) steps and report that count as their 'steps')")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=32)
@@ -70,7 +72,13 @@ def parse():
     ap.add_argument("--no-vit", action="store_true")
     ap.add_argument("--sweep-only", action="store_true", help="debug: measure only the sweep section")
     ap.add_argument("--vit-batch", type=int, default=256)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last of them computed (loss, trainable parameters "
+                         "after the optimiser step, their gradients) to DIR/<name>.npy in float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, n):
@@ -162,13 +170,16 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     n_img = args.cpu_sample_images or args.batch
-    step = cpu_step_fn(build_cpu_reference(args.backbone), n_img)
+    model = build_cpu_reference(args.backbone)
+    step = cpu_step_fn(model, n_img)
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        loss = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, model)
     value = n_img * args.steps / dt
     sample = (f"{n_img} images per step = the stated batch (fwd + bwd + AdamW, text tower recomputed each "
               f"step), {args.steps} steps, PyTorch fp32, {torch.get_num_threads()} threads; oracle port "
@@ -252,6 +263,23 @@ def build_gpu_model(args, device):
     model.train()
     opt = core.make_optimizer(model, 3e-4)
     return model, opt
+
+
+def dump_outputs(out_dir, loss, model):
+    """What a caller of the timed step holds after its last call: the loss, the trainable (DoRA) parameters after
+    the optimiser step and the gradients that step applied.  Inputs and initial weights are seeded, so two builds
+    run with the same arguments can be compared file by file (DoRA r32 on 2 + 1 blocks of ViT-L/14: 1.5 MB)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": torch.as_tensor(loss)}
+    for name, p in model.named_parameters():
+        if p.requires_grad:
+            arrays[f"param.{name}"] = p
+            if p.grad is not None:
+                arrays[f"grad.{name}"] = p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 EPOCHS_PER_CONDITION = 55  # reference sweep mean: 64.0 h * 3600 / 97 conditions / 43.5 s per epoch
@@ -592,6 +620,8 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     ms, launches, _ = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, train_step.last_loss, model)
     # roofline of the dominant kernel: CUDA events around every GEMM launch, which needs the launches to
     # come from the host - the same K steps once more with graph replay switched off (identical kernels)
     # (and with the text tower on the main stream: overlapped kernels would stretch each other's events)

@@ -37,6 +37,10 @@ import os
 import sys
 import tempfile
 
+# both arms run on the CPU whatever the host has: a visible GPU would add CUDA RNG states to the random-state
+# checkpoints, whose keys are compared with tests/golden/clip_pipeline_exec.json
+os.environ["CUDA_VISIBLE_DEVICES"] = ""
+
 import numpy as np
 import torch
 

@@ -12,6 +12,7 @@ import pytest
 
 from hba import analysis, sweep
 from oracle import analysis_ref as ref
+from oracle import ref_loader
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "analysis.json")))
@@ -207,10 +208,30 @@ def test_vit_summary_table_reproduces_the_shipped_csv(tmp_path):
     assert set(analysis.VIT_SUMMARY_COLUMNS) <= set(vit_train.RESULT_COLUMNS)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Data/clip_results"), reason="reference not mounted")
+def _excerpt_tree(root):
+    """The golden excerpt laid out like the reference's Data/ tree: the baseline CSV, the FIG2 runs as
+    clip_results/<type dir>/training_res_run{e}.csv, and Data/vit_results' two CSVs."""
+    clip = root / "clip_results"
+    clip.mkdir(parents=True)
+    frame(GOLD["baseline_raw"]).to_csv(clip / "baseline_clip_results_seed1.csv", index=False)
+    for name, runs in GOLD["fig2_runs"].items():
+        d = clip / analysis.FIG2_TYPE_DIRS[name]
+        d.mkdir()
+        for e, rows in runs.items():
+            frame(rows).to_csv(d / f"training_res_run{e}.csv", index=False)
+    vit = root / "vit_results"
+    vit.mkdir()
+    pd.DataFrame(GOLD["vit_effects_rows"]).to_csv(vit / "perturbation_effects.csv", index=False)
+    (vit / "perturbation_summary_table.csv").write_text(GOLD["vit_summary_csv"])
+    return str(root)
+
+
 def test_fig2_tables_from_the_reference_tree_directly(tmp_path):
-    """The directory-level entry points on the reference's own Data/ tree (only where it is mounted)."""
-    data = "/root/reference/Data"
+    """The directory-level entry points on the reference's own Data/ tree where it is present, else on the golden
+    excerpt of it laid out the same way; the expected values are the reference's either way."""
+    data = os.path.join(ref_loader.REFERENCE_ROOT, "Data")
+    if not os.path.isdir(os.path.join(data, "clip_results")):
+        data = _excerpt_tree(tmp_path / "Data")
     t = analysis.perturbation_type_summary(os.path.join(data, "clip_results", "baseline_clip_results_seed1.csv"),
                                            os.path.join(data, "clip_results"))
     for name, want in GOLD["fig2_expected"].items():

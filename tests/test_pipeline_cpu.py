@@ -117,7 +117,10 @@ def test_random_state_checkpoint_roundtrip(tmp_path):
 
 def test_select_device_has_no_cpu_path():
     import pytest
-    assert core.select_device(0) == torch.device("cuda:0") and core.select_device(-1) == torch.device("cuda")
+    assert core.select_device(0) == torch.device("cuda:0")
+    # -1 is the current CUDA device; without a visible device its index is left open
+    dev = core.select_device(-1)
+    assert dev.type == "cuda" and dev.index == (torch.cuda.current_device() if torch.cuda.is_available() else None)
     with pytest.raises(RuntimeError, match="no CPU path"):
         core.select_device(2)
 

@@ -155,12 +155,33 @@ def test_baseline_row_lookup(tmp_path):
     assert vt.baseline_row(p, 6) is None
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Training/vit_training"), reason="reference not mounted")
 def test_restatement_equals_reference_classes():
-    """The product's and the oracle's wrapper classes against the reference's own (imported with timm stubbed)."""
+    """The product's and the oracle's wrapper classes against the outputs of the reference's own classes stored in
+    tests/golden/vit_measure.json, and against those classes themselves (imported with timm stubbed) where the
+    reference tree is present."""
     from oracle import make_vit_measure_golden as mk
     from oracle import vit_measure_ref as ref
     vt = _vt()
+    gold_base = [(i, l) for i, l in enumerate(GOLD["labels"])]
+    for seed in (42, 7):
+        for cls in (vt.ShuffledLabelsDataset, ref.ShuffledLabelsRef):
+            ds = cls(gold_base, seed)
+            assert [int(ds[i][1]) for i in range(len(ds))] == GOLD[f"label_shuffle_seed{seed}"], (cls, seed)
+        for cls in (vt.TargetNoiseDataset, ref.TargetNoiseRef):
+            ds = cls(gold_base, 10, seed)
+            assert [int(ds[i][1]) for i in range(len(ds))] == GOLD[f"target_noise_seed{seed}"], (cls, seed)
+    from hba import vit
+    for cls in (vit.CosineAnnealingLRWithWarmup, ref.CosineWarmupRef):
+        opt = types.SimpleNamespace(param_groups=[{"lr": 0.1}])
+        s = cls(opt, 5, 100, eta_min=0)
+        lrs = []
+        for _ in range(100):
+            s.step()
+            lrs.append(opt.param_groups[0]["lr"])
+        assert lrs == pytest.approx(GOLD["schedule_meas"], rel=1e-15, abs=1e-18), cls
+        assert s.state_dict() == GOLD["schedule_meas_state"], cls
+    if not os.path.isdir(os.path.join(mk.REF, "Training", "vit_training")):
+        return
     MEAS, VIT = mk.load_reference_scripts()
     base = [(torch.full((2,), float(i)), (3 * i + 1) % 13) for i in range(41)]
     for seed in (0, 42):
