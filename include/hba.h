@@ -268,6 +268,39 @@ int hba_pearson_f64(const double* a, const double* b, int64_t n, double* rho_out
  * embedding row gives rho = NaN.  Needs N(N-1)/2 > 2048; workspace: hba_rank_workspace_bytes(N(N-1)/2). */
 int hba_rdm_spearman(const float* E, int32_t N, int32_t Dm, const double* ref_ranks, double* rdm,
                      double* ranks, double* rho_out, void* workspace, int64_t workspace_bytes, void* stream);
+/* hba_rank_order_f64: as hba_rank_avg_f64 (same keys, passes and NaN ordering; ranks all NaN when any x is NaN)
+ *   and also order [n] uint32, the stable sorted order: x[order[0]] <= x[order[1]] <= ..., equal values in
+ *   index order, NaN at the ends.  Workspace: hba_rank_workspace_bytes(n). */
+int hba_rank_order_f64(const double* x, int64_t n, uint32_t* order, double* ranks, void* workspace,
+                       int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Stimulus-resampling statistics of RSA for N stimuli, P = N(N-1)/2 upper-triangle pairs (k=1, row-major).
+ * Sums are exact int64 sums of centred doubled ranks 2r - (M+1), so outputs are bit-identical run to run;
+ * exact while 2 P^3 / 3 < 2^63: 3 <= N <= 2191.  Outputs are NaN where scipy.stats.spearmanr returns NaN.
+ * hba_rsa_perm_null (Mantel permutation test): for p < n_perm and pi_p = perms[p, :] (int32, a permutation
+ *   of 0..N-1; an entry outside [0, N) gives NaN),
+ *     rho_out[p] = Pearson over i<j of (ref_ranks[i,j], model_ranks[pi_p(i), pi_p(j)])
+ *   = scipy.stats.spearmanr(ref_tri, model_rdm[pi_p][:, pi_p][triu]).  ref_ranks, model_ranks: [P] f64 average
+ *   ranks (hba_rank_avg_f64) of the two triangles.  Workspace: hba_rsa_perm_workspace_bytes(N, n_perm).
+ * hba_rsa_bootstrap (stimulus bootstrap, Nili et al. 2014): for b < n_boot and counts c = counts[b, :] (int32,
+ *   values in [0, N] summing to N; otherwise NaN), every pair {i,j}, i != j, enters with multiplicity c_i c_j
+ *   and pairs of a stimulus with itself are dropped:
+ *     rho_a[b] = spearmanr of (ref, model a) over that expanded multiset of pairs, with the average ranks of
+ *     scipy.stats.rankdata on the expanded multiset = the weighted Pearson of the weighted average ranks.
+ *   NaN when a pair of weight > 0 is NaN in either RDM or a side is constant (fewer than 3 distinct stimuli).
+ *   tri_*: [P] f64 upper triangles; order_*: their sorted order (hba_rank_order_f64).  Model b (tri_b, order_b,
+ *   rho_b: all given or all NULL) is evaluated on the same resamples, for a paired difference rho_a - rho_b.
+ *   Workspace: hba_rsa_boot_workspace_bytes(N, n_boot).
+ */
+int64_t hba_rsa_perm_workspace_bytes(int32_t N, int32_t n_perm);
+int hba_rsa_perm_null(const double* ref_ranks, const double* model_ranks, int32_t N, const int32_t* perms,
+                      int32_t n_perm, double* rho_out, void* workspace, int64_t workspace_bytes, void* stream);
+int64_t hba_rsa_boot_workspace_bytes(int32_t N, int32_t n_boot);
+int hba_rsa_bootstrap(const double* ref_tri, const uint32_t* ref_order, const double* tri_a,
+                      const uint32_t* order_a, const double* tri_b, const uint32_t* order_b, int32_t N,
+                      const int32_t* counts, int32_t n_boot, double* rho_a, double* rho_b, void* workspace,
+                      int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Softmax cross-entropy (nn.CrossEntropyLoss at VIT:291, applied VIT:139) forward + backward:

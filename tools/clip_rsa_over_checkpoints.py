@@ -9,6 +9,9 @@ checkpoint tree (a baseline run and / or the output tree of a sweep), checkpoint
 Reference RDM: `--rdm` (.npy or .mat with one square matrix), else 1 - corrcoef of the 66-D behavioural embedding in
 the two CSV files (rows in the order train csv, then inference csv) - what RDM48_triplet is for the 48-image subset.
 The last stdout line is a JSON record with checkpoints/s (wall clock, max over ranks, cache fill included).
+--permutations N adds the Mantel p-value column behavioral_rsa_p_perm, --bootstrap N the stimulus-bootstrap 95 %
+interval (behavioral_rsa_ci_low / _ci_high) and the number of valid replicates (behavioral_rsa_boot_valid); --seed
+seeds both, identically for every checkpoint.  Without them the CSV has the columns of hba.rsa_scale.RESULT_COLUMNS.
 """
 import argparse
 import json
@@ -34,6 +37,9 @@ def main(argv=None):
     ap.add_argument("--rank", type=int, default=32, dest="dora_rank")
     ap.add_argument("--batch-size", type=int, default=32)
     ap.add_argument("--limit", type=int, default=0)
+    ap.add_argument("--permutations", type=int, default=0, help="Mantel permutations per checkpoint (0: none)")
+    ap.add_argument("--bootstrap", type=int, default=0, help="stimulus-bootstrap replicates per checkpoint (0: none)")
+    ap.add_argument("--seed", type=int, default=0, help="seed of the permutations and resamples")
     a = ap.parse_args(argv)
     import numpy as np
     import pandas as pd
@@ -83,7 +89,8 @@ def main(argv=None):
         raise SystemExit(f"no epoch*_dora_params.pth under {a.checkpoints}")
     t_setup = time.perf_counter() - t_start
     res = rsa_scale.clip_rsa_over_checkpoints(model, loaders, ref, files, device, rank=rank, world_size=world,
-                                              output_csv=a.output_csv or None, log=None, root=a.checkpoints)
+                                              output_csv=a.output_csv or None, log=None, root=a.checkpoints,
+                                              n_perm=a.permutations, n_boot=a.bootstrap, seed=a.seed)
     torch.cuda.synchronize()
     wall = time.perf_counter() - t_start
     if world > 1:

@@ -15,25 +15,9 @@
 #include <math_constants.h>
 
 #include "common.cuh"
+#include "rsa_keys.cuh"
 
 namespace hba {
-
-// ------------------------------------------------------------------------------------------
-// double -> uint64 whose unsigned order equals the numeric order (-0.0 canonicalised to +0.0);
-// every NaN sorts above +inf
-// (integer arithmetic on the two 32-bit halves: nvcc turns `bits | sign` on a reinterpreted double into the
-// floating-point negation DADD -|x|, which returns the canonical NaN without the flipped sign bit)
-__device__ __forceinline__ unsigned long long f64_to_key(double x) {
-  x = x + 0.0;
-  const int hi = __double2hiint(x), lo = __double2loint(x);
-  const int neg = hi >> 31;   // all ones for a negative value
-  const unsigned int khi = (unsigned int)(hi ^ (neg | (int)0x80000000)), klo = (unsigned int)(lo ^ neg);
-  return ((unsigned long long)khi << 32) | klo;
-}
-constexpr unsigned long long kKeyPosInf = 0xFFF0000000000000ull;  // f64_to_key(+inf); NaN keys are larger
-// (a negative-signed NaN maps below -inf: keys < f64_to_key(-inf) = 0x000FFFFFFFFFFFFF)
-constexpr unsigned long long kKeyNegInf = 0x000FFFFFFFFFFFFFull;
-__device__ __forceinline__ bool key_is_nan(unsigned long long k) { return k > kKeyPosInf || k < kKeyNegInf; }
 
 // ------------------------------------------------------------------------------------------
 // RDM: 32x32 pair tiles; each CTA centres its 64 rows in float64 (numpy.cov promotes to f64
@@ -127,10 +111,13 @@ __global__ void __launch_bounds__(256)
 }
 
 // single CTA: bitonic sort of up to 2048 (key, index) pairs in shared memory, tie-run averaging.
-// Any NaN makes every rank NaN (scipy.stats.rankdata, nan_policy='propagate').
+// Any NaN makes every rank NaN (scipy.stats.rankdata, nan_policy='propagate').  kOrder: also writes the stable
+// sorted order (order[p] = index of the p-th smallest key, NaN keys at the ends), which needs the sort even with NaN.
 constexpr int kSmallN = 2048;
+template <bool kOrder>
 __global__ void __launch_bounds__(1024)
-    rank_small_kernel(const double* __restrict__ x, int n, double* __restrict__ ranks) {
+    rank_small_kernel(const double* __restrict__ x, int n, double* __restrict__ ranks,
+                      unsigned int* __restrict__ order) {
   __shared__ unsigned long long sk[kSmallN];
   __shared__ unsigned short si[kSmallN];
   int has_nan = 0;
@@ -141,7 +128,7 @@ __global__ void __launch_bounds__(1024)
     si[i] = (unsigned short)i;
   }
   has_nan = __syncthreads_or(has_nan);
-  if (has_nan) {
+  if (!kOrder && has_nan) {
     for (int i = threadIdx.x; i < n; i += 1024) ranks[i] = CUDART_NAN;
     return;
   }
@@ -164,6 +151,13 @@ __global__ void __launch_bounds__(1024)
     }
   }
   // positions [0, n) now hold the real elements (padding has the largest key or index)
+  if (kOrder) {
+    for (int p = threadIdx.x; p < n; p += 1024) order[p] = si[p];
+    if (has_nan) {
+      for (int i = threadIdx.x; i < n; i += 1024) ranks[i] = CUDART_NAN;
+      return;
+    }
+  }
   for (int p = threadIdx.x; p < n; p += 1024) {
     if (p == 0 || sk[p] != sk[p - 1]) {
       int e = p;
@@ -376,26 +370,6 @@ __global__ void __launch_bounds__(kRadixThreads, 4)
 }
 constexpr size_t kRadixPassSmem = (size_t)kRadixTile * 12 + (kRadixWarps * 256 + 256 + 256 + 16) * 4;
 
-// binary searches in the sorted key array: first index with key >= k / first index with key > k
-__device__ __forceinline__ int64_t lower_bound_key(const unsigned long long* __restrict__ a, int64_t lo,
-                                                   int64_t hi, unsigned long long k) {
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (a[mid] < k) lo = mid + 1;
-    else hi = mid;
-  }
-  return lo;
-}
-__device__ __forceinline__ int64_t upper_bound_key(const unsigned long long* __restrict__ a, int64_t lo,
-                                                   int64_t hi, unsigned long long k) {
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (a[mid] <= k) lo = mid + 1;
-    else hi = mid;
-  }
-  return lo;
-}
-
 // After the sort.  Position p of the sorted order holds (key, original index v); its rank is the mean of the
 // 1-based positions of its tie run (found by binary search, so that even an all-equal input costs O(log n) per
 // element).  ranks_out (optional): ranks[v] = rank.  ref (optional): Pearson sums of (rank, ref[v]) about the
@@ -461,6 +435,19 @@ __global__ void __launch_bounds__(256)
     r /= sqrt(t[2]);
     *rho = (r != r) ? r : fmin(fmax(r, -1.0), 1.0);
   }
+}
+
+// After the sort: the stable sorted order (original index of every sorted position) out of whichever value buffer
+// the executed passes left it in; identity when no digit pass ran (all keys equal).
+__global__ void __launch_bounds__(256)
+    sorted_order_kernel(const unsigned int* __restrict__ vbuf0, const unsigned int* __restrict__ vbuf1, int64_t n,
+                        RadixCtl* __restrict__ ctl, unsigned int* __restrict__ order) {
+  const unsigned int n32 = (unsigned int)n;
+  int executed = 0;
+  for (int d = 0; d < kDigits; ++d) executed += digit_is_constant(ctl, d, n32) ? 0 : 1;
+  const unsigned int* vals = (executed & 1) ? vbuf1 : vbuf0;
+  for (int64_t p = blockIdx.x * 256ll + threadIdx.x; p < n; p += (int64_t)gridDim.x * 256)
+    order[p] = executed == 0 ? (unsigned int)p : vals[p];
 }
 
 // ------------------------------------------------------------------------------------------
@@ -615,7 +602,7 @@ extern "C" int hba_rank_avg_f64(const double* x, int64_t n, double* ranks, void*
   HBA_REQUIRE(n < (1ll << 30), "hba_rank_avg_f64: n too large");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (n <= kSmallN) {
-    rank_small_kernel<<<1, 1024, 0, s>>>(x, (int)n, ranks);
+    rank_small_kernel<false><<<1, 1024, 0, s>>>(x, (int)n, ranks, nullptr);
     return check_launch("rank_small_kernel");
   }
   HBA_REQUIRE(workspace && workspace_bytes >= hba_rank_workspace_bytes(n) &&
@@ -623,6 +610,27 @@ extern "C" int hba_rank_avg_f64(const double* x, int64_t n, double* ranks, void*
               "hba_rank_avg_f64: workspace too small or not 256-byte aligned (need %lld bytes)",
               (long long)hba_rank_workspace_bytes(n));
   return rank_large(x, n, rank_workspace_layout(workspace, n), ranks, nullptr, nullptr, s);
+}
+
+extern "C" int hba_rank_order_f64(const double* x, int64_t n, uint32_t* order, double* ranks, void* workspace,
+                                  int64_t workspace_bytes, void* stream) {
+  HBA_REQUIRE(x && order && ranks && n > 0, "hba_rank_order_f64: bad arguments");
+  HBA_REQUIRE(n < (1ll << 30), "hba_rank_order_f64: n too large");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n <= kSmallN) {
+    rank_small_kernel<true><<<1, 1024, 0, s>>>(x, (int)n, ranks, order);
+    return check_launch("rank_small_kernel");
+  }
+  HBA_REQUIRE(workspace && workspace_bytes >= hba_rank_workspace_bytes(n) &&
+                  ((uintptr_t)workspace & 255) == 0,
+              "hba_rank_order_f64: workspace too small or not 256-byte aligned (need %lld bytes)",
+              (long long)hba_rank_workspace_bytes(n));
+  const RankWorkspace w = rank_workspace_layout(workspace, n);
+  HBA_CHECK(rank_large(x, n, w, ranks, nullptr, nullptr, s));
+  int g = (int)((n + 255) / 256);
+  if (g > kFinalBlocks) g = kFinalBlocks;
+  sorted_order_kernel<<<g, 256, 0, s>>>(w.v0, w.v1, n, w.ctl, order);
+  return check_launch("sorted_order_kernel");
 }
 
 extern "C" int hba_pearson_f64(const double* a, const double* b, int64_t n, double* rho_out,

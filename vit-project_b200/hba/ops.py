@@ -43,7 +43,7 @@ class EventProfile:
         class _Lib:
             def __getattr__(self, name):
                 fn = getattr(real.load(), name)
-                if not name.startswith("hba_") or name in ("hba_last_error", "hba_rank_workspace_bytes"):
+                if not name.startswith("hba_") or name == "hba_last_error" or name.endswith("_workspace_bytes"):
                     return fn
 
                 def bracketed(*args):
@@ -380,6 +380,50 @@ def rdm_spearman(E, ref_ranks, rho_out, workspace, rdm=None, ranks=None):
                                        workspace.numel(), _stream()), "hba_rdm_spearman", 11)
 
 
+def rank_order_f64(x, order, ranks, workspace):
+    """ranks as rank_avg_f64, and order [n] int32 (uint32 bits): the stable sorted order of x."""
+    n = x.numel()
+    assert x.dtype == torch.float64 and ranks.dtype == torch.float64 and order.dtype == torch.int32
+    assert x.is_contiguous() and order.numel() == n and ranks.numel() == n
+    check(_lib.load().hba_rank_order_f64(_p(x), n, _p(order), _p(ranks), _p(workspace), workspace.numel(), _stream()),
+          "hba_rank_order_f64", 1 if n <= 2048 else 11)
+
+
+def rsa_perm_workspace_bytes(N, n_perm):
+    return int(_lib.load().hba_rsa_perm_workspace_bytes(N, n_perm))
+
+
+def rsa_perm_null(ref_ranks, model_ranks, perms, rho_out, workspace):
+    """Mantel null: rho_out[p] = Spearman rho of the reference against the model relabelled by perms[p]
+    (perms [n_perm, N] int32, every row a permutation - the caller checks that)."""
+    n_perm, N = perms.shape
+    P = N * (N - 1) // 2
+    assert ref_ranks.dtype == model_ranks.dtype == rho_out.dtype == torch.float64 and perms.dtype == torch.int32
+    assert ref_ranks.numel() == model_ranks.numel() == P and rho_out.numel() >= n_perm and perms.is_contiguous()
+    check(_lib.load().hba_rsa_perm_null(_p(ref_ranks), _p(model_ranks), N, _p(perms), n_perm, _p(rho_out),
+                                        _p(workspace), workspace.numel(), _stream()), "hba_rsa_perm_null", 3)
+
+
+def rsa_boot_workspace_bytes(N, n_boot):
+    return int(_lib.load().hba_rsa_boot_workspace_bytes(N, n_boot))
+
+
+def rsa_bootstrap(ref_tri, ref_order, tri_a, order_a, counts, rho_a, workspace, tri_b=None, order_b=None, rho_b=None):
+    """Stimulus bootstrap: rho_a[b] (and rho_b[b]) = Spearman rho of the reference against model a (b) over the
+    pairs of the resample with counts[b] (counts [n_boot, N] int32, each row summing to N)."""
+    n_boot, N = counts.shape
+    P = N * (N - 1) // 2
+    assert counts.dtype == torch.int32 and counts.is_contiguous() and rho_a.numel() >= n_boot
+    for t in (ref_tri, tri_a, tri_b):
+        assert t is None or (t.dtype == torch.float64 and t.numel() == P)
+    for t in (ref_order, order_a, order_b):
+        assert t is None or (t.dtype == torch.int32 and t.numel() == P)
+    kernels = 2 + 6 * (3 if tri_b is not None else 2)
+    check(_lib.load().hba_rsa_bootstrap(_p(ref_tri), _p(ref_order), _p(tri_a), _p(order_a), _p(tri_b), _p(order_b), N,
+                                        _p(counts), n_boot, _p(rho_a), _p(rho_b), _p(workspace), workspace.numel(),
+                                        _stream()), "hba_rsa_bootstrap", kernels)
+
+
 def softmax_ce(logits, labels, loss, d_logits, correct, workspace):
     B, Cc = logits.shape
     check(_lib.load().hba_softmax_ce_fwd_bwd(_p(logits), logits.stride(0), _p(labels), B, Cc, _p(loss),
@@ -471,7 +515,8 @@ def _device_guarded(fn):
 for _name in ("gemm", "split_bf16", "layernorm_fwd", "layernorm_bwd", "im2col_patches", "assemble_tokens_ln",
               "embed_tokens", "gather_rows", "attention_fwd", "attention_bwd_row0", "dora_merge_fwd", "dora_merge_bwd",
               "cos_head_fwd", "cos_head_bwd", "cos_mse_fwd", "cos_mse_bwd", "adamw_multi", "sgd_multi", "sgd_staged",
-              "rdm_f64", "rank_avg_f64", "pearson_f64", "rdm_spearman", "softmax_ce", "colsum", "layernorm_param_grad",
+              "rdm_f64", "rank_avg_f64", "pearson_f64", "rdm_spearman", "rank_order_f64", "rsa_perm_null",
+              "rsa_bootstrap", "softmax_ce", "colsum", "layernorm_param_grad",
               "attention_bwd", "layernorm_bwd_fused", "attention_fwd_lse", "attention_bwd_lse", "add_rows",
               "nonfinite_flag"):
     globals()[_name] = _device_guarded(globals()[_name])

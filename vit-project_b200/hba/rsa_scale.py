@@ -24,6 +24,9 @@ import numpy as np
 import torch
 
 RESULT_COLUMNS = ("checkpoint", "run", "epoch", "behavioral_rsa_rho", "behavioral_rsa_p_value")
+# written only when asked for (n_perm > 0 / n_boot > 0): Mantel p-value, stimulus-bootstrap 95 % interval of rho
+PERMUTATION_COLUMNS = ("behavioral_rsa_p_perm",)
+BOOTSTRAP_COLUMNS = ("behavioral_rsa_ci_low", "behavioral_rsa_ci_high", "behavioral_rsa_boot_valid")
 _EPOCH = re.compile(r"epoch(\d+)_dora_params\.pth$")
 
 
@@ -64,11 +67,14 @@ def embeddings(model, loaders, device):
 
 
 def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank=0, world_size=1, output_csv=None,
-                              log=print, root=None, evaluator=None, embed_fn=None):
+                              log=print, root=None, evaluator=None, embed_fn=None, n_perm=0, n_boot=0, seed=0):
     """-> (rows, per-rank stats) on rank 0 | None.  `model`: CLIPHBA with its adapters applied (weights of the
     checkpoints are loaded with strict=False exactly as NEW:1159 does); `loaders`: ResidentLoaders whose concatenation
     is the image set in the order of `reference_rdm`'s rows.  `evaluator` / `embed_fn` default to the libhba ones
-    (hba.rsa.RSAEvaluator, `embeddings`); the world-2 `gloo` test of the sharding passes CPU stand-ins."""
+    (hba.rsa.RSAEvaluator, `embeddings`); the world-2 `gloo` test of the sharding passes CPU stand-ins.
+    n_perm > 0 adds PERMUTATION_COLUMNS (RSAEvaluator.permutation_test), n_boot > 0 adds BOOTSTRAP_COLUMNS
+    (RSAEvaluator.bootstrap, 95 % percentile interval); `seed` seeds both, so every checkpoint sees the same
+    permutations and resamples."""
     if evaluator is None:
         from .rsa import RSAEvaluator
         evaluator = RSAEvaluator(reference_rdm, device)
@@ -92,6 +98,11 @@ def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank
         rows.append({"checkpoint": rel, "run": os.path.basename(os.path.dirname(os.path.dirname(path))) or ".",
                      "epoch": int(_EPOCH.search(path).group(1)), "behavioral_rsa_rho": rho,
                      "behavioral_rsa_p_value": p})
+        if n_perm > 0:
+            rows[-1]["behavioral_rsa_p_perm"] = evaluator.permutation_test(emb, n_perm=n_perm, seed=seed)[1]
+        if n_boot > 0:
+            (lo, hi), _, valid = evaluator.bootstrap(emb, n_boot=n_boot, seed=seed)
+            rows[-1].update(behavioral_rsa_ci_low=lo, behavioral_rsa_ci_high=hi, behavioral_rsa_boot_valid=valid)
         if log is not None:
             log(f"[rank {rank}] {rel}: rho {rho:.6f}")
     stats = {"rank": rank, "checkpoints": len(rows), "embed_s": t_emb, "rsa_tail_s": t_rsa}
@@ -109,5 +120,7 @@ def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank
     if output_csv:
         import pandas as pd
         os.makedirs(os.path.dirname(os.path.abspath(output_csv)), exist_ok=True)
-        pd.DataFrame(rows, columns=list(RESULT_COLUMNS)).to_csv(output_csv, index=False)
+        columns = (list(RESULT_COLUMNS) + (list(PERMUTATION_COLUMNS) if n_perm > 0 else [])
+                   + (list(BOOTSTRAP_COLUMNS) if n_boot > 0 else []))
+        pd.DataFrame(rows, columns=columns).to_csv(output_csv, index=False)
     return rows, stats
