@@ -162,7 +162,7 @@ def run_arm(arm):
                 perturb_seed=42, previous_training_res_path=f"{b}/res.csv"))
             out["runs"][name] = summarise(d, f"{d}/res.csv", f"{d}/dora", f"{d}/rand")
         # another adapter placement than the drivers' 2 + 1: every block of the miniature adapted (NEW:484-513 is general)
-        # (2 + 2 in the fp32 parity mode: the text tower's general path; 3 + 2 in the bf16 mode: at the pipeline's
+        # (2 + 2 in the fp32 parity mode: two live text blocks; 3 + 2 in the bf16 mode: at the pipeline's
         # 224-pixel images the vision tower has T = 257 tokens, beyond the fp32 form of the full attention backward)
         for name, nv, nt, mode in (("baseline_2p2", 2, 2, "fp32"), ("baseline_3p2", 3, 2, "bf16")):
             if stack is not None:

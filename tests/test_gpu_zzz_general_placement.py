@@ -1,5 +1,5 @@
 """GPU test of adapter placements beyond the reference drivers' 2 vision + 1 text (apply_dora_to_ViT is general,
-NEW:484-513): hba.engine's general path - every block from the first adapted one on all rows, backward through MLP,
+NEW:484-513): hba.engine runs every block from the first adapted one on all rows, backward through MLP,
 out_proj, softmax attention (hba_attention_bwd), in_proj and ln_1 of each - against the oracle model with torch
 autograd.  The same cases run on the CPU restatement of libhba in tests/test_host_on_ref_lib_cpu.py (sequencing); here
 the kernels are the real ones.  (File name: sorts after every other GPU test.)"""
@@ -24,12 +24,12 @@ def _custom_state_dict(vision_layers, transformer_layers, seed=1):
 
 
 # (native 224-pixel images only: T = 257 / 77 are the shapes every kernel involved has been run at on the B200; the
-# fp32 form of the vision tower's general path needs T <= 200 and is covered on the CPU restatement)
+# fp32 form of more than two live vision blocks needs T <= 200 and is covered on the CPU restatement)
 @pytest.mark.parametrize("blocks,adapters,res,precision,tol_loss,tol_grad", [
     ((3, 2), (3, 2), 224, "bf16", 3e-2, 1.5e-1),    # every block live, T = 257 like ViT-L/14 (all-bf16 attention backward)
     ((4, 3), (3, 2), 224, "bf16", 3e-2, 1.5e-1),    # a frozen block below the live ones in both towers
-    ((4, 3), (2, 3), 224, "fp32", 1e-3, 2e-3),      # text tower general in the parity mode (causal fp32 attention backward)
-    ((3, 2), (2, 2), 224, "bf16", 3e-2, 1.5e-1),    # text tower general, vision on the 2 + 1 path
+    ((4, 3), (2, 3), 224, "fp32", 1e-3, 2e-3),      # three live text blocks in the parity mode (causal fp32 attention backward)
+    ((3, 2), (2, 2), 224, "bf16", 3e-2, 1.5e-1),    # two live text blocks, the last 2 vision blocks live
 ])
 def test_general_adapter_placement_matches_the_oracle_model_on_the_device(blocks, adapters, res, precision, tol_loss,
                                                                           tol_grad):

@@ -120,7 +120,7 @@ def test_run_behavioral_training_equals_the_reference_executed(tmp_path):
     repo's `run_behavioral_training` on the CPU restatement of libhba (fp32 mode, resident loaders, trunk cache,
     fused MSE, FusedAdamW), from the same image / csv / .mat / checkpoint files: a 3-epoch baseline, two conditions
     resumed from its epoch-2 checkpoints (random targets, label shuffle), one that perturbs epoch 1 from scratch, and
-    two baselines with other adapter placements (2 + 2 in fp32 mode, 3 + 2 in bf16 mode: the general path).
+    two baselines with other adapter placements (2 + 2 in fp32 mode, 3 + 2 in bf16 mode: deeper live ranges).
     Losses within 2e-5 (fp32 re-association), RSA rho / p within 1e-6, and - exactly - epochs, perturbation flags,
     files, checkpoint keys, optimizer step counts and the torch / NumPy / DataLoader-generator states at the end
     (which also pins the RNG draws of the model construction, clip.replay_constructor_draws)."""
@@ -216,13 +216,13 @@ def _custom_state_dict(vision_layers, transformer_layers, seed=1):
     ((3, 2), (3, 2), 112, "fp32", 2e-4),      # resized positional table (T = 65): the fp32 form of the full backward
     ((4, 3), (3, 2), 112, "fp32", 2e-4),      # a frozen block below the live ones in both towers
     ((4, 3), (4, 3), 224, "bf16", 8e-2),
-    ((4, 3), (3, 1), 112, "fp32", 2e-4),      # vision general, text on the 2 + 1 path
-    ((4, 3), (2, 3), 112, "fp32", 2e-4),      # text general, vision on the 2 + 1 path
+    ((4, 3), (3, 1), 112, "fp32", 2e-4),      # three live vision blocks, only the last text block live
+    ((4, 3), (2, 3), 112, "fp32", 2e-4),      # three live text blocks, the last 2 vision blocks live
 ])
 def test_general_adapter_placement_matches_the_oracle_model(blocks, adapters, res, precision, tol):
     """apply_dora_to_ViT(n_vision_layers, n_transformer_layers) is general (NEW:484-513); the reference drivers use
-    2 + 1.  Any other placement runs the general path of hba.engine (every block from the first adapted one on all
-    rows, backward through MLP / out_proj / attention / in_proj / ln_1 of each) - here on the CPU restatement of libhba
+    2 + 1.  Any other placement makes more of each tower live in hba.engine (every block from the first adapted one on
+    all rows, backward through MLP / out_proj / attention / in_proj / ln_1 of each) - here on the CPU restatement of libhba
     against the oracle model with torch autograd: loss and the gradients of every adapter tensor."""
     import hba
     from oracle import clip_ref, dora_ref
@@ -251,7 +251,7 @@ def test_general_adapter_placement_matches_the_oracle_model(blocks, adapters, re
             lp = crit(product(images), targets)
             lp.backward()
             with torch.no_grad():
-                again = product(images)              # the no-grad forward (evaluation) takes the same general path
+                again = product(images)              # the no-grad forward (evaluation) runs the same blocks
         assert abs(float(lp.detach()) - float(lo.detach())) <= tol * abs(float(lo.detach()))
         assert abs(float(crit(again, targets)) - float(lp.detach())) <= 1e-6 * abs(float(lp.detach()))
         named_p = [(n, p) for n, p in product.named_parameters() if p.requires_grad]
@@ -260,7 +260,7 @@ def test_general_adapter_placement_matches_the_oracle_model(blocks, adapters, re
         for (n, a), (_, b) in zip(named_p, named_o):
             assert a.grad is not None and float((a.grad - b.grad).abs().max() / b.grad.abs().max()) <= tol, n
         if max(adapters[0] - 2, adapters[1] - 1) > 0:
-            assert "hba_attention_bwd" in lib.calls       # the full attention backward of the general path
+            assert "hba_attention_bwd" in lib.calls       # the full attention backward below the last block
     finally:
         hba.set_precision("bf16")
 
@@ -326,10 +326,10 @@ def test_fp32_mode_refuses_deep_vision_placement_at_257_tokens():
         hba.set_precision("bf16")
 
 
-def _abi_trace_of_default_placement():
+def _abi_trace(sd, adapters, res, precisions):
     """(names + every scalar argument + which pointers are null) of all C-ABI calls of: staging, three training
-    steps of the 2 + 1 placement (no cache / cache fill / cache hit) with FusedAdamW, one evaluation batch - in both
-    precision modes."""
+    steps of the placement `adapters` = (n_vision, n_text) (no cache / cache fill / cache hit at the model's native
+    resolution) with FusedAdamW, one evaluation batch - in each precision mode of `precisions`."""
     import ctypes as C
     import hba
     from hba._lib import SIGNATURES
@@ -361,17 +361,16 @@ def _abi_trace_of_default_placement():
     real = libhba_ref.RefLib
     libhba_ref.RefLib = Tracing
     try:
-        sd = clip_ref.synthetic_state_dict("ViT-tiny/14", seed=1)
         tokens = torch.stack([clip_ref.tokenize(p) for p in ("metallic; artificial", "food-related", "animal-related",
                                                              "textile")])
         g = torch.Generator().manual_seed(0)
-        images = torch.randn(3, 3, 224, 224, generator=g)
+        images = torch.randn(3, 3, res, res, generator=g)
         targets = torch.randn(3, 4, generator=g)
-        for precision in ("bf16", "fp32"):
+        for precision in precisions:
             hba.set_precision(precision)
             product = dora_ref.CLIPHBARef(pclip.build_model(sd), tokens)
             torch.manual_seed(123)
-            dora_ref.apply_dora_ref(product, 2, 1, r=8, layer_cls=hba.DoRALayer)
+            dora_ref.apply_dora_ref(product, *adapters, r=8, layer_cls=hba.DoRALayer)
             dora_ref.switch_dora_ref(product, layer_cls=hba.DoRALayer)
             with libhba_ref.emulated_device():
                 opt = FusedAdamW(product.parameters(), lr=3e-4)
@@ -391,16 +390,10 @@ def _abi_trace_of_default_placement():
     return trace
 
 
-def test_c_abi_call_trace_of_the_reference_placement_is_pinned():
-    """The kernel sequence of the reference drivers' placement (2 vision + 1 text adapters, BDRV:28-30) is what every
-    B200 measurement and GPU parity run of this repo exercised.  Its C-ABI call trace on the CPU restatement - entry
-    points, shapes, leading dimensions, flags, which optional pointers are given - is pinned by a digest: a change of
-    hba.engine / hba.dora / hba.optim that alters what is launched for this placement must be deliberate (regenerate:
-    HBA_WRITE_TRACE_GOLDEN=1)."""
+def _check_trace_golden(trace, golden):
     import hashlib
-    trace = _abi_trace_of_default_placement()
     digest = hashlib.sha256(repr(trace).encode()).hexdigest()
-    path = os.path.join(GOLD, "c_abi_trace_2p1.json")
+    path = os.path.join(GOLD, golden)
     counts = {}
     for name, _ in trace:
         counts[name] = counts.get(name, 0) + 1
@@ -410,3 +403,80 @@ def test_c_abi_call_trace_of_the_reference_placement_is_pinned():
     gold = json.load(open(path))
     assert len(trace) == gold["calls"] and counts == gold["per_entry"], (len(trace), counts)
     assert digest == gold["sha256"]
+
+
+def test_c_abi_call_trace_of_the_reference_placement_is_pinned():
+    """The kernel sequence of the reference drivers' placement (2 vision + 1 text adapters, BDRV:28-30) is what every
+    B200 measurement and GPU parity run of this repo exercised.  Its C-ABI call trace on the CPU restatement - entry
+    points, shapes, leading dimensions, flags, which optional pointers are given - is pinned by a digest: a change of
+    hba.engine / hba.dora / hba.optim that alters what is launched for this placement must be deliberate (regenerate:
+    HBA_WRITE_TRACE_GOLDEN=1)."""
+    from oracle import clip_ref
+    _check_trace_golden(_abi_trace(clip_ref.synthetic_state_dict("ViT-tiny/14", seed=1), (2, 1), 224, ("bf16", "fp32")),
+                        "c_abi_trace_2p1.json")
+
+
+@pytest.mark.parametrize("blocks,adapters,res,precision,golden", [
+    (None, (3, 2), 224, "bf16", "c_abi_trace_3p2_bf16.json"),          # every block of the miniature live, trunk cache
+    ((4, 3), (2, 3), 112, "fp32", "c_abi_trace_2p3_fp32_112.json"),    # three live text blocks above a frozen one
+])
+def test_c_abi_call_trace_of_deeper_placements_is_pinned(blocks, adapters, res, precision, golden):
+    """The same pin for placements with live blocks below the last one: their forward keeps only what the backward
+    reads, and their backward walks the live blocks down to the lowest trainable adapter."""
+    from oracle import clip_ref
+    sd = clip_ref.synthetic_state_dict("ViT-tiny/14", seed=1) if blocks is None else _custom_state_dict(*blocks)
+    _check_trace_golden(_abi_trace(sd, adapters, res, (precision,)), golden)
+
+
+@pytest.mark.parametrize("blocks,adapters,res,precision", [
+    (None, (2, 1), 224, "bf16"),
+    ((4, 3), (3, 2), 112, "fp32"),
+])
+def test_tower_forwards_use_disjoint_workspaces(blocks, adapters, res, precision):
+    """The text tower's forward runs on a side stream concurrently with the vision tower's (HBA_TEXT_STREAM): a
+    workspace both request would be raced on by the device.  Every Engine._buf key requested under the vision forward
+    (vision_trunk / vision_head) must differ from every key requested under the text forward (text_features), in
+    training steps with and without the trunk cache and in evaluation."""
+    import inspect
+    import hba
+    from hba.engine import Engine, TrunkCache
+    from oracle import clip_ref, dora_ref
+    from oracle.libhba_ref import emulated_device
+    from src.models.CLIPs.clip_hba import clip as pclip
+    keys = {"vision": set(), "text": set()}
+    real_buf = Engine._buf
+
+    def recording_buf(self, name, shape, dtype=torch.float32, zero=False):
+        for frame in inspect.stack(0):
+            tower = {"vision_trunk": "vision", "vision_head": "vision", "text_features": "text"}.get(frame.function)
+            if tower:
+                keys[tower].add((name, tuple(shape), dtype))
+                break
+        return real_buf(self, name, shape, dtype, zero)
+
+    sd = clip_ref.synthetic_state_dict("ViT-tiny/14", seed=1) if blocks is None else _custom_state_dict(*blocks)
+    tokens = torch.stack([clip_ref.tokenize(p) for p in ("metallic; artificial", "food-related")])
+    images = torch.randn(3, 3, res, res, generator=torch.Generator().manual_seed(0))
+    try:
+        hba.set_precision(precision)
+        Engine._buf = recording_buf
+        product = dora_ref.CLIPHBARef(pclip.build_model(sd), tokens)
+        torch.manual_seed(123)
+        dora_ref.apply_dora_ref(product, *adapters, r=4, layer_cls=hba.DoRALayer)
+        dora_ref.switch_dora_ref(product, layer_cls=hba.DoRALayer)
+        with emulated_device():
+            eng = product.clip_model.hba_engine()
+            eng.trunk_cache = TrunkCache(8)
+            for ids in (None, [1, 2, 3], [1, 2, 3]):
+                eng.batch_ids = ids
+                product(images).square().mean().backward()
+            with torch.no_grad():
+                eng.batch_ids = [1, 2, 3]
+                product(images)
+    finally:
+        Engine._buf = real_buf
+        hba.set_precision("bf16")
+    assert keys["vision"] and keys["text"]
+    assert not keys["vision"] & keys["text"], sorted(keys["vision"] & keys["text"])
+    assert all(k[0].startswith(("v", "keep.v")) for k in keys["vision"]), sorted(keys["vision"])
+    assert all(k[0].startswith(("t", "keep.t")) for k in keys["text"]), sorted(keys["text"])

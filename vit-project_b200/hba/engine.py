@@ -10,11 +10,14 @@ fp32 re-association):
   * text tower: embedding, L_t causal blocks; after the last attention only the EOT rows are kept
     (everything after it is row-wise);
   * cosine logits  exp(logit_scale) * <img, txt>.
-Backward covers exactly the sub-graph that reaches trainable parameters in the reference setup
-(NEW:484-544: `out_proj` of the last <= 2 vision blocks and of the last text block): it returns
-dL/dW for those `out_proj.weight` tensors; the DoRA chain rule on top is hba.dora (fused) or plain
-autograd when the reference's own DoRALayer is used.  Deeper placements (apply_dora_to_ViT is general)
-take the general path further down: all rows of every block from the first adapted one, full backward.
+Each tower has one live range, blocks [first, L) with first = L - n_live: the first adapted block, and
+at least the last 2 vision / last 1 text blocks - the reference drivers' placement (NEW:484-544, BDRV:28-30).
+Blocks below it are frozen and run in place (or come from the trunk / text cache), blocks [first, L-1)
+run on all rows and keep only what the backward reads, the last block runs on the CLS / EOT rows.
+Backward covers exactly the sub-graph that reaches trainable parameters: the last block's rows, then
+down through the live blocks to the lowest trainable adapter.  It returns dL/dW of the adapters'
+`out_proj.weight` tensors; the DoRA chain rule on top is hba.dora (fused) or plain autograd when the
+reference's own DoRALayer is used.
 
 Precision modes (hba.set_precision):
   "bf16": bf16 operands, fp32 accumulate (tcgen05 kind::f16), fp32 residual stream / LN / softmax
@@ -84,7 +87,6 @@ class Engine:
         self.loss_out = None      # the fused loss of the last forward that carried a LossRequest
         self._text_cache = None
         self._gen = 0
-        self.launches = 0  # kernels launched by the last run_forward / run_backward (our own count)
 
     # ---------------------------------------------------------------- staging
     @property
@@ -239,15 +241,18 @@ class Engine:
         return self._pos_cache[grid_now]
 
     # ---------------------------------------------------------------- building blocks
+    def _act_dtype(self):
+        """dtype of the kept qkv / MLP pre-activations and of the all-row attention gradients."""
+        return torch.float32 if self.split else torch.bfloat16
+
     def _qkv_buffer(self, tag, M, d):
-        return self._buf(tag + ".qkv", (M, 3 * d), torch.float32 if self.split else torch.bfloat16)
+        return self._buf(tag + ".qkv", (M, 3 * d), self._act_dtype())
 
     def _gemm_qkv(self, h, w_in, b_in, qkv, M):
         if self.split:
             ops.gemm(h, w_in, M, bias=b_in, out_f32=qkv)
         else:
             ops.gemm(h, w_in, M, bias=b_in, out=Operand(qkv, M, qkv.shape[1], 0))
-        self.launches += 1
 
     def _adapter_operands(self, W):
         """bf16 operands of an adapter weight W [out, in]: (w [out,in], wt [in,out])."""
@@ -266,8 +271,15 @@ class Engine:
             base = Wd.contiguous()
             ops.split_bf16(base, w)
             ops.split_bf16(base, wt, transpose=True)
-        self.launches += 2
         return w, wt
+
+    def _block_weights(self, blk, adapters, i, need_grad):
+        """(w [out,in], wt [in,out], bias, trainable) of block i's out_proj."""
+        if blk.adapter:
+            W, bias = adapters[i]
+            w, wt = self._adapter_operands(W)
+            return w, wt, bias.detach(), bool(need_grad and W.requires_grad)
+        return blk.w_out, blk.w_out_t, blk.b_out, False
 
     def _skinny(self, tag, R, N, K):
         """Split-K arguments of a row GEMM (R = the CLS / EOT rows, one row tile): its N / 256 output tiles would
@@ -281,45 +293,96 @@ class Engine:
             return {}
         return {"k_slices": s, "k_workspace": self._buf(tag + ".kws", (s * R * N,))}
 
-    def _block_full(self, tw, blk, tag, x_in, x_mid, x_out, B, w_out, b_out, keep=None):
-        """One full residual attention block on all M = B*T rows (x_* are fp32 [M, d])."""
-        a = self._attn_part(tw, blk, tag, x_in, B, keep.get("a_f32") if keep else None)
-        self._live_part(tw, blk, tag, a, x_in, x_mid, x_out, B, w_out, b_out, keep)
-
-    def _attn_part(self, tw, blk, tag, x_in, B, a_f32=None):
-        """ln_1 -> in_proj -> softmax attention on all rows; returns the attention output as a GEMM
-        operand (and in fp32 when `a_f32` is given).  Frozen in every block of the reference setup."""
-        T, d, H = tw.T, tw.d, tw.heads
+    def _attn_part(self, tw, blk, tag, x_in, B, a, qkv=None, a_f32=None):
+        """ln_1 -> in_proj -> softmax attention on all rows into the GEMM operand `a` (and in fp32 into `a_f32` when
+        given).  `qkv` receives the projections when the attention backward reads them, else the tower's scratch."""
+        T, d = tw.T, tw.d
         M = B * T
         h = self._opbuf(tag + ".h", M, d)
         ops.layernorm_fwd(x_in, M, d, blk.ln1_w, blk.ln1_b, LN_EPS, y=h)
-        qkv = self._qkv_buffer(tag, M, d)
+        if qkv is None:
+            qkv = self._qkv_buffer(tag, M, d)
         self._gemm_qkv(h, blk.w_in, blk.b_in, qkv, M)
-        a = self._opbuf(tag + ".a", M, d)
-        ops.attention_fwd(qkv, B, T, H, causal=tw.causal, out=a, out_f32=a_f32)
-        self.launches += 3
-        return a
+        ops.attention_fwd(qkv, B, T, tw.heads, causal=tw.causal, out=a, out_f32=a_f32)
 
-    def _live_part(self, tw, blk, tag, a, x_in, x_mid, x_out, B, w_out, b_out, keep=None):
-        """out_proj (+ residual) -> ln_2 -> MLP (+ residual) on all rows."""
+    def _live_part(self, tw, blk, tag, a, x_in, x_mid, x_out, B, w_out, b_out, h_pre=None):
+        """out_proj (+ residual) -> ln_2 -> MLP (+ residual) on all rows (x_* are fp32 [M, d], possibly the same)."""
         d = tw.d
         M = B * tw.T
         ops.gemm(a, w_out, M, bias=b_out, residual=x_in, out_f32=x_mid)
         h = self._opbuf(tag + ".h", M, d)
         ops.layernorm_fwd(x_mid, M, d, blk.ln2_w, blk.ln2_b, LN_EPS, y=h)
         hid = self._opbuf(tag + ".hid", M, 4 * d)
-        ops.gemm(h, blk.w_fc, M, bias=blk.b_fc, act=HBA_ACT_QUICKGELU, out=hid,
-                 pre_out=keep.get("h_pre") if keep else None)
+        ops.gemm(h, blk.w_fc, M, bias=blk.b_fc, act=HBA_ACT_QUICKGELU, out=hid, pre_out=h_pre)
         ops.gemm(hid, blk.w_proj, M, bias=blk.b_proj, residual=x_mid, out_f32=x_out)
-        self.launches += 4
 
-    def _rows_tail(self, tw, blk, tag, a_rows, x_res, R, w_out, b_out, keep):
-        """out_proj + MLP of a block on R selected rows (CLS rows / EOT rows).
-        a_rows: Operand [R, d] (attention output rows); x_res: fp32 view [R, *] of the block input
-        rows (row stride arbitrary).  Returns x_out [R, d] fp32."""
-        d = tw.d
+    def _frozen_blocks(self, tw, tag, x, B, upto):
+        """Blocks [0, upto) in place on all rows of x (fp32 [B*T, d]): nothing below the first adapter is
+        differentiated."""
+        for blk in tw.blocks[:upto]:
+            if blk.adapter:
+                raise RuntimeError("libhba: an adapter below the staged live blocks (restage: Engine.prepare)")
+            a = self._opbuf(tag + ".a", B * tw.T, tw.d)
+            self._attn_part(tw, blk, tag, x, B, a)
+            self._live_part(tw, blk, tag, a, x, x, x, B, blk.w_out, blk.b_out)
+
+    def _live_blocks_fwd(self, tw, tag, x, B, adapters, need_grad, cache_ctx=None, keep_input=False):
+        """Blocks [first, L-1) on all M = B*T rows, `first` = L - tw.n_live.  The backward walks them down from the top
+        and stops at the lowest trainable adapter, so a block keeps
+          * its qkv when the attention backward runs through it (a trainable adapter below it);
+          * its MLP pre-activation, x_mid and x_out (the input of the block above) when the backward passes through
+            its MLP (a trainable adapter at or below it);
+          * its attention output as a GEMM operand (the dW operand) when it is trainable.
+        Otherwise it runs in place on x like a frozen block - except on the input itself when `keep_input` (the text
+        trunk cache).  cache_ctx: the vision trunk cache, which holds the first live block's input and attention output.
+        -> (x, {block index: what its backward reads}, whether a trainable adapter sits in [first, L-1))."""
+        L, d, M = len(tw.blocks), tw.d, B * tw.T
+        first = L - tw.n_live
+        blocks, reach = {}, False
+        for i in range(first, L - 1):
+            blk = tw.blocks[i]
+            w, wt, bias, train = self._block_weights(blk, adapters, i, need_grad)
+            below, reach = reach, reach or train
+            name = f"{tag}{i}"
+            # (block L-2 may leave its dW operand in the tower's scratch: no later block writes it)
+            a = self._opbuf(name + ".a" if train and i < L - 2 else tag + ".a", M, d)
+            qkv = None
+            if i == first and cache_ctx is not None and cache_ctx["hit"]:
+                a_f32 = cache_ctx["a"]
+                ops.split_bf16(a_f32, a)
+            else:
+                fill = i == first and cache_ctx is not None
+                # (the dW reads the operand `a`; a trainable block writes the fp32 copy all the same)
+                a_f32 = self._keep(name + ".a_f32", (M, d)) if train or fill else None
+                if below:
+                    qkv = self._keep(name + ".qkv", (M, 3 * d), self._act_dtype())
+                self._attn_part(tw, blk, tag, x, B, a, qkv, a_f32)
+                if fill:
+                    cache_ctx["cache"].store(cache_ctx["ids"], x, a_f32)
+            x_mid = self._keep(name + ".x_mid", (M, d)) if reach or (keep_input and i == first) else x
+            x_out = self._keep(name + ".x_out", (M, d)) if reach else x_mid
+            h_pre = self._keep(name + ".h_pre", (M, 4 * d), self._act_dtype()) if reach else None
+            self._live_part(tw, blk, tag, a, x, x_mid, x_out, B, w, bias, h_pre)
+            if reach:
+                blocks[i] = {"train": train, "below": below, "a_op": a, "qkv": qkv, "x_in": x, "x_mid": x_mid,
+                             "h_pre": h_pre, "wt": wt}
+            x = x_out
+        return x, blocks, reach
+
+    def _last_block_keep(self, tag, R, d, train, below, x_in, wt):
+        """What the backward reads of the last block's R rows - None when no gradient passes through it."""
+        if not (train or below):
+            return None
+        return {"x_mid": self._keep(tag + ".xmidZ", (R, d)), "x_out": self._keep(tag + ".xoutZ", (R, d)),
+                "h_pre": self._keep(tag + ".hpreZ", (R, 4 * d), self._act_dtype()), "x_in": x_in, "wt": wt}
+
+    def _last_rows(self, tw, tag, a_rows, x_rows, R, w_out, b_out, keep, ln, proj_t):
+        """out_proj + MLP of the last block on R selected rows (CLS rows / EOT rows), then the final LN and the
+        projection.  a_rows: Operand [R, d] (attention output rows); x_rows: fp32 view [R, *] of the block input rows
+        (row stride arbitrary).  Returns the features [R, E] fp32."""
+        blk, d = tw.blocks[-1], tw.d
         x_mid = keep["x_mid"] if keep else self._buf(tag + ".xmid", (R, d))
-        ops.gemm(a_rows, w_out, R, bias=b_out, residual=x_res, out_f32=x_mid, **self._skinny(tag, R, d, d))
+        ops.gemm(a_rows, w_out, R, bias=b_out, residual=x_rows, out_f32=x_mid, **self._skinny(tag, R, d, d))
         h = self._opbuf(tag + ".h2", max(R, 128), d)
         ops.layernorm_fwd(x_mid, R, d, blk.ln2_w, blk.ln2_b, LN_EPS, y=h)
         hid = self._opbuf(tag + ".hid2", max(R, 128), 4 * d)
@@ -328,8 +391,11 @@ class Engine:
         x_out = keep["x_out"] if keep else self._buf(tag + ".xout", (R, d))
         ops.gemm(hid, blk.w_proj, R, bias=blk.b_proj, residual=x_mid, out_f32=x_out,
                  **self._skinny(tag, R, d, 4 * d))
-        self.launches += 4
-        return x_out
+        hp = self._opbuf(tag + ".lnf", max(R, 128), d)
+        ops.layernorm_fwd(x_out, R, d, ln[0], ln[1], LN_EPS, y=hp)
+        feat = self._keep(tag + ".feat", (R, self.E))
+        ops.gemm(hp, proj_t, R, out_f32=feat, **self._skinny(tag, R, self.E, d))
+        return feat
 
     # ---------------------------------------------------------------- forward
     def _keep(self, name, shape, dtype=torch.float32):
@@ -360,346 +426,90 @@ class Engine:
         x = self._buf("v.x", (M, d))
         ops.assemble_tokens_ln(conv, B, npatch, d, self.cls, self._positional(grid), self.ln_pre[0],
                                self.ln_pre[1], LN_EPS, x)
-        self.launches += 3
-        for i in range(upto):
-            blk = tw.blocks[i]
-            if blk.adapter:
-                raise RuntimeError("libhba: an adapter below the staged live blocks (restage: Engine.prepare)")
-            self._block_full(tw, blk, "v", x, x, x, B, blk.w_out, blk.b_out)
+        self._frozen_blocks(tw, "v", x, B, upto)
         return x, tw
 
     def vision_head(self, x, tw, B, adapters, need_grad, cache_ctx=None):
-        """Blocks L-2 (full) and L-1 (CLS row only) + ln_post + proj.  `adapters` maps block index
-        -> (W, bias) for adapter blocks.  Returns (img_feat [B,E] fp32, saved dict)."""
-        L = len(tw.blocks)
-        T, d, H = tw.T, tw.d, tw.heads
+        """Live blocks [first, L-1) on all rows (x: their input), block L-1 for the CLS query rows, ln_post, proj.
+        `adapters` maps block index -> (W, bias) for adapter blocks.  Returns (img_feat [B,E] fp32, saved dict)."""
+        L, T, d = len(tw.blocks), tw.T, tw.d
         M = B * T
-        saved = {"B": B, "T": T, "tw": tw}
-        # ---- block P = L-2, all rows
-        if L >= 2:
-            blkP = tw.blocks[L - 2]
-            keepP = None
-            if blkP.adapter:
-                Wp, bp = adapters[L - 2]
-                wP, _ = self._adapter_operands(Wp)
-                trainP = need_grad and Wp.requires_grad
-                saved["trainP"] = trainP
-                if trainP:
-                    keepP = {"h_pre": self._keep("hpreP", (M, 4 * d),
-                                                 torch.float32 if self.split else torch.bfloat16)}
-                    saved["keepP"] = keepP
-                bP = bp.detach()
-            else:
-                wP, bP = blkP.w_out, blkP.b_out
-                saved["trainP"] = False
-            x_mid = self._keep("xmidP", (M, d)) if keepP else x
-            x_out = self._keep("xoutP", (M, d)) if need_grad else x
-            a_f32 = None
-            if cache_ctx is not None and cache_ctx["hit"]:
-                # frozen half of block P (ln_1, in_proj, attention) comes from the trunk cache
-                a_f32 = cache_ctx["a"]
-                a = self._opbuf("v.a", M, d)
-                ops.split_bf16(a_f32, a)
-                self.launches += 1
-            else:
-                fill = cache_ctx is not None
-                if keepP or fill:
-                    a_f32 = self._keep("aP", (M, d))
-                a = self._attn_part(tw, blkP, "v", x, B, a_f32)
-                if fill:
-                    cache_ctx["cache"].store(cache_ctx["ids"], x, a_f32)
-            if keepP:
-                keepP["a_f32"] = a_f32
-                keepP["a_op"] = a
-            self._live_part(tw, blkP, "v", a, x, x_mid, x_out, B, wP, bP, keep=keepP)
-            if keepP:
-                keepP["x_mid"] = x_mid
-            x = x_out
-        # ---- block Z = L-1, CLS query rows only
-        blkZ = tw.blocks[L - 1]
-        if blkZ.adapter:
-            Wz, bz = adapters[L - 1]
-            wZ, wtZ = self._adapter_operands(Wz)
-            bZ = bz.detach()
-            trainZ = need_grad and Wz.requires_grad
-        else:
-            wZ, wtZ, bZ, trainZ = blkZ.w_out, None, blkZ.b_out, False
-        keepZ = None
-        if need_grad:
-            keepZ = {"x_mid": self._keep("xmidZ", (B, d)), "x_out": self._keep("xoutZ", (B, d)),
-                     "h_pre": self._keep("hpreZ", (B, 4 * d),
-                                         torch.float32 if self.split else torch.bfloat16),
-                     "a_f32": self._keep("aZ", (B, d)), "x_in": x, "wtZ": wtZ}
-        h = self._opbuf("v.h", M, d)
-        ops.layernorm_fwd(x, M, d, blkZ.ln1_w, blkZ.ln1_b, LN_EPS, y=h)
-        qkv = self._keep("qkvZ", (M, 3 * d), torch.float32 if self.split else torch.bfloat16) \
-            if need_grad else self._qkv_buffer("v", M, d)
-        self._gemm_qkv(h, blkZ.w_in, blkZ.b_in, qkv, M)
-        a_cls = self._opbuf("v.acls", max(B, 128), d)
-        ops.attention_fwd(qkv, B, T, H, first_row_only=True, out=a_cls,
-                          out_f32=keepZ["a_f32"] if keepZ else None)
-        x_cls = x.view(B, T * d)[:, :d]  # CLS rows of the block input, row stride T*d
-        x_out = self._rows_tail(tw, blkZ, "v", a_cls, x_cls, B, wZ, bZ, keepZ)
-        hp = self._opbuf("v.lnpost", max(B, 128), d)
-        ops.layernorm_fwd(x_out, B, d, self.ln_post[0], self.ln_post[1], LN_EPS, y=hp)
-        feat = self._keep("imgfeat", (B, self.E))
-        ops.gemm(hp, self.proj_t, B, out_f32=feat, **self._skinny("v", B, self.E, d))
-        self.launches += 4
-        saved.update(trainZ=trainZ, keepZ=keepZ, qkvZ=qkv)
-        return feat, saved
-
-    def text_features(self, tokens, adapters, need_grad):
-        """Text tower -> txt_feat [S, E]; the trunk up to the last attention is cached per token
-        tensor (the prompts never change, NEW:282)."""
-        tw = self.txt
-        S, T = tokens.shape
-        d, H, L = tw.d, tw.heads, len(tw.blocks)
-        M = S * T
-        key = (tokens.data_ptr(), tokens._version, S, T)
-        cache = self._text_cache if (self.cache_text and self._text_cache
-                                     and self._text_cache["key"] == key) else None
-        if cache is None:
-            x = self._buf("t.x", (M, d))
-            ops.embed_tokens(tokens, self.tok_table, self.tpos, x)
-            self.launches += 1
-            for i in range(L - 1):
-                blk = tw.blocks[i]
-                if blk.adapter:
-                    raise RuntimeError("libhba: an adapter below the last text block on the 2 + 1 path (restage: Engine.prepare)")
-                self._block_full(tw, blk, "t", x, x, x, S, blk.w_out, blk.b_out)
-            blkZ = tw.blocks[L - 1]
-            h = self._opbuf("t.h", M, d)
-            ops.layernorm_fwd(x, M, d, blkZ.ln1_w, blkZ.ln1_b, LN_EPS, y=h)
-            qkv = self._qkv_buffer("t", M, d)
-            self._gemm_qkv(h, blkZ.w_in, blkZ.b_in, qkv, M)
-            a_all = self._buf("t.a_f32", (M, d))
-            ops.attention_fwd(qkv, S, T, H, causal=True, out_f32=a_all)
-            eot = (tokens.argmax(dim=-1) + torch.arange(S, device=tokens.device) * T).contiguous()
-            # (persistent buffers, not fresh tensors: they are produced on the side stream and read by
-            # the backward pass on the main stream - nothing here may be recycled by the caching allocator)
-            a_eot = self._buf("t.a_eot", (S, d))
-            x_eot = self._buf("t.x_eot", (S, d))
-            ops.gather_rows(a_all, eot, d, a_eot)
-            ops.gather_rows(x, eot, d, x_eot)
-            a_op = self._opbuf("t.a_op", max(S, 128), d, zero=True)
-            ops.split_bf16(a_eot, a_op)
-            self.launches += 6
-            # (the entry keeps the token tensor alive: the key holds its ADDRESS, and the caching allocator would hand
-            # the address of a freed prompt tensor to the next model's prompts - other class names, same key)
-            cache = {"key": key, "a_eot": a_eot, "x_eot": x_eot, "a_op": a_op, "tokens": tokens}
-            if self.cache_text:
-                self._text_cache = cache
-        blkZ = tw.blocks[L - 1]
-        if blkZ.adapter:
-            Wz, bz = adapters[L - 1]
-            wZ, _ = self._adapter_operands(Wz)
-            bZ = bz.detach()
-            trainZ = need_grad and Wz.requires_grad
-        else:
-            wZ, bZ, trainZ = blkZ.w_out, blkZ.b_out, False
-        keepZ = None
-        if need_grad:
-            keepZ = {"x_mid": self._keep("t.xmidZ", (S, d)), "x_out": self._keep("t.xoutZ", (S, d)),
-                     "h_pre": self._keep("t.hpreZ", (S, 4 * d),
-                                         torch.float32 if self.split else torch.bfloat16),
-                     "a_f32": cache["a_eot"]}
-        x_out = self._rows_tail(tw, blkZ, "t", cache["a_op"], cache["x_eot"], S, wZ, bZ, keepZ)
-        hp = self._opbuf("t.lnfinal", max(S, 128), d)
-        ops.layernorm_fwd(x_out, S, d, self.ln_final[0], self.ln_final[1], LN_EPS, y=hp)
-        feat = self._keep("txtfeat", (S, self.E))
-        ops.gemm(hp, self.tproj_t, S, out_f32=feat, **self._skinny("t", S, self.E, d))
-        self.launches += 2
-        return feat, {"S": S, "trainZ": trainZ, "keepZ": keepZ}
-
-    # ---------------------------------------------------------------- general adapter placement
-    # apply_dora_to_ViT(n_vision_layers, n_transformer_layers) is general (NEW:484-513); the reference drivers use 2 + 1
-    # (BDRV:28-30), which is what the pruned graph above serves.  More adapted blocks make more of each tower live: the
-    # methods below run every block from the first adapted one on ALL rows, keep what its backward needs, and walk the
-    # blocks back through MLP, out_proj, softmax attention (hba_attention_bwd, recomputed from the kept qkv), in_proj
-    # and ln_1.  Same kernels as the 2 + 1 path; only taken when the placement asks for it.
-    def _general_dtype(self):
-        return torch.float32 if self.split else torch.bfloat16
-
-    def _full_block_fwd(self, tw, blk, name, x_in, B, w_out, b_out, need_grad, keep_attention, a_cached=None):
-        """One live block on all rows with everything its backward needs kept under `name`.
-        -> (x_out, kept dict).  a_cached: the block's attention output from the trunk cache (first live block)."""
-        d, T, H = tw.d, tw.T, tw.heads
-        M = B * T
-        dt = self._general_dtype()
-        kept = {"x_in": x_in}
-        if a_cached is not None:
-            a_f32 = a_cached
-            a = self._opbuf(name + ".a", M, d)
-            ops.split_bf16(a_f32, a)
-            self.launches += 1
-        else:
-            h = self._opbuf(name + ".h", M, d)
-            ops.layernorm_fwd(x_in, M, d, blk.ln1_w, blk.ln1_b, LN_EPS, y=h)
-            qkv = self._keep(name + ".qkv", (M, 3 * d), dt) if (need_grad and keep_attention) \
-                else self._qkv_buffer(name, M, d)
-            self._gemm_qkv(h, blk.w_in, blk.b_in, qkv, M)
-            a = self._opbuf(name + ".a", M, d)
-            a_f32 = self._keep(name + ".a_f32", (M, d))
-            ops.attention_fwd(qkv, B, T, H, causal=tw.causal, out=a, out_f32=a_f32)
-            self.launches += 3
-            kept["qkv"] = qkv
-        kept["a_f32"], kept["a_op"] = a_f32, a
-        x_mid = self._keep(name + ".x_mid", (M, d))
-        x_out = self._keep(name + ".x_out", (M, d))
-        kept["x_mid"] = x_mid
-        kept["h_pre"] = self._keep(name + ".h_pre", (M, 4 * d), dt) if need_grad else None
-        self._live_part(tw, blk, name, a, x_in, x_mid, x_out, B, w_out, b_out,
-                        keep={"h_pre": kept["h_pre"]} if need_grad else None)
-        return x_out, kept
-
-    def _block_weights(self, blk, adapters, i, need_grad):
-        """(w [out,in], wt [in,out], bias, trainable) of block i's out_proj."""
-        if blk.adapter:
-            W, bias = adapters[i]
-            w, wt = self._adapter_operands(W)
-            return w, wt, bias.detach(), bool(need_grad and W.requires_grad)
-        return blk.w_out, blk.w_out_t, blk.b_out, False
-
-    def vision_head_general(self, x, tw, B, adapters, need_grad, cache_ctx=None):
-        """Blocks first..L-2 on all rows, block L-1 for the CLS query row, ln_post, proj - `first` = the first adapted
-        block.  Returns (img_feat, saved) like vision_head."""
-        L, T, d, H = len(tw.blocks), tw.T, tw.d, tw.heads
-        first = L - tw.n_live
-        M = B * T
-        if self.split and T > 200:
+        if tw.n_live > 2 and self.split and T > 200:
             raise NotImplementedError("libhba fp32 mode: more than two adapted vision blocks need the full attention "
                                       "backward, whose fp32 form holds T <= 200 tokens (use the bf16 mode)")
-        saved = {"B": B, "T": T, "tw": tw, "general": True, "first": first, "blocks": {}}
-        trains = {}
-        for i in range(first, L - 1):
-            blk = tw.blocks[i]
-            w, wt, bias, train = self._block_weights(blk, adapters, i, need_grad)
-            trains[i] = train
-            a_cached = None
-            if i == first and cache_ctx is not None and cache_ctx["hit"]:
-                a_cached = cache_ctx["a"]
-            x_out, kept = self._full_block_fwd(tw, blk, f"vg{i}", x, B, w, bias, need_grad, keep_attention=i > first,
-                                               a_cached=a_cached)
-            if i == first and cache_ctx is not None and not cache_ctx["hit"]:
-                cache_ctx["cache"].store(cache_ctx["ids"], x, kept["a_f32"])
-            kept.update(train=train, wt=wt)
-            saved["blocks"][i] = kept
-            x = x_out
-        # ---- block Z = L-1, CLS query rows only (as in vision_head)
-        blkZ = tw.blocks[L - 1]
-        wZ, wtZ, bZ, trainZ = self._block_weights(blkZ, adapters, L - 1, need_grad)
-        keepZ = None
-        if need_grad:
-            keepZ = {"x_mid": self._keep("xmidZ", (B, d)), "x_out": self._keep("xoutZ", (B, d)),
-                     "h_pre": self._keep("hpreZ", (B, 4 * d), self._general_dtype()),
-                     "a_f32": self._keep("aZ", (B, d)), "x_in": x, "wtZ": wtZ}
+        x, blocks, below = self._live_blocks_fwd(tw, "v", x, B, adapters, need_grad, cache_ctx)
+        blk = tw.blocks[L - 1]
+        w, wt, bias, train = self._block_weights(blk, adapters, L - 1, need_grad)
+        keep = self._last_block_keep("v", B, d, train, below, x, wt)
         h = self._opbuf("v.h", M, d)
-        ops.layernorm_fwd(x, M, d, blkZ.ln1_w, blkZ.ln1_b, LN_EPS, y=h)
-        qkv = self._keep("qkvZ", (M, 3 * d), self._general_dtype()) if need_grad else self._qkv_buffer("v", M, d)
-        self._gemm_qkv(h, blkZ.w_in, blkZ.b_in, qkv, M)
+        ops.layernorm_fwd(x, M, d, blk.ln1_w, blk.ln1_b, LN_EPS, y=h)
+        qkv = self._keep("v.qkvZ", (M, 3 * d), self._act_dtype()) if below else self._qkv_buffer("v", M, d)
+        self._gemm_qkv(h, blk.w_in, blk.b_in, qkv, M)
         a_cls = self._opbuf("v.acls", max(B, 128), d)
-        ops.attention_fwd(qkv, B, T, H, first_row_only=True, out=a_cls, out_f32=keepZ["a_f32"] if keepZ else None)
-        x_cls = x.view(B, T * d)[:, :d]
-        x_out = self._rows_tail(tw, blkZ, "v", a_cls, x_cls, B, wZ, bZ, keepZ)
-        hp = self._opbuf("v.lnpost", max(B, 128), d)
-        ops.layernorm_fwd(x_out, B, d, self.ln_post[0], self.ln_post[1], LN_EPS, y=hp)
-        feat = self._keep("imgfeat", (B, self.E))
-        ops.gemm(hp, self.proj_t, B, out_f32=feat, **self._skinny("v", B, self.E, d))
-        self.launches += 4
-        saved.update(trainZ=trainZ, keepZ=keepZ, qkvZ=qkv, trains=trains)
-        return feat, saved
+        a_f32 = self._keep("v.aZ", (B, d)) if keep else None
+        ops.attention_fwd(qkv, B, T, tw.heads, first_row_only=True, out=a_cls, out_f32=a_f32)
+        x_cls = x.view(B, T * d)[:, :d]  # CLS rows of the block input, row stride T*d
+        feat = self._last_rows(tw, "v", a_cls, x_cls, B, w, bias, keep, self.ln_post, self.proj_t)
+        if keep:
+            keep.update(a_f32=a_f32, qkv=qkv)
+        return feat, {"tw": tw, "R": B, "blocks": blocks, "below": below, "trainZ": train, "keepZ": keep}
 
-    def text_features_general(self, tokens, adapters, need_grad):
-        """Text tower with more than one adapted block: blocks below the first adapted one are cached per token tensor
-        (frozen), the rest runs on all S*T rows; after the last attention only the EOT rows are kept."""
+    def _eot_attention(self, x, eot, S, qkv=None):
+        """ln_1 -> in_proj -> causal attention of the last text block on all rows, then the EOT rows of its output and
+        of its input.  -> (attention operand, attention fp32, block input), each [S, d]."""
         tw = self.txt
-        S, T = tokens.shape
-        d, H, L = tw.d, tw.heads, len(tw.blocks)
-        first = L - tw.n_live
-        M = S * T
-        key = (tokens.data_ptr(), tokens._version, S, T, "general", first)
-        cache = self._text_cache if (self.cache_text and self._text_cache
-                                     and self._text_cache["key"] == key) else None
-        if cache is None:
-            x = self._buf("t.x", (M, d))
-            ops.embed_tokens(tokens, self.tok_table, self.tpos, x)
-            self.launches += 1
-            for i in range(first):
-                blk = tw.blocks[i]
-                self._block_full(tw, blk, "t", x, x, x, S, blk.w_out, blk.b_out)
-            eot = (tokens.argmax(dim=-1) + torch.arange(S, device=tokens.device) * T).contiguous()
-            cache = {"key": key, "x_first": x, "eot": eot, "tokens": tokens}
-            if self.cache_text:
-                self._text_cache = cache
-        x, eot = cache["x_first"], cache["eot"]
-        saved = {"S": S, "general": True, "first": first, "blocks": {}, "eot": eot}
-        trains = {}
-        for i in range(first, L - 1):
-            blk = tw.blocks[i]
-            w, wt, bias, train = self._block_weights(blk, adapters, i, need_grad)
-            trains[i] = train
-            x, kept = self._full_block_fwd(tw, blk, f"tg{i}", x, S, w, bias, need_grad, keep_attention=i > first)
-            kept.update(train=train, wt=wt)
-            saved["blocks"][i] = kept
-        blkZ = tw.blocks[L - 1]
-        wZ, wtZ, bZ, trainZ = self._block_weights(blkZ, adapters, L - 1, need_grad)
-        dt = self._general_dtype()
+        M, d, blk = S * tw.T, tw.d, tw.blocks[-1]
         h = self._opbuf("t.h", M, d)
-        ops.layernorm_fwd(x, M, d, blkZ.ln1_w, blkZ.ln1_b, LN_EPS, y=h)
-        qkv = self._keep("t.qkvZ", (M, 3 * d), dt) if need_grad else self._qkv_buffer("t", M, d)
-        self._gemm_qkv(h, blkZ.w_in, blkZ.b_in, qkv, M)
+        ops.layernorm_fwd(x, M, d, blk.ln1_w, blk.ln1_b, LN_EPS, y=h)
+        if qkv is None:
+            qkv = self._qkv_buffer("t", M, d)
+        self._gemm_qkv(h, blk.w_in, blk.b_in, qkv, M)
         a_all = self._buf("t.a_f32", (M, d))
-        ops.attention_fwd(qkv, S, T, H, causal=True, out_f32=a_all)
-        a_eot = self._keep("t.a_eot_g", (S, d))
-        x_eot = self._keep("t.x_eot_g", (S, d))
+        ops.attention_fwd(qkv, S, tw.T, tw.heads, causal=True, out_f32=a_all)
+        # (persistent buffers, not fresh tensors: they are produced on the side stream and read by
+        # the backward pass on the main stream - nothing here may be recycled by the caching allocator)
+        a_eot = self._buf("t.a_eot", (S, d))
+        x_eot = self._buf("t.x_eot", (S, d))
         ops.gather_rows(a_all, eot, d, a_eot)
         ops.gather_rows(x, eot, d, x_eot)
         a_op = self._opbuf("t.a_op", max(S, 128), d, zero=True)
         ops.split_bf16(a_eot, a_op)
-        self.launches += 6
-        keepZ = None
-        if need_grad:
-            keepZ = {"x_mid": self._keep("t.xmidZ", (S, d)), "x_out": self._keep("t.xoutZ", (S, d)),
-                     "h_pre": self._keep("t.hpreZ", (S, 4 * d), dt), "a_f32": a_eot, "x_in": x, "qkv": qkv, "wtZ": wtZ}
-        x_out = self._rows_tail(tw, blkZ, "t", a_op, x_eot, S, wZ, bZ, keepZ)
-        hp = self._opbuf("t.lnfinal", max(S, 128), d)
-        ops.layernorm_fwd(x_out, S, d, self.ln_final[0], self.ln_final[1], LN_EPS, y=hp)
-        feat = self._keep("txtfeat", (S, self.E))
-        ops.gemm(hp, self.tproj_t, S, out_f32=feat, **self._skinny("t", S, self.E, d))
-        self.launches += 2
-        saved.update(trainZ=trainZ, keepZ=keepZ, trains=trains)
-        return feat, saved
+        return a_op, a_eot, x_eot
 
-    def _blocks_bwd_general(self, tw, side, saved, dx, B, grads):
-        """dx [M, d] = dL/d(output of block L-2) on entry.  Walks the live full blocks back to the first adapted one,
-        collecting dL/dW of every trainable out_proj; stops as soon as nothing trainable is left below."""
-        L, d, H = len(tw.blocks), tw.d, tw.heads
-        T = saved["T"] if side == "v" else tw.T
-        M = B * T
-        first, trains = saved["first"], saved["trains"]
-        dt = self._general_dtype()
-        for i in range(L - 2, first - 1, -1):
-            blk, kp = tw.blocks[i], saved["blocks"][i]
-            tag = f"{side}bg{i}"
-            self._mlp_rows_bwd(blk, tag, dx, M, d, kp["h_pre"], kp["x_mid"])       # dx := dL/d(out_proj output)
-            if trains[i]:
-                grads[(side, i)] = self._dw(tag, dx, kp["a_f32"], M, d, d, a_op=kp["a_op"])
-            if not any(trains[j] for j in range(first, i)):
-                break
-            g = self._grad_operand(tag + ".gy", dx, M, d)
-            d_a = self._buf(tag + ".da", (M, d), dt)       # (bf16 mode: the all-bf16 form of hba_attention_bwd)
-            if self.split:
-                ops.gemm(g, kp["wt"], M, out_f32=d_a)
-            else:
-                ops.gemm(g, kp["wt"], M, out=Operand(d_a, M, d, 0))
-            d_qkv = self._buf(tag + ".dqkv", (M, 3 * d), dt)
-            ops.attention_bwd(kp["qkv"], B, T, H, d_a, d_qkv, causal=tw.causal)
-            gq = self._grad_operand(tag + ".gq", d_qkv, M, 3 * d) if self.split else Operand(d_qkv, M, 3 * d, 0)
-            d_ln1 = self._buf(tag + ".dln1", (M, d))
-            ops.gemm(gq, blk.w_in_t, M, out_f32=d_ln1)
-            # residual: dL/dx_in = dL/d(out_proj output) + ln_1 backward of the attention branch
-            ops.layernorm_bwd(d_ln1, kp["x_in"], M, d, blk.ln1_w, LN_EPS, dx, accumulate=True)
-            self.launches += 4
+    def text_features(self, tokens, adapters, need_grad):
+        """Text tower -> (txt_feat [S, E], saved dict).  Everything frozen is cached per token tensor (the prompts never
+        change, NEW:282): blocks [0, first) and, when only the last block is live, its attention and EOT rows too.
+        Blocks [first, L-1) run on all S*T rows; after the last attention only the EOT rows are kept."""
+        tw = self.txt
+        S, T = tokens.shape
+        d, L = tw.d, len(tw.blocks)
+        first = L - tw.n_live
+        key = (tokens.data_ptr(), tokens._version, S, T, first)
+        cache = self._text_cache if (self.cache_text and self._text_cache
+                                     and self._text_cache["key"] == key) else None
+        if cache is None:
+            x = self._buf("t.x", (S * T, d))
+            ops.embed_tokens(tokens, self.tok_table, self.tpos, x)
+            self._frozen_blocks(tw, "t", x, S, first)
+            eot = (tokens.argmax(dim=-1) + torch.arange(S, device=tokens.device) * T).contiguous()
+            # (the entry keeps the token tensor alive: the key holds its ADDRESS, and the caching allocator would hand
+            # the address of a freed prompt tensor to the next model's prompts - other class names, same key)
+            cache = {"key": key, "x": x, "eot": eot, "tokens": tokens}
+            if first == L - 1:
+                cache["rows"] = self._eot_attention(x, eot, S)
+            if self.cache_text:
+                self._text_cache = cache
+        x, blocks, below = self._live_blocks_fwd(tw, "t", cache["x"], S, adapters, need_grad, keep_input=True)
+        qkv = self._keep("t.qkvZ", (S * T, 3 * d), self._act_dtype()) if below else None
+        a_op, a_eot, x_eot = cache["rows"] if "rows" in cache else self._eot_attention(x, cache["eot"], S, qkv)
+        blk = tw.blocks[L - 1]
+        w, wt, bias, train = self._block_weights(blk, adapters, L - 1, need_grad)
+        keep = self._last_block_keep("t", S, d, train, below, x, wt)
+        feat = self._last_rows(tw, "t", a_op, x_eot, S, w, bias, keep, self.ln_final, self.tproj_t)
+        if keep:
+            keep.update(a_f32=a_eot, qkv=qkv)
+        return feat, {"tw": tw, "R": S, "blocks": blocks, "below": below, "trainZ": train, "keepZ": keep,
+                      "eot": cache["eot"]}
 
     def _side_stream(self):
         st = self.__dict__.get("_side")
@@ -710,7 +520,6 @@ class Engine:
     def run_forward(self, images, tokens, pos_embedding, v_adapters, t_adapters, need_grad):
         """-> (pred [B, S] fp32 (fresh tensor), saved state for run_backward)."""
         self.ensure(images.device)
-        self.launches = 0
         self._pos_flag = bool(pos_embedding)
         tokens = tokens.reshape(-1, tokens.shape[-1])
         if tokens.dtype != torch.int64:
@@ -740,25 +549,20 @@ class Engine:
         # fill the SMs the vision tower's kernel tails leave idle, and vice versa.  Same kernels, same
         # arguments: results are unchanged.  Fork / join are stream events, so the pair is captured into a
         # CUDA graph as two parallel branches.  HBA_TEXT_STREAM=0 keeps everything on one stream.
-        general_v, general_t = self.vis.n_live > 2, self.txt.n_live > 1
-        text_fn = self.text_features_general if general_t else self.text_features
         side = None
         if os.environ.get("HBA_TEXT_STREAM", "1") != "0":
             main = torch.cuda.current_stream(self.device)
             side = self._side_stream()
             side.wait_stream(main)    # fork: the adapters' merged weights were produced on the main stream
             with torch.cuda.stream(side):
-                txt_feat, st = text_fn(tokens, t_adapters, need_grad)
+                txt_feat, st = self.text_features(tokens, t_adapters, need_grad)
         if cache_ctx is not None and cache_ctx["hit"]:
             x, tw = cache_ctx["x"], self.vis
         else:
-            x, tw = self.vision_trunk(images, max(L - max(self.vis.n_live, 2), 0))
-        if general_v:
-            img_feat, sv = self.vision_head_general(x, tw, B, v_adapters, need_grad, cache_ctx)
-        else:
-            img_feat, sv = self.vision_head(x, tw, B, v_adapters, need_grad, cache_ctx)
+            x, tw = self.vision_trunk(images, L - self.vis.n_live)
+        img_feat, sv = self.vision_head(x, tw, B, v_adapters, need_grad, cache_ctx)
         if side is None:
-            txt_feat, st = text_fn(tokens, t_adapters, need_grad)
+            txt_feat, st = self.text_features(tokens, t_adapters, need_grad)
         else:
             main.wait_stream(side)   # join: the cosine head needs both towers
         pred = torch.empty(B, txt_feat.shape[0], device=self.device)
@@ -770,7 +574,6 @@ class Engine:
             ops.cos_mse_fwd(img_feat, txt_feat, self.logit_scale, pred, B=B, target=req.target, loss=loss,
                             bad_step=req.bad_step, bad_total=req.bad_total, total=req.total,
                             workspace=self._buf("head.ws", (B + 1,), zero=True))
-        self.launches += 1
         self._gen += 1
         return pred, {"v": sv, "t": st, "img_feat": img_feat, "txt_feat": txt_feat, "gen": self._gen,
                       "loss": loss, "pred": pred.detach(), "target": req.target if req is not None else None}
@@ -784,7 +587,6 @@ class Engine:
         else:
             op = self._opbuf(name, max(rows, 128), cols)
             ops.split_bf16(g[:rows], op)
-        self.launches += 1
         return op
 
     def _mlp_rows_bwd(self, blk, tag, dxo, R, d, h_pre, x_mid):
@@ -795,7 +597,6 @@ class Engine:
         d_ln2 = self._buf(tag + ".dln2", (R, d))
         ops.gemm(gh, blk.w_fc_t, R, out_f32=d_ln2, **self._skinny(tag, R, d, 4 * d))
         ops.layernorm_bwd(d_ln2, x_mid, R, d, blk.ln2_w, LN_EPS, dxo, accumulate=True)
-        self.launches += 3
 
     def _dw(self, tag, dY, a_f32, R, d_out, d_in, a_op=None):
         """dW[out, in] = sum_r dY[r, out] a[r, in]: both operands are read MN-major (as [K = rows, M / N]
@@ -809,7 +610,6 @@ class Engine:
         ws = self._buf("b.k_ws", (s * d_out * d_in,)) if s > 1 else None
         ops.gemm(Operand(A.buf, R, d_out, A.lo_off), Operand(Bo.buf, R, d_in, Bo.lo_off), a_mn=True, b_mn=True,
                  K=R, out_f32=dW, k_slices=s, k_workspace=ws)
-        self.launches += 2 if s > 1 else 1
         return dW
 
     def run_backward(self, saved, d_pred, d_loss=None):
@@ -819,7 +619,6 @@ class Engine:
         if saved["gen"] != self._gen:
             raise RuntimeError("libhba: backward called after a newer forward pass overwrote the "
                                "saved activations (call backward before the next forward)")
-        self.launches = 0
         grads = {}
         img_feat, txt_feat = saved["img_feat"], saved["txt_feat"]
         B, S, E = img_feat.shape[0], txt_feat.shape[0], self.E
@@ -833,136 +632,84 @@ class Engine:
                 d_pred = d_pred + (2.0 / saved["pred"].numel()) * d_loss * (saved["pred"] - saved["target"])
             ops.cos_head_bwd(img_feat, txt_feat, self.logit_scale, d_img, d_txt,
                              d_pred=d_pred.contiguous().float())
-        self.launches += 1
-        # ------------------------------------------------ text: last block, EOT rows
-        st = saved["t"]
-        if st.get("general"):
-            self._text_backward_general(st, d_txt, grads)
-        elif st["trainZ"]:
-            tw = self.txt
-            d, L = tw.d, len(tw.blocks)
-            blk, kz = tw.blocks[L - 1], st["keepZ"]
-            g = self._grad_operand("tb.g0", d_txt, S, E)
-            d_lnf = self._buf("tb.dlnf", (S, d))
-            ops.gemm(g, self.tproj_n, S, out_f32=d_lnf, **self._skinny("tb", S, d, E))
-            dxo = self._buf("tb.dxo", (S, d))
-            ops.layernorm_bwd(d_lnf, kz["x_out"], S, d, self.ln_final[0], LN_EPS, dxo)
-            self.launches += 2
-            self._mlp_rows_bwd(blk, "tb", dxo, S, d, kz["h_pre"], kz["x_mid"])
-            grads[("t", L - 1)] = self._dw("tb", dxo, kz["a_f32"], S, d, d)
-        # ------------------------------------------------ vision
-        sv = saved["v"]
-        tw = sv["tw"]
-        L, d, T, H = len(tw.blocks), tw.d, sv["T"], tw.heads
-        M = B * T
-        if sv.get("general"):
-            self._vision_backward_general(sv, d_img, B, grads)
-        elif sv["trainZ"] or sv.get("trainP"):
-            blkZ, kz = tw.blocks[L - 1], sv["keepZ"]
-            g = self._grad_operand("vb.g0", d_img, B, E)
-            d_lnp = self._buf("vb.dlnp", (B, d))
-            ops.gemm(g, self.proj_n, B, out_f32=d_lnp, **self._skinny("vb", B, d, E))
-            dxo = self._buf("vb.dxo", (B, d))
-            ops.layernorm_bwd(d_lnp, kz["x_out"], B, d, self.ln_post[0], LN_EPS, dxo)
-            self.launches += 2
-            self._mlp_rows_bwd(blkZ, "vb", dxo, B, d, kz["h_pre"], kz["x_mid"])  # dxo = dY_Z
-            if sv["trainZ"]:
-                grads[("v", L - 1)] = self._dw("vb", dxo, kz["a_f32"], B, d, d)
-            if sv.get("trainP"):
-                blkP, kp = tw.blocks[L - 2], sv["keepP"]
-                wtZ = kz["wtZ"] if kz["wtZ"] is not None else self._frozen_wt(blkZ)
-                g2 = self._grad_operand("vb.g2", dxo, B, d)
-                d_a = self._buf("vb.da", (B, d))
-                ops.gemm(g2, wtZ, B, out_f32=d_a, **self._skinny("vb", B, d, d))
-                d_qkv = self._buf("vb.dqkv", (M, 3 * d))
-                ops.attention_bwd_row0(sv["qkvZ"], B, T, H, d_a, d_qkv)
-                gq = self._grad_operand("vb.gq", d_qkv, M, 3 * d)
-                d_ln1 = self._buf("vb.dln1", (M, d))
-                ops.gemm(gq, blkZ.w_in_t, M, out_f32=d_ln1)
-                dx = self._buf("vb.dx", (M, d))
-                ops.layernorm_bwd(d_ln1, kz["x_in"], M, d, blkZ.ln1_w, LN_EPS, dx)
-                ops.add_rows(dx, dxo, B, d, dst_row_step=T)  # residual path of the CLS rows
-                self.launches += 5
-                self._mlp_rows_bwd(blkP, "vbP", dx, M, d, kp["h_pre"], kp["x_mid"])  # dx = dY_P
-                grads[("v", L - 2)] = self._dw("vbP", dx, kp["a_f32"], M, d, d, a_op=kp.get("a_op"))
+        self._tower_bwd("t", saved["t"], d_txt, grads)
+        self._tower_bwd("v", saved["v"], d_img, grads)
         return grads
 
-    def _text_backward_general(self, st, d_txt, grads):
-        tw = self.txt
-        S, d, L, T, H = st["S"], tw.d, len(tw.blocks), tw.T, tw.heads
-        M = S * T
-        E = self.E
-        trains, first = st["trains"], st["first"]
-        below = any(trains[j] for j in range(first, L - 1))
-        if not (st["trainZ"] or below):
+    def _tower_bwd(self, side, s, d_feat, grads):
+        """Backward of one tower from dL/d(features): projection, final LN and MLP of the last block on its R rows (CLS
+        / EOT rows) and its out_proj dW; then, when a trainable adapter sits below, out_proj dX, the last attention's
+        backward onto all rows of its input, and the walk down the live full blocks."""
+        if not (s["trainZ"] or s["below"]):
             return
-        blk, kz = tw.blocks[L - 1], st["keepZ"]
-        g = self._grad_operand("tb.g0", d_txt, S, E)
-        d_lnf = self._buf("tb.dlnf", (S, d))
-        ops.gemm(g, self.tproj_n, S, out_f32=d_lnf, **self._skinny("tb", S, d, E))
-        dxo = self._buf("tb.dxo", (S, d))
-        ops.layernorm_bwd(d_lnf, kz["x_out"], S, d, self.ln_final[0], LN_EPS, dxo)
-        self.launches += 2
-        self._mlp_rows_bwd(blk, "tb", dxo, S, d, kz["h_pre"], kz["x_mid"])          # dxo := dL/d(out_proj output), EOT rows
-        if st["trainZ"]:
-            grads[("t", L - 1)] = self._dw("tb", dxo, kz["a_f32"], S, d, d)
-        if not below:
+        tw, R, kz = s["tw"], s["R"], s["keepZ"]
+        L, d, T, H = len(tw.blocks), tw.d, tw.T, tw.heads
+        M = R * T
+        blk, tag = tw.blocks[L - 1], side + "b"
+        ln, proj_n = (self.ln_post, self.proj_n) if side == "v" else (self.ln_final, self.tproj_n)
+        g = self._grad_operand(tag + ".g0", d_feat, R, self.E)
+        d_ln = self._buf(tag + ".dln", (R, d))
+        ops.gemm(g, proj_n, R, out_f32=d_ln, **self._skinny(tag, R, d, self.E))
+        dxo = self._buf(tag + ".dxo", (R, d))
+        ops.layernorm_bwd(d_ln, kz["x_out"], R, d, ln[0], LN_EPS, dxo)
+        self._mlp_rows_bwd(blk, tag, dxo, R, d, kz["h_pre"], kz["x_mid"])   # dxo := dL/d(out_proj output) of the rows
+        if s["trainZ"]:
+            grads[(side, L - 1)] = self._dw(tag, dxo, kz["a_f32"], R, d, d)
+        if not s["below"]:
             return
-        # below the last block: its attention saw every row of the block input
-        wtZ = kz["wtZ"] if kz["wtZ"] is not None else self._frozen_wt(blk)
-        g2 = self._grad_operand("tb.g2", dxo, S, d)
-        d_a_eot = self._buf("tb.da_eot", (S, d))
-        ops.gemm(g2, wtZ, S, out_f32=d_a_eot, **self._skinny("tb", S, d, d))
-        dt = self._general_dtype()
-        d_a = self._buf("tb.da", (M, d), dt)
-        d_a.zero_()
-        d_a.index_copy_(0, st["eot"], d_a_eot.to(dt))
-        d_qkv = self._buf("tb.dqkv", (M, 3 * d), dt)
-        ops.attention_bwd(kz["qkv"], S, T, H, d_a, d_qkv, causal=True)
-        gq = self._grad_operand("tb.gq", d_qkv, M, 3 * d) if self.split else Operand(d_qkv, M, 3 * d, 0)
-        d_ln1 = self._buf("tb.dln1", (M, d))
+        wt = kz["wt"] if kz["wt"] is not None else self._frozen_wt(blk)
+        g2 = self._grad_operand(tag + ".g2", dxo, R, d)
+        d_a = self._buf(tag + ".da", (R, d))
+        ops.gemm(g2, wt, R, out_f32=d_a, **self._skinny(tag, R, d, d))
+        if side == "v":   # only the CLS query rows were attended from
+            d_qkv = self._buf(tag + ".dqkv", (M, 3 * d))
+            ops.attention_bwd_row0(kz["qkv"], R, T, H, d_a, d_qkv)
+            gq = self._grad_operand(tag + ".gq", d_qkv, M, 3 * d)
+        else:             # the causal attention of every row, with a zero gradient outside the EOT rows
+            dt = self._act_dtype()
+            d_a_all = self._buf(tag + ".da_all", (M, d), dt)
+            d_a_all.zero_()
+            d_a_all.index_copy_(0, s["eot"], d_a.to(dt))
+            d_qkv = self._buf(tag + ".dqkv", (M, 3 * d), dt)
+            ops.attention_bwd(kz["qkv"], R, T, H, d_a_all, d_qkv, causal=True)
+            gq = self._grad_operand(tag + ".gq", d_qkv, M, 3 * d) if self.split else Operand(d_qkv, M, 3 * d, 0)
+        d_ln1 = self._buf(tag + ".dln1", (M, d))
         ops.gemm(gq, blk.w_in_t, M, out_f32=d_ln1)
-        dx = self._buf("tb.dx", (M, d))
+        dx = self._buf(tag + ".dx", (M, d))
         ops.layernorm_bwd(d_ln1, kz["x_in"], M, d, blk.ln1_w, LN_EPS, dx)
-        dx.index_add_(0, st["eot"], dxo)                                             # residual path of the EOT rows
-        self.launches += 4
-        self._blocks_bwd_general(tw, "t", st, dx, S, grads)
+        # residual path of the CLS / EOT rows
+        if side == "v":
+            ops.add_rows(dx, dxo, R, d, dst_row_step=T)
+        else:
+            dx.index_add_(0, s["eot"], dxo)
+        self._blocks_bwd(tw, side, s["blocks"], dx, R, grads)
 
-    def _vision_backward_general(self, sv, d_img, B, grads):
-        tw = sv["tw"]
-        L, d, T, H = len(tw.blocks), tw.d, sv["T"], tw.heads
+    def _blocks_bwd(self, tw, side, blocks, dx, B, grads):
+        """dx [M, d] = dL/d(output of block L-2) on entry.  Walks the live full blocks down, collecting dL/dW of every
+        trainable out_proj, and stops at the lowest trainable adapter."""
+        L, d, T, H = len(tw.blocks), tw.d, tw.T, tw.heads
         M = B * T
-        E = self.E
-        trains, first = sv["trains"], sv["first"]
-        below = any(trains[j] for j in range(first, L - 1))
-        if not (sv["trainZ"] or below):
-            return
-        blkZ, kz = tw.blocks[L - 1], sv["keepZ"]
-        g = self._grad_operand("vb.g0", d_img, B, E)
-        d_lnp = self._buf("vb.dlnp", (B, d))
-        ops.gemm(g, self.proj_n, B, out_f32=d_lnp, **self._skinny("vb", B, d, E))
-        dxo = self._buf("vb.dxo", (B, d))
-        ops.layernorm_bwd(d_lnp, kz["x_out"], B, d, self.ln_post[0], LN_EPS, dxo)
-        self.launches += 2
-        self._mlp_rows_bwd(blkZ, "vb", dxo, B, d, kz["h_pre"], kz["x_mid"])         # dxo := dL/d(out_proj output), CLS rows
-        if sv["trainZ"]:
-            grads[("v", L - 1)] = self._dw("vb", dxo, kz["a_f32"], B, d, d)
-        if not below:
-            return
-        wtZ = kz["wtZ"] if kz["wtZ"] is not None else self._frozen_wt(blkZ)
-        g2 = self._grad_operand("vb.g2", dxo, B, d)
-        d_a = self._buf("vb.da", (B, d))
-        ops.gemm(g2, wtZ, B, out_f32=d_a, **self._skinny("vb", B, d, d))
-        d_qkv = self._buf("vb.dqkv", (M, 3 * d))
-        ops.attention_bwd_row0(sv["qkvZ"], B, T, H, d_a, d_qkv)
-        gq = self._grad_operand("vb.gq", d_qkv, M, 3 * d)
-        d_ln1 = self._buf("vb.dln1", (M, d))
-        ops.gemm(gq, blkZ.w_in_t, M, out_f32=d_ln1)
-        dx = self._buf("vb.dx", (M, d))
-        ops.layernorm_bwd(d_ln1, kz["x_in"], M, d, blkZ.ln1_w, LN_EPS, dx)
-        ops.add_rows(dx, dxo, B, d, dst_row_step=T)                                   # residual path of the CLS rows
-        self.launches += 5
-        self._blocks_bwd_general(tw, "v", sv, dx, B, grads)
+        for i in range(L - 2, -1, -1):
+            blk, kp = tw.blocks[i], blocks[i]
+            tag = f"{side}bg{i}"
+            self._mlp_rows_bwd(blk, tag, dx, M, d, kp["h_pre"], kp["x_mid"])       # dx := dL/d(out_proj output)
+            if kp["train"]:
+                grads[(side, i)] = self._dw(tag, dx, None, M, d, d, a_op=kp["a_op"])
+            if not kp["below"]:
+                break
+            g = self._grad_operand(tag + ".gy", dx, M, d)
+            d_a = self._buf(tag + ".da", (M, d), self._act_dtype())   # (bf16 mode: the all-bf16 form of hba_attention_bwd)
+            if self.split:
+                ops.gemm(g, kp["wt"], M, out_f32=d_a)
+            else:
+                ops.gemm(g, kp["wt"], M, out=Operand(d_a, M, d, 0))
+            d_qkv = self._buf(tag + ".dqkv", (M, 3 * d), self._act_dtype())
+            ops.attention_bwd(kp["qkv"], B, T, H, d_a, d_qkv, causal=tw.causal)
+            gq = self._grad_operand(tag + ".gq", d_qkv, M, 3 * d) if self.split else Operand(d_qkv, M, 3 * d, 0)
+            d_ln1 = self._buf(tag + ".dln1", (M, d))
+            ops.gemm(gq, blk.w_in_t, M, out_f32=d_ln1)
+            # residual: dL/dx_in = dL/d(out_proj output) + ln_1 backward of the attention branch
+            ops.layernorm_bwd(d_ln1, kp["x_in"], M, d, blk.ln1_w, LN_EPS, dx, accumulate=True)
 
     def _frozen_wt(self, blk):
         if getattr(blk, "w_out_t", None) is not None:
@@ -972,11 +719,12 @@ class Engine:
 
 
 class TrunkCache:
-    """HBM cache of the frozen vision trunk per image: the input of block L-2 and that block's
-    attention output (ln_1 -> in_proj -> attention is frozen-on-frozen there), both fp32.
+    """HBM cache of the frozen vision trunk per image: the input of the first live block (`first`, L-2 in the
+    reference drivers' placement) and that block's attention output (ln_1 -> in_proj -> attention is
+    frozen-on-frozen there), both fp32.
 
-    Exactness: train images are never augmented (NEW:183-188) and blocks 0..L-3 plus the attention
-    half of block L-2 hold no trainable parameter (NEW:665-669), so for an un-perturbed image these
+    Exactness: train images are never augmented (NEW:183-188) and blocks below `first` plus the attention
+    half of block `first` hold no trainable parameter (NEW:665-669), so for an un-perturbed image these
     activations are identical in every epoch; the cached path runs the same kernels on the same
     values and is bit-identical to recomputation.  Callers must not pass ids for perturbed images
     (`image_noise`, `uniform_images` windows, NEW:880-916)."""
