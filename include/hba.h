@@ -319,7 +319,9 @@ int hba_softmax_ce_fwd_bwd(const float* logits, int64_t ld, const int64_t* label
  * hba_layernorm_param_grad: dgamma_dbeta[0:cols] (+)= sum_r dy * xhat, [cols:2cols] (+)= sum_r dy;
  *   workspace >= 2*rows + 256*cols floats.
  * hba_attention_bwd: full softmax-attention backward, d_out [B*T, H*64] -> d_qkv [B*T, 3*H*64]
- *   (dtypes HBA_DT_*: (bf16, bf16|f32, bf16) or (f32, f32, f32)).
+ *   (dtypes HBA_DT_*: (bf16, bf16|f32, bf16) or (f32, f32, f32); with bf16 qkv an f32 d_out is rounded to
+ *   bf16 on load, like qkv); T <= 288, and T <= 203 with f32 qkv
+ *   (its tiles must fit 227 KB of shared memory); HBA_ERR_ARG otherwise.
  */
 int hba_colsum(const void* x, int32_t dtype, int64_t rows, int32_t cols, int64_t ld, float* out,
                int32_t accumulate, float* workspace, void* stream);

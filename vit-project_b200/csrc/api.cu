@@ -113,6 +113,38 @@ int make_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t 
   return HBA_OK;
 }
 
+// 3-D bf16 tensor [batch, rows, cols] (row stride ld elements, batch stride rows * ld) with box
+// [1, box_rows, 64 cols]: a box that starts inside one batch entry and runs past its last row reads
+// zeros there, never the next entry's first rows.
+int make_tma_3d_bf16(CUtensorMap* map, const void* ptr, uint64_t batch, uint64_t rows, uint64_t cols,
+                     uint64_t ld, uint32_t box_rows, uint32_t box_cols) {
+  EncodeTiledFn fn = get_encode_fn();
+  if (!fn) {
+    set_error("cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
+    return HBA_ERR_CUDA;
+  }
+  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0 || (ld * 2) % 16 != 0) {
+    set_error("TMA operand must be 16-byte aligned with a 16-byte multiple row pitch (ptr=%p ld=%llu)",
+              ptr, (unsigned long long)ld);
+    return HBA_ERR_ARG;
+  }
+  cuuint64_t gdim[3] = {cols, rows, batch};
+  cuuint64_t gstr[2] = {ld * 2, rows * ld * 2};
+  cuuint32_t box[3] = {box_cols, box_rows, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), gdim, gstr, box,
+                  estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  box_cols * 2 == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled failed with CUresult %d (batch=%llu rows=%llu cols=%llu ld=%llu box=%ux%u)",
+              (int)r, (unsigned long long)batch, (unsigned long long)rows, (unsigned long long)cols,
+              (unsigned long long)ld, box_rows, box_cols);
+    return HBA_ERR_CUDA;
+  }
+  return HBA_OK;
+}
+
 }  // namespace hba
 
 extern "C" {

@@ -4,7 +4,7 @@
 //
 // Persistent kernel, one CTA per SM, looping over (sequence, head) units.  The unit's Q, K, V and dO
 // rows are fetched by TMA out of the packed [B*T, 3*H*64] QKV activation and the [B*T, H*64] output
-// gradient.  Keys are the TMEM lanes (one thread per key), queries the TMEM columns, so the two
+// gradient, both addressed as [B, T, cols] so that rows past a sequence's end read as zero.  Keys are the TMEM lanes (one thread per key), queries the TMEM columns, so the two
 // "transposed" products dV = P^T dO and dK = dS^T Q take their A operand straight from tensor memory:
 //
 //   per key tile t (128 keys) and query half h (<= 128 queries):
@@ -190,21 +190,20 @@ __global__ void __launch_bounds__(kThreads, 1)
     for (int n = 0; n < my_units; ++n) {
       const int u = blockIdx.x + n * gridDim.x;
       const int b = u / g.H, h = u % g.H;
-      const int row0 = b * g.T;
       // every UMMA of the previous unit has read shared memory (and so have the compute warps, which
       // arrive on p_full after their last generic-proxy reads)
       if (n > 0) mbar_wait(in_empty, (uint32_t)((n - 1) & 1));
       if (elect_one()) {
         mbar_arrive_expect_tx(in_full, bytes);
-        tma_load_2d(sQ, &tma_qkv0, in_full, h * kHd, row0);
-        tma_load_2d(sK, &tma_qkv0, in_full, d + h * kHd, row0);
-        tma_load_2d(sV, &tma_qkv0, in_full, 2 * d + h * kHd, row0);
-        tma_load_2d(sDO, &tma_do0, in_full, h * kHd, row0);
+        tma_load_3d(sQ, &tma_qkv0, in_full, h * kHd, 0, b);
+        tma_load_3d(sK, &tma_qkv0, in_full, d + h * kHd, 0, b);
+        tma_load_3d(sV, &tma_qkv0, in_full, 2 * d + h * kHd, 0, b);
+        tma_load_3d(sDO, &tma_do0, in_full, h * kHd, 0, b);
         if (rows1 > 0) {
-          tma_load_2d(sQ + 128 * kRowBytes, &tma_qkv1, in_full, h * kHd, row0 + 128);
-          tma_load_2d(sK + 128 * kRowBytes, &tma_qkv1, in_full, d + h * kHd, row0 + 128);
-          tma_load_2d(sV + 128 * kRowBytes, &tma_qkv1, in_full, 2 * d + h * kHd, row0 + 128);
-          tma_load_2d(sDO + 128 * kRowBytes, &tma_do1, in_full, h * kHd, row0 + 128);
+          tma_load_3d(sQ + 128 * kRowBytes, &tma_qkv1, in_full, h * kHd, 128, b);
+          tma_load_3d(sK + 128 * kRowBytes, &tma_qkv1, in_full, d + h * kHd, 128, b);
+          tma_load_3d(sV + 128 * kRowBytes, &tma_qkv1, in_full, 2 * d + h * kHd, 128, b);
+          tma_load_3d(sDO + 128 * kRowBytes, &tma_do1, in_full, h * kHd, 128, b);
         }
       }
       __syncwarp();
@@ -431,12 +430,13 @@ int attention_bwd_tc_launch(const __nv_bfloat16* qkv, int64_t ld_qkv, int B, int
   g.o = o, g.ld_o = ld_o, g.lse = lse, g.d_qkv = d_qkv, g.ld_dqkv = ld_dqkv;
   const uint32_t rows0 = g.rows < 128 ? g.rows : 128;
   const uint32_t rows1 = g.rows > 128 ? g.rows - 128 : 16;  // (unused map when there is one tile)
+  // [B, T, cols] maps: rows >= T of a sequence (the boxes are T rounded up to 16) read as zero, not as the
+  // next sequence's first rows, whose non-finite values would survive the P / dS = 0 masking
   CUtensorMap q0, q1, d0, d1;
-  const uint64_t nrows = (uint64_t)B * T;
-  HBA_CHECK(make_tma_2d_bf16(&q0, qkv, nrows, (uint64_t)3 * H * kHd, ld_qkv, rows0, 64));
-  HBA_CHECK(make_tma_2d_bf16(&q1, qkv, nrows, (uint64_t)3 * H * kHd, ld_qkv, rows1, 64));
-  HBA_CHECK(make_tma_2d_bf16(&d0, d_out, nrows, (uint64_t)H * kHd, ld_do, rows0, 64));
-  HBA_CHECK(make_tma_2d_bf16(&d1, d_out, nrows, (uint64_t)H * kHd, ld_do, rows1, 64));
+  HBA_CHECK(make_tma_3d_bf16(&q0, qkv, B, T, (uint64_t)3 * H * kHd, ld_qkv, rows0, 64));
+  HBA_CHECK(make_tma_3d_bf16(&q1, qkv, B, T, (uint64_t)3 * H * kHd, ld_qkv, rows1, 64));
+  HBA_CHECK(make_tma_3d_bf16(&d0, d_out, B, T, (uint64_t)H * kHd, ld_do, rows0, 64));
+  HBA_CHECK(make_tma_3d_bf16(&d1, d_out, B, T, (uint64_t)H * kHd, ld_do, rows1, 64));
   int ctas = num_sms();
   if (g.n_units < ctas) ctas = g.n_units;
   attention_bwd_tc_kernel<<<ctas, kThreads, kSmemBytes, stream>>>(q0, q1, d0, d1, g);

@@ -3,8 +3,8 @@
 //
 // Persistent kernel, one CTA per SM, looping over (sequence, head) units; a unit is one or two
 // 128-row query tiles ("items").  Everything a unit needs (its Q tiles and all K / V rows) is fetched
-// by TMA straight out of the packed [B*T, 3*H*64] bf16 QKV activation into one of two shared-memory
-// buffers, so the loads of unit u+1 overlap the math of unit u.
+// by TMA straight out of the packed [B*T, 3*H*64] bf16 QKV activation (addressed as [B, T, 3*H*64], so
+// that rows past a sequence's end read as zero) into one of two shared-memory buffers, so the loads of unit u+1 overlap the math of unit u.
 //
 //   S = Q K^T   UMMA 128 x NK x 64 (A, B from smem, SWIZZLE_128B K-major), fp32 in TMEM
 //   softmax     one thread per query row: tcgen05.ld S, max, exp2 on the SFU, P packed to bf16 and
@@ -196,7 +196,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
     for (int n = 0; n < my_units; ++n) {
       const int u = blockIdx.x + n * gridDim.x;
       const int b = u / g.H, h = u % g.H;
-      const int row0 = b * g.T;
       const int buf = n & 1;
       mbar_wait(&kv_empty[buf], ((n >> 1) & 1) ^ 1);
       if (elect_one()) {
@@ -205,15 +204,15 @@ __global__ void __launch_bounds__(kTcThreads, 1)
         uint8_t* sV = sK + kTcKVBytes;
         mbar_arrive_expect_tx(&kv_full[buf], bytes);
         for (int t = 0; t < g.n_tiles; ++t)
-          tma_load_2d(sQ + t * kTcQBytes, &tma128, &kv_full[buf], h * kTcHd, row0 + t * 128);
+          tma_load_3d(sQ + t * kTcQBytes, &tma128, &kv_full[buf], h * kTcHd, t * 128, b);
         for (int i = 0; i < full; ++i) {
-          tma_load_2d(sK + i * kTcQBytes, &tma128, &kv_full[buf], d + h * kTcHd, row0 + i * 128);
-          tma_load_2d(sV + i * kTcQBytes, &tma128, &kv_full[buf], 2 * d + h * kTcHd, row0 + i * 128);
+          tma_load_3d(sK + i * kTcQBytes, &tma128, &kv_full[buf], d + h * kTcHd, i * 128, b);
+          tma_load_3d(sV + i * kTcQBytes, &tma128, &kv_full[buf], 2 * d + h * kTcHd, i * 128, b);
         }
         for (int i = 0; i < tail; ++i) {
           const int r = full * 128 + i * 16;
-          tma_load_2d(sK + r * kTcRowBytes, &tma16, &kv_full[buf], d + h * kTcHd, row0 + r);
-          tma_load_2d(sV + r * kTcRowBytes, &tma16, &kv_full[buf], 2 * d + h * kTcHd, row0 + r);
+          tma_load_3d(sK + r * kTcRowBytes, &tma16, &kv_full[buf], d + h * kTcHd, r, b);
+          tma_load_3d(sV + r * kTcRowBytes, &tma16, &kv_full[buf], 2 * d + h * kTcHd, r, b);
         }
       }
       __syncwarp();
@@ -568,10 +567,12 @@ int attention_tc_launch(const __nv_bfloat16* qkv, int64_t ld_qkv, int B, int T, 
   g.qkv = qkv, g.ld_qkv = ld_qkv;
   g.trace = g_attn_trace;
   g.lse = lse;
+  // [B, T, 3*H*64] maps: the row boxes are rounded up to 16 / 128 rows, and rows >= T of a sequence read
+  // as zero instead of the next sequence's (non-finite values there must not reach P = 0 x K / V)
   CUtensorMap t128, t16;
-  const uint64_t rows = (uint64_t)B * T, cols = (uint64_t)3 * H * kTcHd;
-  HBA_CHECK(make_tma_2d_bf16(&t128, qkv, rows, cols, ld_qkv, 128, 64));
-  HBA_CHECK(make_tma_2d_bf16(&t16, qkv, rows, cols, ld_qkv, 16, 64));
+  const uint64_t cols = (uint64_t)3 * H * kTcHd;
+  HBA_CHECK(make_tma_3d_bf16(&t128, qkv, B, T, cols, ld_qkv, 128, 64));
+  HBA_CHECK(make_tma_3d_bf16(&t16, qkv, B, T, cols, ld_qkv, 16, 64));
   int ctas = num_sms();
   if (g.n_units < ctas) ctas = g.n_units;
   cudaError_t e = launch_pdl(attention_tc_kernel, dim3(ctas), dim3(kTcThreads), kTcSmemBytes, stream, t128, t16, g);

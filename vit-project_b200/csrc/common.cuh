@@ -63,6 +63,9 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 // 2-D bf16 row-major tensor map, box = [box_rows, box_cols]; 64-column boxes use SWIZZLE_128B
 int make_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld,
                      uint32_t box_rows, uint32_t box_cols);
+// [batch, rows, cols] bf16 with box [1, box_rows, box_cols]: rows past the end of a batch entry read as zero
+int make_tma_3d_bf16(CUtensorMap* map, const void* ptr, uint64_t batch, uint64_t rows, uint64_t cols,
+                     uint64_t ld, uint32_t box_rows, uint32_t box_cols);
 
 #define HBA_CHECK(expr)                  \
   do {                                   \
@@ -172,6 +175,15 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* m, uin
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
       "%4}], [%2];" ::"r"(smem_u32(dst)),
       "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+      : "memory");
+}
+
+__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0,
+                                            int c1, int c2) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
+      "%4, %5}], [%2];" ::"r"(smem_u32(dst)),
+      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
 

@@ -262,6 +262,7 @@ __device__ __forceinline__ void stpair(uint32_t* row, int w, float a, float b) {
 constexpr int kAbWarps = 8;
 constexpr int kAbMaxT = 288;
 constexpr int kAbChunks = kAbMaxT / 32;
+constexpr int kAbMaxSmem = 227 * 1024;  // dynamic shared memory of one CTA
 
 template <bool F32>
 __device__ __forceinline__ float dot64(const uint32_t* __restrict__ a, const uint32_t* __restrict__ b) {
@@ -401,6 +402,8 @@ static int launch_attention_bwd(const void* qkv, int64_t ld_qkv, int B, int T, i
                                 cudaStream_t s) {
   const size_t smem = sizeof(uint32_t) * 4 * (size_t)T * AbSt<sizeof(TI) == 4>::pitch + sizeof(float) * 3 * (size_t)T +
                       sizeof(float) * kAbWarps * 2 * kAbMaxT;
+  HBA_REQUIRE(smem <= kAbMaxSmem, "hba_attention_bwd: T=%d needs %zu bytes of shared memory (max %d; fp32 qkv: T <= 203)",
+              T, smem, kAbMaxSmem);
   static SmemAttr attr;
   HBA_CHECK(ensure_dyn_smem(attention_bwd_kernel<TI, TG, TO>, smem, attr, "attention_bwd_kernel"));
   attention_bwd_kernel<TI, TG, TO><<<B * H, kAbWarps * 32, smem, s>>>(
