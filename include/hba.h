@@ -40,10 +40,13 @@ int hba_device_check(void);
  * timm ViT-B/16 linears of VIT:138-140.
  *   A, B are bf16, K-major (row-major [rows, ld]) by default; lda/ldb % 8 == 0.  With a_mn_major /
  *   b_mn_major the operand is stored [K, M] / [K, N] instead (MN-major UMMA descriptors), which gives
- *   dW = dY^T X and dX = dY W without any transposed copy.  K % 64 == 0 unless nsplit == 1.
+ *   dW = dY^T X and dX = dY W without any transposed copy.  Any K > 0: TMA zero-fills a ragged last
+ *   k-block past K, except where the hi part of a K-major fp32-mode operand lies inside the tensor map - that
+ *   hi part must be zero in columns [K, ceil64(K)), and its lo offset at least ceil64(K).
  *   nsplit == 1: plain bf16 product.
  *   nsplit == 3: "fp32 mode" — A and B each hold a hi part at column 0 and a lo part at column
- *     offset a_lo_off / b_lo_off (x ~= hi + lo, both bf16); the kernel accumulates
+ *     offset a_lo_off / b_lo_off (x ~= hi + lo, both bf16; the offset is at least ceil64(K) for a
+ *     K-major operand, at least M resp. N for an MN-major one); the kernel accumulates
  *     hi.hi + lo.hi + hi.lo in fp32 (error ~2^-16 relative per product).
  * Epilogue, applied per element v = alpha * acc (+ bias[n]):
  *   pre_out (optional) receives v (the pre-activation, for the backward pass)
@@ -78,7 +81,8 @@ typedef struct hba_gemm_params {
   const float* residual; /* [M, ldr] fp32 or NULL */
   int32_t ldr;
   int32_t act;
-  const void* aux; /* [M, ld_aux] pre-activation for *_GRAD */
+  const void* aux; /* [M, ld_aux] pre-activation for *_GRAD; with ld_aux % 4 == 0 16-byte (f32) / 8-byte (bf16)
+                      aligned */
   int32_t ld_aux;
   int32_t aux_dtype; /* HBA_DT_* */
   void* pre_out;     /* [M, ld_pre] or NULL */
@@ -100,8 +104,9 @@ typedef struct hba_gemm_params {
                          out_f32, out_bf16 hi / lo).  Needs k_workspace, N % 4 == 0, no transpose_out / colsum */
   float* k_workspace; /* >= k_slices * M * N floats, 16-byte aligned */
   float* colsum_partial; /* or NULL: [ceil(M / 32), N] fp32 receiving, per 32-row group, the column sums
-                            of the bf16 output (hi part) - the bias gradient of the previous Linear fused
-                            into the GEMM that produces its dY (VIT:143); sum the groups with hba_colsum */
+                            of the bf16 output's hi part (in fp32 mode too: the lo part is not summed) - the
+                            bias gradient of the previous Linear fused into the GEMM that produces its dY
+                            (VIT:143); sum the groups with hba_colsum */
 } hba_gemm_params;
 
 int hba_gemm_bf16(const hba_gemm_params* p, void* stream);

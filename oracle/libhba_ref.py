@@ -86,8 +86,8 @@ def _act(v, act, aux):
         return v
     if act == 1:                                   # QuickGELU: x * sigmoid(1.702 x)
         return v * torch.sigmoid(1.702 * v)
-    if act == 2:                                   # erf-GELU
-        return torch.nn.functional.gelu(v)
+    if act == 2:                                   # erf-GELU (torch's fp32 CPU gelu is off by ~1e-3 near -3.5)
+        return torch.nn.functional.gelu(v.double()).to(v.dtype)
     a = aux.float()
     if act == 3:                                   # v * QuickGELU'(aux)
         s = torch.sigmoid(1.702 * a)
@@ -171,6 +171,8 @@ class RefLib:
         _require(0 <= p.act <= 4, "bad act")
         if p.act in (3, 4):
             _require(p.aux, "activation gradient needs aux")
+            _require(p.ld_aux % 4 != 0 or _al(p.aux, 16 if p.aux_dtype == 0 else 8),
+                     "aux with ld % 4 == 0 must be 16-byte (f32) / 8-byte (bf16) aligned")
         if p.transpose_out:
             _require(p.act == 0 and not p.residual and not p.pre_out, "transpose_out supports alpha and bias only")
         else:

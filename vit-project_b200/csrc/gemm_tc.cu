@@ -240,6 +240,9 @@ __device__ __forceinline__ void epilogue_chunk_coalesced(const GemmArgs& g, floa
   const int col = col0 + 4 * cq;
   const int nvalid = g.N - col;  // >= 4: the whole float4 is in range
   const bool vec = nvalid >= 4;
+  // lanes that take the vector path: in a chunk that N cuts (N % 16 != 0) the lanes of the columns past N
+  // do not, and the column-sum shuffles below must name only the lanes that execute them
+  const unsigned vec_lanes = g.colsum ? __ballot_sync(0xffffffffu, vec) : 0u;
   constexpr bool kGrad = (ACT == HBA_ACT_QUICKGELU_GRAD || ACT == HBA_ACT_GELU_ERF_GRAD);
   // loads that do not depend on the accumulator are issued first (they overlap the transposition)
   Vec4 bias = {{0.f, 0.f, 0.f, 0.f}};
@@ -351,11 +354,11 @@ __device__ __forceinline__ void epilogue_chunk_coalesced(const GemmArgs& g, floa
         }
       }
 #pragma unroll
-      for (int o = LPR; o < 32; o <<= 1) {
-        s0 += __shfl_xor_sync(0xffffffffu, s0, o);
-        s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-        s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-        s3 += __shfl_xor_sync(0xffffffffu, s3, o);
+      for (int o = LPR; o < 32; o <<= 1) {   // (lane ^ o keeps the column granule cq: vec_lanes holds both)
+        s0 += __shfl_xor_sync(vec_lanes, s0, o);
+        s1 += __shfl_xor_sync(vec_lanes, s1, o);
+        s2 += __shfl_xor_sync(vec_lanes, s2, o);
+        s3 += __shfl_xor_sync(vec_lanes, s3, o);
       }
       if (rsub == 0)
         *reinterpret_cast<float4*>(g.colsum + (size_t)(row0 >> 5) * g.N + col) = make_float4(s0, s1, s2, s3);
@@ -904,8 +907,12 @@ extern "C" int hba_gemm_bf16(const hba_gemm_params* p, void* stream) {
                 "hba_gemm_bf16: lo offsets must lie behind the hi part and be multiples of 8");
   HBA_REQUIRE(p->out_f32 || p->out_bf16 || p->pre_out, "hba_gemm_bf16: no output");
   HBA_REQUIRE(p->act >= HBA_ACT_NONE && p->act <= HBA_ACT_GELU_ERF_GRAD, "hba_gemm_bf16: bad act");
-  if (p->act == HBA_ACT_QUICKGELU_GRAD || p->act == HBA_ACT_GELU_ERF_GRAD)
+  if (p->act == HBA_ACT_QUICKGELU_GRAD || p->act == HBA_ACT_GELU_ERF_GRAD) {
     HBA_REQUIRE(p->aux != nullptr, "hba_gemm_bf16: activation gradient needs aux");
+    // with ld_aux % 4 == 0 the epilogue loads aux four elements at a time (float4 / 8-byte bf16 vectors)
+    HBA_REQUIRE(p->ld_aux % 4 != 0 || ((uintptr_t)p->aux & (p->aux_dtype == HBA_DT_F32 ? 15 : 7)) == 0,
+                "hba_gemm_bf16: aux with ld %% 4 == 0 must be 16-byte (f32) / 8-byte (bf16) aligned");
+  }
   if (p->transpose_out)
     HBA_REQUIRE(p->act == HBA_ACT_NONE && !p->residual && !p->pre_out,
                 "hba_gemm_bf16: transpose_out supports alpha and bias only");
