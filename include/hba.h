@@ -57,7 +57,7 @@ int hba_device_check(void);
  *   transpose_out != 0 writes the outputs as [N, M] (ld* are then row strides of that layout);
  *     only alpha and bias apply in that mode (no act / residual / pre_out)
  * Scheduling (no effect on results): persistent CTA pairs, 256 x 256 tiles; the tiles of a partial last round are
- * cut into 2 or 4 column slabs (HBA_GEMM_TAIL_SPLIT=0 disables), every element still accumulates its K products
+ * cut into 2 or 4 column slabs when that shortens the round; every element still accumulates its K products
  * in the same order, so the output bits do not depend on M, on max_ctas or on the split.
  */
 enum {

@@ -70,7 +70,7 @@ def act_slope(act, z, aux=None):
 
 def sfu_error(act, z, aux=None):
     """Bound on the error of the kernel's fp32 / SFU evaluation of the activation at an exact argument
-    (gemm_tc.cu:94-133), absolute, per element.
+    (gemm_tc.cu:78-115), absolute, per element.
       QuickGELU  v / (1 + ex2(-1.702 log2e v)): ex2.approx 2 ulp, __fdividef 2 ulp, and the rounded argument
                  moves exp by u |1.702 v| relative -> |v| (2^-20 + 1.702 |v| u).
       GELU       relu(v) - |v| h(|v|), h = 0.5 erfc: Abramowitz-Stegun 7.1.26 is good to 1.5e-7 in erf, 7.5e-8 in h;
@@ -170,33 +170,31 @@ def bound(ref, tau_, act=NONE, out="f32", bias=None, residual=None, alpha=1.0, p
 
 
 # ---------------------------------------------------------------------------------------- branch map
-def k_stages(BN, cg=2):
-    """GemmCfg<BN, CG>::kStages (gemm_tc.cu:45): smem ring stages of 16 KB of A plus (BN / CG) x 64 of B."""
-    return min(8, (192 * 1024) // (BM * BK * 2 + (BN // cg) * BK * 2))
+def k_stages(BN):
+    """GemmCfg<BN>::kStages (gemm_tc.cu:42): smem ring stages of 16 KB of A plus (BN / 2) x 64 of B."""
+    return min(8, (192 * 1024) // (BM * BK * 2 + (BN // 2) * BK * 2))
 
 
-def branches(M, N, K, nsplit=1, a_mn=False, b_mn=False, k_slices=1, max_ctas=0, num_sms=NUM_SMS, tail_split=True,
-             cta_group=2):
+def branches(M, N, K, nsplit=1, a_mn=False, b_mn=False, k_slices=1, max_ctas=0, num_sms=NUM_SMS):
     """What hba_gemm_bf16 / launch_gemm do with a problem (gemm_tc.cu line numbers)."""
-    BN = 256 if N >= 256 else 128                                   # :978 `wide`
-    TM = BM * cta_group
-    kblocks = -(-K // BK)                                            # :942
-    slices = min(max(k_slices, 1), kblocks)                          # :943-944
+    BN = 256 if N >= 256 else 128                                   # :903 `wide`
+    TM = 2 * BM                                                      # a CTA pair's tile rows
+    kblocks = -(-K // BK)                                            # :875
+    slices = min(max(k_slices, 1), kblocks)                          # :876-877
     kb_per = kblocks
-    if slices > 1:                                                   # :951-953 every slice owns >= 1 k-block
+    if slices > 1:                                                   # :884-886 every slice owns >= 1 k-block
         kb_per = -(-kblocks // slices)
         slices = -(-kblocks // kb_per)
     last_slice_kb = kblocks - (slices - 1) * kb_per
     m_tiles, n_tiles = -(-M // TM), -(-N // BN)
-    tiles = m_tiles * n_tiles                                        # :836
-    workers = num_sms // cta_group                                   # :837-839
-    if max_ctas > 0 and max_ctas // cta_group < workers:
-        workers = max(max_ctas // cta_group, 1)
+    tiles = m_tiles * n_tiles                                        # :770
+    workers = num_sms // 2                                           # :771-773
+    if max_ctas > 0 and max_ctas // 2 < workers:
+        workers = max(max_ctas // 2, 1)
     if tiles * slices < workers:
         workers = tiles * slices
-    f, tail_first = 1, tiles                                         # :844-861 tail split
-    if (BN == 256 and cta_group == 2 and slices == 1 and not a_mn and not b_mn and tail_split and tiles > workers
-            and tiles % workers):
+    f, tail_first = 1, tiles                                         # :778-794 tail split
+    if BN == 256 and slices == 1 and not a_mn and not b_mn and tiles > workers and tiles % workers:
         rem = tiles % workers
         cost2 = -(-(rem * 2) // workers) * 0.75
         cost4 = -(-(rem * 4) // workers) * 0.65
@@ -206,7 +204,7 @@ def branches(M, N, K, nsplit=1, a_mn=False, b_mn=False, k_slices=1, max_ctas=0, 
             f = 4
         if f > 1:
             tail_first = tiles - rem
-    items = tail_first + (tiles - tail_first) * f if f > 1 else tiles * slices   # :502-503
+    items = tail_first + (tiles - tail_first) * f if f > 1 else tiles * slices   # :475-476
     per_worker = -(-items // workers)
     slab_past_n = any((t % n_tiles) * BN + s * (BN // f) >= N for t in range(tail_first, tiles) for s in range(f))
     m_rem = M % TM
@@ -215,9 +213,9 @@ def branches(M, N, K, nsplit=1, a_mn=False, b_mn=False, k_slices=1, max_ctas=0, 
         "rounds": per_worker, "acc_reuse": per_worker > 2,
         "tail_f": f, "tail_first": tail_first, "slab_past_n": slab_past_n,
         "kblocks": kblocks, "k_ragged": K % BK != 0,
-        "kiters_min": last_slice_kb * nsplit, "kiters_lt_stages": last_slice_kb * nsplit < k_stages(BN, cta_group),
+        "kiters_min": last_slice_kb * nsplit, "kiters_lt_stages": last_slice_kb * nsplit < k_stages(BN),
         "slices": slices, "kb_per_slice": kb_per, "short_last_slice": slices > 1 and last_slice_kb < kb_per,
-        "m_tail": "none" if m_rem == 0 else ("peer_empty" if cta_group == 2 and m_rem <= BM else "peer_partial"),
+        "m_tail": "none" if m_rem == 0 else ("peer_empty" if m_rem <= BM else "peer_partial"),
         "m_warp_partial": M % 32 != 0,
         "n_mod_bn": N % BN, "n_mod16": N % 16, "n_mod4": N % 4,
     }

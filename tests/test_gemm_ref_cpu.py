@@ -156,10 +156,8 @@ def test_branch_map_hand_cases():
     assert (b["slices"], b["kb_per_slice"], b["kiters_min"], b["short_last_slice"]) == (3, 3, 1, True)
     assert branches(66, 768, 100, k_slices=8)["slices"] == 2        # no more slices than k-blocks
     assert branches(64, 64, 64, k_slices=8)["slices"] == 1
-    # MN-major operands, split-K and the single-CTA variant never split the tail
+    # MN-major operands and split-K never split the tail
     assert branches(8224, 3072, 1024, a_mn=True)["tail_f"] == 1
-    assert branches(8224, 3072, 1024, cta_group=1)["tail_f"] == 1
-    assert branches(8224, 3072, 1024, tail_split=False)["tail_f"] == 1
     # BN, stages, M tails
     assert branches(100, 255, 64)["BN"] == 128 and branches(100, 256, 64)["BN"] == 256
     assert branches(100, 512, 5 * 64)["kiters_lt_stages"] and not branches(100, 512, 6 * 64)["kiters_lt_stages"]
@@ -215,13 +213,12 @@ def test_epilogue_schedules_reach_every_scheduling_form():
 
 def test_gpu_test_file_dry_runs_on_the_cpu_restatement():
     """tests/test_gpu_gemm_shapes.py itself, run by pytest on the CPU with libhba served by its restatement; left
-    out: the production shapes (fp64 references of up to 50432 x 3072 x 768 are minutes of CPU time), the child
-    processes of the environment knobs (they load the device library), and what the restatement does not restate:
-    that the device reads the hi part's padding (the restatement reads [0, K) only) and bit-exact row slices or
-    repeats (its torch matmul picks kernels by shape)."""
+    out: the production shapes (fp64 references of up to 50432 x 3072 x 768 are minutes of CPU time) and what the
+    restatement does not restate: that the device reads the hi part's padding (the restatement reads [0, K) only)
+    and bit-exact row slices or repeats (its torch matmul picks kernels by shape)."""
     tool = os.path.join(ROOT, "tests", "emulate_clip_gpu_tests.py")
     out = subprocess.run([sys.executable, tool, os.path.join(ROOT, "tests", "test_gpu_gemm_shapes.py"), "-k",
-                          "not production and not env_knobs and not zero_padded_hi and not repeated and not row_slices"],
+                          "not production and not zero_padded_hi and not repeated and not row_slices"],
                          capture_output=True, text=True, timeout=3000, env=dict(os.environ, OMP_NUM_THREADS="8"))
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
     tail = [l for l in out.stdout.splitlines() if " passed" in l][-1]

@@ -3,7 +3,7 @@ ViT-B/16 at batch 256 (M = 50432): TFLOP/s per shape from CUDA events on the lau
 sampled by nvidia-smi during each shape's timed loop, and (yardstick only, never the product path)
 torch.matmul / cuBLAS on the same shape under the same conditions.
 
-    python tools/bench_gemm.py [--seconds 1.0]        (HBA_GEMM_CTA_GROUP=1 for the single-CTA variant)
+    python tools/bench_gemm.py [--seconds 1.0]
 """
 import argparse
 import json
@@ -84,8 +84,7 @@ def main():
     if a.only:
         shapes = [s for s in shapes if s[0] in a.only.split(",")]
     clk = Clock()
-    out = {"cta_group": os.environ.get("HBA_GEMM_CTA_GROUP", "2"), "debug": os.environ.get("HBA_GEMM_DEBUG", "0"),
-           "split": sp, "shapes": {}}
+    out = {"split": sp, "shapes": {}}
     for name, M, N, K, kind in shapes:
         A = Operand.empty(M, K, sp, dev)
         B = Operand.empty(N, K, sp, dev)

@@ -3,8 +3,6 @@
 #include <cstdio>
 #include <mutex>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace hba {
@@ -73,17 +71,6 @@ static EncodeTiledFn get_encode_fn() {
 
 // 2-D bf16 row-major tensor [rows, cols] with row stride ld (elements); box = [box_rows, 64 cols]
 // (64 bf16 = 128 B = one SWIZZLE_128B atom row).  Out-of-bounds elements read as zero.
-bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    // opt-in: measured on the CLIP-HBA step (30 steps, A/B on one box, twice): 8.04 / 7.99 ms with, 8.03 / 8.00 ms
-    // without - the launch gap it hides is not where the step's time goes
-    const char* e = getenv("HBA_PDL");
-    on = (e && e[0] == '1') ? 1 : 0;
-  }
-  return on == 1;
-}
-
 int make_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld,
                      uint32_t box_rows, uint32_t box_cols) {
   EncodeTiledFn fn = get_encode_fn();

@@ -134,13 +134,7 @@ struct AttnTcArgs {
   const __nv_bfloat16* qkv;
   int64_t ld_qkv;
   float* lse;        // optional [B, H, T]: log2-domain log-sum-exp per row (P = 2^(s*scale - lse)), for the backward
-  long long* trace;  // debug: per-item phase time stamps of CTA 0 (hba_debug_attention_trace), else null
 };
-
-#define HBA_TRACE(item, slot)                                                        \
-  do {                                                                             \
-    if (g.trace && blockIdx.x == 0 && lane == 0 && (item) < 64) g.trace[(item) * 8 + (slot)] = clock64(); \
-  } while (0)
 
 __global__ void __launch_bounds__(kTcThreads, 1)
     attention_tc_kernel(const __grid_constant__ CUtensorMap tma128,
@@ -182,8 +176,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();                // (secondary of the qkv GEMM: barriers and TMEM are set up before qkv exists)
-  pdl_launch_dependents();   // the out_proj GEMM that follows may set itself up on SMs as this grid's CTAs retire
 
   // units of this CTA: u = blockIdx.x + n * gridDim.x, n = 0 .. my_units-1
   const int my_units = (g.n_units - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
@@ -226,7 +218,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       const int region = j & 1, buf = n & 1;
       mbar_wait(&p_full[region], (j >> 1) & 1);
       tc_fence_after();
-      HBA_TRACE(j, 1);
       if (elect_one()) {
         const uint32_t tP = tmem_base + region * kTcRegionCols, tO = tP + kTcOCol;
         const uint64_t v_desc =
@@ -250,7 +241,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       if (i == 1) mbar_wait(&p_full[0], 0);
       mbar_wait(&r_free[region], ((i >> 1) & 1) ^ 1);
       tc_fence_after();
-      HBA_TRACE(i, 0);
       if (elect_one()) {
         const uint32_t q_addr = smem_base + buf * kTcBufBytes + tile * kTcQBytes;
         const uint64_t q_desc = make_smem_desc_sw128(q_addr);
@@ -305,7 +295,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       const int nv_max = __reduce_max_sync(0xffffffffu, nvalid);
       mbar_wait(&s_full[grp], use & 1);
       tc_fence_after();
-      if (q == 2) HBA_TRACE(i, 2);
       // Both passes read S in 32-column chunks, double buffered: the tcgen05.ld of chunk k+1 is issued
       // (unconditionally, address clamped to the last chunk) before chunk k is processed, so a TMEM
       // round trip overlaps the math.  Four independent partial maxima / sums keep the dependent
@@ -336,7 +325,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
         }
       }
       mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-      if (q == 2) HBA_TRACE(i, 3);
       const float mxs = mx * g.scale_log2;
       // pass 2: p = 2^(s * scale - max * scale), packed to bf16 over the S columns already consumed
       float s4[4] = {0.f, 0.f, 0.f, 0.f};
@@ -381,7 +369,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       tmem_st_wait();
       tc_fence_before();
       __syncwarp();
-      if (q == 2) HBA_TRACE(i, 4);
       if (lane == 0) mbar_arrive(&p_full[grp]);
       const float p_extra = extra_valid ? ex2_approx(fmaf(s_extra, g.scale_log2, -mxs)) : 0.f;
       sum += p_extra;
@@ -389,7 +376,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       // ---- O epilogue ----
       mbar_wait(&o_full[grp], use & 1);
       tc_fence_after();
-      if (q == 2) HBA_TRACE(i, 5);
       const float inv = __fdividef(1.0f, sum);
       const int64_t grow = (int64_t)b * g.T + qi;
       uint32_t o_all[64];
@@ -400,7 +386,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&r_free[grp]);
-      if (q == 2) HBA_TRACE(i, 7);
       float f[64];
 #pragma unroll
       for (int j = 0; j < 64; ++j) f[j] = __uint_as_float(o_all[j]);
@@ -448,7 +433,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
             *reinterpret_cast<uint4*>(obase + (int64_t)(4 * k) * g.ld_out) = ov[k];
       }
       __syncwarp();
-      if (q == 2) HBA_TRACE(i, 6);
       if (lane == 0) mbar_arrive(&kv_empty[buf]);
     }
   } else {
@@ -534,8 +518,6 @@ __global__ void __launch_bounds__(kTcThreads, 1)
   if (warp == 1) tmem_dealloc(tmem_base, kTcTmemCols);
 }
 
-static long long* g_attn_trace = nullptr;
-
 // host launcher, called from hba_attention_fwd (attention.cu) for bf16 activations
 int attention_tc_launch(const __nv_bfloat16* qkv, int64_t ld_qkv, int B, int T, int H, int causal,
                         __nv_bfloat16* out, int64_t ld_out, float* out_f32, int64_t ld_of, float* lse,
@@ -565,7 +547,6 @@ int attention_tc_launch(const __nv_bfloat16* qkv, int64_t ld_qkv, int B, int T, 
   g.out = out, g.ld_out = ld_out, g.out_f32 = out_f32, g.ld_of = ld_of;
   g.scale_log2 = 1.4426950408889634f * 0.125f;
   g.qkv = qkv, g.ld_qkv = ld_qkv;
-  g.trace = g_attn_trace;
   g.lse = lse;
   // [B, T, 3*H*64] maps: the row boxes are rounded up to 16 / 128 rows, and rows >= T of a sequence read
   // as zero instead of the next sequence's (non-finite values there must not reach P = 0 x K / V)
@@ -575,20 +556,8 @@ int attention_tc_launch(const __nv_bfloat16* qkv, int64_t ld_qkv, int B, int T, 
   HBA_CHECK(make_tma_3d_bf16(&t16, qkv, B, T, cols, ld_qkv, 16, 64));
   int ctas = num_sms();
   if (g.n_units < ctas) ctas = g.n_units;
-  cudaError_t e = launch_pdl(attention_tc_kernel, dim3(ctas), dim3(kTcThreads), kTcSmemBytes, stream, t128, t16, g);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    set_error("attention_tc_kernel launch: %s", cudaGetErrorString(e));
-    return HBA_ERR_CUDA;
-  }
+  attention_tc_kernel<<<ctas, kTcThreads, kTcSmemBytes, stream>>>(t128, t16, g);
   return check_launch("attention_tc_kernel");
 }
 
 }  // namespace hba
-
-// debug hook (not part of include/hba.h): device buffer of >= 512 int64 receiving clock64() stamps of
-// CTA 0, [item][slot]: 0 S issued, 1 PV issued, 2 S seen, 3 max pass done, 4 P written, 5 O seen,
-// 6 epilogue done; nullptr switches the trace off
-extern "C" void hba_debug_attention_trace(void* device_buffer) {
-  hba::g_attn_trace = static_cast<long long*>(device_buffer);
-}

@@ -44,22 +44,6 @@ int ensure_dyn_smem(Kernel kernel, size_t bytes, SmemAttr& st, const char* name)
   st.configured[dev] = bytes;
   return HBA_OK;
 }
-// HBA_PDL=1 (opt-in): kernels that can set themselves up before their inputs exist are launched with the
-// programmatic-stream-serialization attribute and call pdl_wait() before touching global memory
-bool pdl_enabled();
-// <<<grid, block, smem, stream>>> with that attribute (plain launch unless HBA_PDL=1)
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                       Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
 // 2-D bf16 row-major tensor map, box = [box_rows, box_cols]; 64-column boxes use SWIZZLE_128B
 int make_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld,
                      uint32_t box_rows, uint32_t box_cols);
@@ -107,14 +91,6 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
 __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
   __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
-}
-
-// ---- PTX: programmatic dependent launch (no-ops unless the launch carried the programmatic attribute) ----
-__device__ __forceinline__ void pdl_launch_dependents() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-__device__ __forceinline__ void pdl_wait() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 // ---- PTX: shared-memory addresses, mbarrier ----

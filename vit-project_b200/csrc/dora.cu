@@ -8,8 +8,6 @@
 // A CTA owns 8 consecutive output columns (one 32-byte sector per D row) and all `in` rows, so the
 // column norm is a CTA-local reduction and D is read exactly once (single pass, V kept in
 // registers).  The rank-r update costs in*out*r FMAs (33.5 M at 1024^2 x 32): negligible.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace hba {
@@ -624,12 +622,7 @@ __global__ void __launch_bounds__(256)
 }
 
 static bool dora_cluster_ok(int in_f, int out_f, int r) {
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("HBA_DORA_CLUSTER");
-    enabled = (e && e[0] == '0') ? 0 : 1;
-  }
-  return enabled && in_f <= 8 * kTR && in_f % 8 == 0 && out_f % kTC == 0 && r <= kRankMax && r % 4 == 0;
+  return in_f <= 8 * kTR && in_f % 8 == 0 && out_f % kTC == 0 && r <= kRankMax && r % 4 == 0;
 }
 
 template <typename Kernel, typename... Args>

@@ -11,14 +11,11 @@
 //                      multicast tcgen05.commit frees the smem slot / publishes the tile in both CTAs
 //   warps 2..9         epilogue: tcgen05.ld 32 lanes x 32 columns -> registers -> fused
 //                      bias / QuickGELU / GELU / activation-gradient / residual -> global
-// HBA_GEMM_CTA_GROUP=1 selects the single-CTA variant (128 x BN tiles) for A/B measurements.
 // "fp32 mode" (nsplit == 3) runs three bf16 passes per k-block over hi/lo split operands
 // (hi.hi + lo.hi + hi.lo), which reproduces fp32 products to ~2^-16 on the bf16 tensor pipe.
 //
 // Replaces F.linear at torch/nn/functional.py:6244 (in_proj), :6690 (out_proj) and the CLIP / timm
 // MLP linears reached through the reference's CLIPHBA.forward (NEW:298) and VIT:138-140.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace hba {
@@ -34,33 +31,19 @@ constexpr int kEpiWarps = 16;
 constexpr int kChunkCols = 16;
 constexpr int kGemmThreads = 64 + 32 * kEpiWarps;
 
-// CG = CTAs per UMMA (cta_group): with CG == 2 a CTA pair computes a 256 x BN tile, each CTA staging
-// its own 128 rows of A and only HALF of the B tile -> 1/3 fewer bytes through the L2->SM fabric per
-// FLOP than 128 x BN tiles (the fabric, not the tensor pipe, bounded the single-CTA kernel: 10.7 TB/s
-// of TMA traffic at 44 % tensor-pipe utilisation, profiles/r01_gemm_attn_ncu_full.md)
-template <int BN, int CG>
+// A CTA pair computes a 256 x BN tile, each CTA staging its own 128 rows of A and only HALF of the B
+// tile -> 1/3 fewer bytes through the L2->SM fabric per FLOP than 128 x BN tiles (the fabric, not the
+// tensor pipe, bounded a single-CTA kernel: 10.7 TB/s of TMA traffic at 44 % tensor-pipe utilisation,
+// profiles/r01_gemm_attn_ncu_full.md)
+template <int BN>
 struct GemmCfg {
   static constexpr int kABytes = BM * BK * 2;
-  static constexpr int kBBytes = (BN / CG) * BK * 2;
+  static constexpr int kBBytes = (BN / 2) * BK * 2;
   static constexpr int kStages = (192 * 1024) / (kABytes + kBBytes) > 8 ? 8 : (192 * 1024) / (kABytes + kBBytes);
   static constexpr int kTmemCols = 2 * BN;  // two accumulator stages
   static constexpr int kStagingBytes = kEpiWarps * 32 * kChunkCols * 4;  // per-warp transposition tiles of the epilogue
   static constexpr int kSmemBytes = kStages * (kABytes + kBBytes) + kStagingBytes + 1024 /*align*/ + 256 /*bars*/;
 };
-
-template <int CG>
-__device__ __forceinline__ void tma_load(void* dst, const CUtensorMap* m, uint32_t bar_addr, int c0,
-                                         int c1) {
-  if constexpr (CG == 2) {
-    tma_load_2d_pair(dst, m, bar_addr, c0, c1);
-  } else {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
-        "%4}], [%2];" ::"r"(smem_u32(dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_addr), "r"(c0), "r"(c1)
-        : "memory");
-  }
-}
 
 struct GemmArgs {
   int M, N, K;
@@ -88,7 +71,6 @@ struct GemmArgs {
   // ~all CTA pairs busy for 1 / tail_f of a tile time.  Every output element still accumulates its K products in
   // the same order: results are bit-identical to the unsplit schedule.
   int tail_first, tail_f;
-  int debug;       // HBA_GEMM_DEBUG (measurement only): 1 = epilogue drains TMEM but stores nothing, 2 = no TMA loads
 };
 
 // x * sigmoid(1.702 x) on the SFU fast paths (ex2.approx + rcp.approx, ~2 ulp): the epilogue of the
@@ -437,15 +419,15 @@ __device__ __forceinline__ GemmItem decode_item(const GemmArgs& g, int item, int
   return it;
 }
 
-template <int BN, int CG, int ACT>
+template <int BN, int ACT>
 __global__ void __launch_bounds__(kGemmThreads, 1)
     gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                    const __grid_constant__ CUtensorMap tma_b2, const __grid_constant__ CUtensorMap tma_b4,
                    const GemmArgs g) {
-  using Cfg = GemmCfg<BN, CG>;
+  using Cfg = GemmCfg<BN>;
   constexpr int kStages = Cfg::kStages;
-  constexpr int BNC = BN / CG;   // rows of B this CTA stages per k-block
-  constexpr int TM = BM * CG;    // rows of C per tile (per CTA pair when CG == 2)
+  constexpr int BNC = BN / 2;   // rows of B this CTA stages per k-block
+  constexpr int TM = 2 * BM;    // rows of C per tile (per CTA pair)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
                                              ~static_cast<uintptr_t>(1023));
@@ -463,8 +445,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
   // UTCHMMA / UTMALDG)
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
-  const int rank = (CG == 2) ? (int)cluster_ctarank() : 0;  // 0 = leader (issues the UMMAs)
-  const int worker = blockIdx.x / CG, num_workers = gridDim.x / CG;
+  const int rank = (int)cluster_ctarank();  // 0 = leader (issues the UMMAs)
+  const int worker = blockIdx.x / 2, num_workers = gridDim.x / 2;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tma_a);
@@ -475,27 +457,15 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tfull_bar[i], 1);
-      mbar_init(&tempty_bar[i], kEpiWarps * CG);  // one arrival per epilogue warp of the pair
+      mbar_init(&tempty_bar[i], kEpiWarps * 2);  // one arrival per epilogue warp of the pair
     }
     mbar_fence_init();
   }
-  if (warp == 1) {
-    if constexpr (CG == 2) tmem_alloc_pair(tmem_slot, Cfg::kTmemCols);
-    else tmem_alloc(tmem_slot, Cfg::kTmemCols);
-  }
+  if (warp == 1) tmem_alloc_pair(tmem_slot, Cfg::kTmemCols);
   tc_fence_before();
-  if constexpr (CG == 2) cluster_sync_all();  // the peer's barriers must be live before any remote arrive
-  else __syncthreads();
+  cluster_sync_all();  // the peer's barriers must be live before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // Programmatic dependent launch (HBA_PDL): everything above - barrier init, TMEM allocation, descriptor
-  // prefetch, the cluster rendezvous - touches no global memory and may run while the PRECEDING kernel of the
-  // stream is still draining its last tiles; the wait returns once that kernel has completed and flushed.
-  // launch_dependents (AFTER the wait: whatever a dependent reads before its own wait was then written by
-  // kernels that have completed) lets the NEXT kernel's CTAs do the same on SMs as this grid's CTAs retire.
-  // Both are no-ops when the kernel was launched without the programmatic attribute.
-  pdl_wait();
-  pdl_launch_dependents();
 
   const int num_m_tiles = (g.M + TM - 1) / TM;
   const int num_n_tiles = (g.N + BN - 1) / BN;
@@ -511,27 +481,21 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
       int stage = 0;
       uint32_t phase = 0;
       // where this CTA's TMA bytes are accounted: the pair leader's barriers
-      const uint32_t full0 = (CG == 2) ? mapa_u32(&full_bar[0], 0) : smem_u32(&full_bar[0]);
+      const uint32_t full0 = mapa_u32(&full_bar[0], 0);
       for (int item = worker; item < total_items; item += num_workers) {
         const GemmItem wi = decode_item<BN>(g, item, total_tiles);
         const int tile = wi.tile, slice = wi.slice;
-        const int bnc = wi.bn / CG;   // rows of B this CTA stages for the item
+        const int bnc = wi.bn / 2;   // rows of B this CTA stages for the item
         const int m0 = (tile / num_n_tiles) * TM + rank * BM;
         const int n0 = (tile % num_n_tiles) * BN + wi.n_off + rank * bnc;
         const CUtensorMap* tmb = wi.bn == BN ? &tma_b : (wi.bn * 2 == BN ? &tma_b2 : &tma_b4);
-        const uint32_t stage_bytes = (uint32_t)(CG * (Cfg::kABytes + bnc * BK * 2));
+        const uint32_t stage_bytes = (uint32_t)(2 * (Cfg::kABytes + bnc * BK * 2));
         const int kb_end = min(kblocks, (slice + 1) * kb_per);
         for (int kb = slice * kb_per; kb < kb_end; ++kb) {
           for (int s = 0; s < g.nsplit; ++s) {
             const int a_col = kb * BK + (s == 1 ? g.a_lo_off : 0);
             const int b_col = kb * BK + (s == 2 ? g.b_lo_off : 0);
             mbar_wait(&empty_bar[stage], phase ^ 1);
-            if (g.debug & 2) {
-              if (rank == 0 && elect_one()) mbar_arrive(&full_bar[stage]);
-              __syncwarp();
-              if (++stage == kStages) stage = 0, phase ^= 1;
-              continue;
-            }
             uint8_t* dA = sA + stage * Cfg::kABytes;
             uint8_t* dB = sB + stage * Cfg::kBBytes;
             const uint32_t fb = full0 + 8u * stage;
@@ -539,20 +503,20 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
             if (rank == 0)
               mbar_arrive_expect_tx(&full_bar[stage], stage_bytes);
             if (!g.a_mn) {
-              tma_load<CG>(dA, &tma_a, fb, a_col, m0);
+              tma_load_2d_pair(dA, &tma_a, fb, a_col, m0);
             } else {  // [K, M] storage: BM/64 boxes of 64 k-rows x 64 m-columns, 8 KB apart (LBO)
 #pragma unroll
               for (int j = 0; j < BM / 64; ++j)
-                tma_load<CG>(dA + j * 8192, &tma_a, fb, m0 + 64 * j + (s == 1 ? g.a_lo_off : 0),
-                             kb * BK);
+                tma_load_2d_pair(dA + j * 8192, &tma_a, fb, m0 + 64 * j + (s == 1 ? g.a_lo_off : 0),
+                                 kb * BK);
             }
             if (!g.b_mn) {
-              tma_load<CG>(dB, tmb, fb, b_col, n0);
+              tma_load_2d_pair(dB, tmb, fb, b_col, n0);
             } else {
 #pragma unroll
               for (int j = 0; j < BNC / 64; ++j)
-                tma_load<CG>(dB + j * 8192, &tma_b, fb, n0 + 64 * j + (s == 2 ? g.b_lo_off : 0),
-                             kb * BK);
+                tma_load_2d_pair(dB + j * 8192, &tma_b, fb, n0 + 64 * j + (s == 2 ? g.b_lo_off : 0),
+                                 kb * BK);
             }
             }
             __syncwarp();
@@ -591,18 +555,11 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
 #pragma unroll
           for (int k = 0; k < BK / 16; ++k) {
             const uint32_t accum = (it > 0 || k > 0) ? 1u : 0u;
-            if constexpr (CG == 2)
-              umma_bf16_pair(d_tmem, a_desc + a_step * k, b_desc + b_step * k, idesc, accum);
-            else
-              umma_bf16(d_tmem, a_desc + a_step * k, b_desc + b_step * k, idesc, accum);
+            umma_bf16_pair(d_tmem, a_desc + a_step * k, b_desc + b_step * k, idesc, accum);
           }
-          // frees the smem slot (in both CTAs of a pair) once these MMAs have read it
-          if constexpr (CG == 2) umma_commit_pair(&empty_bar[stage], 3);
-          else umma_commit(&empty_bar[stage]);
-          if (it == kiters - 1) {
-            if constexpr (CG == 2) umma_commit_pair(&tfull_bar[acc], 3);
-            else umma_commit(&tfull_bar[acc]);
-          }
+          // frees the smem slot (in both CTAs of the pair) once these MMAs have read it
+          umma_commit_pair(&empty_bar[stage], 3);
+          if (it == kiters - 1) umma_commit_pair(&tfull_bar[acc], 3);
           }
           __syncwarp();
           if (++stage == kStages) stage = 0, phase ^= 1;
@@ -615,9 +572,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     const int q = warp & 3;  // TMEM lane quarter this warp may access
     const int part = (warp - 2) >> 2;  // which 1 / (kEpiWarps / 4) of the tile's columns this warp drains
     constexpr int kParts = kEpiWarps / 4;
-    const uint32_t tempty_addr[2] = {
-        (CG == 2) ? mapa_u32(&tempty_bar[0], 0) : smem_u32(&tempty_bar[0]),
-        (CG == 2) ? mapa_u32(&tempty_bar[1], 0) : smem_u32(&tempty_bar[1])};
+    const uint32_t tempty_addr[2] = {mapa_u32(&tempty_bar[0], 0), mapa_u32(&tempty_bar[1], 0)};
     int acc = 0;
     uint32_t acc_phase = 0;
     // The epilogue's own inputs (residual / pre-activation rows of this warp's half tile) are pulled
@@ -661,7 +616,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
         tmem_ld_chunk(taddr, r);
         tmem_ld_wait();
         const int col = n0 + c * kChunkCols;
-        if (g.debug & 1) continue;
         if (g.transpose_out) {
           if (row < g.M && col < g.N) epilogue_chunk_transposed(g, r, row, col);
         } else if (m0 + q * 32 < g.M && col < g.N) {  // warp-uniform
@@ -676,13 +630,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     }
   }
   tc_fence_before();
-  if constexpr (CG == 2) {
-    cluster_sync_relaxed();  // the leader's UMMAs read the peer's smem and signal its barriers until the end
-    if (warp == 1) tmem_dealloc_pair(tmem_base, Cfg::kTmemCols);
-  } else {
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, Cfg::kTmemCols);
-  }
+  cluster_sync_relaxed();  // the leader's UMMAs read the peer's smem and signal its barriers until the end
+  if (warp == 1) tmem_dealloc_pair(tmem_base, Cfg::kTmemCols);
 }
 
 // out[r, c] = epilogue(sum_s part[s][r, c])  (split-K reduction, fixed order: deterministic).  The epilogue is
@@ -761,15 +710,6 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const ReduceArgs a) 
   }
 }
 
-static int gemm_cta_group() {
-  static int cg = 0;
-  if (cg == 0) {
-    const char* e = getenv("HBA_GEMM_CTA_GROUP");
-    cg = (e && e[0] == '1') ? 1 : 2;
-  }
-  return cg;
-}
-
 // Encoding a CUtensorMap costs ~1 us of host time (cuTensorMapEncodeTiled) and every GEMM launch needs two; the
 // operands of a training step are the same few hundred (pointer, shape, stride, box) tuples step after step, so
 // the encoded descriptors are kept in a small direct-mapped, per-thread cache.  A descriptor depends on nothing but
@@ -806,21 +746,12 @@ static int cached_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, 
   return HBA_OK;
 }
 
-static bool tail_split_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("HBA_GEMM_TAIL_SPLIT");
-    on = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
-}
-
-template <int BN, int CG, int ACT>
+template <int BN, int ACT>
 static int launch_gemm(const hba_gemm_params* p, const GemmArgs& g, cudaStream_t stream) {
-  using Cfg = GemmCfg<BN, CG>;
+  using Cfg = GemmCfg<BN>;
   static SmemAttr smem_attr;
-  HBA_CHECK(ensure_dyn_smem(gemm_tc_kernel<BN, CG, ACT>, Cfg::kSmemBytes, smem_attr, "gemm_tc_kernel"));
-  constexpr int BNC = BN / CG;
+  HBA_CHECK(ensure_dyn_smem(gemm_tc_kernel<BN, ACT>, Cfg::kSmemBytes, smem_attr, "gemm_tc_kernel"));
+  constexpr int BNC = BN / 2;
   const uint64_t a_cols = (uint64_t)p->K + (p->nsplit == 3 ? (uint64_t)p->a_lo_off : 0);
   const uint64_t b_cols = (uint64_t)p->K + (p->nsplit == 3 ? (uint64_t)p->b_lo_off : 0);
   CUtensorMap ta, tb;
@@ -836,9 +767,9 @@ static int launch_gemm(const hba_gemm_params* p, const GemmArgs& g, cudaStream_t
     const uint64_t cols = (uint64_t)p->N + (p->nsplit == 3 ? (uint64_t)p->b_lo_off : 0);
     HBA_CHECK(cached_tma_2d_bf16(&tb, p->B, p->K, cols, p->ldb, 64, 64));
   }
-  const int tiles = ((p->M + BM * CG - 1) / (BM * CG)) * ((p->N + BN - 1) / BN);
-  int workers = num_sms() / CG;
-  if (p->max_ctas > 0 && p->max_ctas / CG < workers) workers = p->max_ctas / CG > 0 ? p->max_ctas / CG : 1;
+  const int tiles = ((p->M + 2 * BM - 1) / (2 * BM)) * ((p->N + BN - 1) / BN);
+  int workers = num_sms() / 2;  // CTA pairs
+  if (p->max_ctas > 0 && p->max_ctas / 2 < workers) workers = p->max_ctas / 2 > 0 ? p->max_ctas / 2 : 1;
   if (tiles * g.k_slices < workers) workers = tiles * g.k_slices;
   // tail splitting: cut the tiles of a partial last round into 2 or 4 column slabs when that shortens the round.
   // Slab times relative to a full tile (the kernel is bound by the bytes an SM takes in per k-block: its 16 KB of A
@@ -847,8 +778,8 @@ static int launch_gemm(const hba_gemm_params* p, const GemmArgs& g, cudaStream_t
   GemmArgs ga = g;
   ga.tail_first = tiles, ga.tail_f = 1;
   CUtensorMap tb2 = tb, tb4 = tb;
-  if (BN == 256 && CG == 2 && g.k_slices == 1 && !p->a_mn_major && !p->b_mn_major && tail_split_enabled() &&
-      tiles > workers && tiles % workers != 0) {
+  if (BN == 256 && g.k_slices == 1 && !p->a_mn_major && !p->b_mn_major && tiles > workers &&
+      tiles % workers != 0) {
     const int rem = tiles % workers;
     const double cost1 = 1.0;
     const double cost2 = ((rem * 2 + workers - 1) / workers) * 0.75;
@@ -863,26 +794,21 @@ static int launch_gemm(const hba_gemm_params* p, const GemmArgs& g, cudaStream_t
     }
   }
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(workers * CG));
+  cfg.gridDim = dim3((unsigned)(workers * 2));
   cfg.blockDim = dim3(kGemmThreads);
   cfg.dynamicSmemBytes = Cfg::kSmemBytes;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  if (pdl_enabled()) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
-  cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, CG, ACT>, ta, tb, tb2, tb4, ga);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, ACT>, ta, tb, tb2, tb4, ga);
   if (e != cudaSuccess) {
     cudaGetLastError();
-    set_error("gemm_tc_kernel<%d,%d> launch: %s", BN, CG, cudaGetErrorString(e));
+    set_error("gemm_tc_kernel<%d> launch: %s", BN, cudaGetErrorString(e));
     return HBA_ERR_CUDA;
   }
   return check_launch("gemm_tc_kernel");
@@ -973,18 +899,10 @@ extern "C" int hba_gemm_bf16(const hba_gemm_params* p, void* stream) {
     g.out_f32 = p->k_workspace;
     g.ld_f32 = p->N;
   }
-  {
-    static int dbg = -1;
-    if (dbg < 0) {
-      const char* e = getenv("HBA_GEMM_DEBUG");
-      dbg = e ? atoi(e) : 0;
-    }
-    g.debug = dbg;
-  }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const bool wide = p->N >= 256;
   if (g.k_slices > 1) {
-    const int rc = wide ? launch_gemm<256, 2, HBA_ACT_NONE>(p, g, s) : launch_gemm<128, 2, HBA_ACT_NONE>(p, g, s);
+    const int rc = wide ? launch_gemm<256, HBA_ACT_NONE>(p, g, s) : launch_gemm<128, HBA_ACT_NONE>(p, g, s);
     if (rc != HBA_OK) return rc;
     const size_t n4 = (size_t)p->M * (p->N / 4);
     int blocks = (int)((n4 + 255) / 256);
@@ -992,25 +910,16 @@ extern "C" int hba_gemm_bf16(const hba_gemm_params* p, void* stream) {
     splitk_reduce_kernel<<<blocks, 256, 0, s>>>(red);
     return check_launch("splitk_reduce_kernel");
   }
-  if (gemm_cta_group() == 2) {
-    switch (p->act) {
+  switch (p->act) {
 #define HBA_GEMM_CASE(A) \
   case A:                \
-    return wide ? launch_gemm<256, 2, A>(p, g, s) : launch_gemm<128, 2, A>(p, g, s);
-      HBA_GEMM_CASE(HBA_ACT_NONE)
-      HBA_GEMM_CASE(HBA_ACT_QUICKGELU)
-      HBA_GEMM_CASE(HBA_ACT_GELU_ERF)
-      HBA_GEMM_CASE(HBA_ACT_QUICKGELU_GRAD)
-      HBA_GEMM_CASE(HBA_ACT_GELU_ERF_GRAD)
+    return wide ? launch_gemm<256, A>(p, g, s) : launch_gemm<128, A>(p, g, s);
+    HBA_GEMM_CASE(HBA_ACT_NONE)
+    HBA_GEMM_CASE(HBA_ACT_QUICKGELU)
+    HBA_GEMM_CASE(HBA_ACT_GELU_ERF)
+    HBA_GEMM_CASE(HBA_ACT_QUICKGELU_GRAD)
+    HBA_GEMM_CASE(HBA_ACT_GELU_ERF_GRAD)
 #undef HBA_GEMM_CASE
-    }
   }
-  // single-CTA variant (HBA_GEMM_CTA_GROUP=1): kept for A/B measurements of the plain and QuickGELU paths
-  if (p->act == HBA_ACT_NONE)
-    return wide ? launch_gemm<256, 1, HBA_ACT_NONE>(p, g, s) : launch_gemm<128, 1, HBA_ACT_NONE>(p, g, s);
-  if (p->act == HBA_ACT_QUICKGELU)
-    return wide ? launch_gemm<256, 1, HBA_ACT_QUICKGELU>(p, g, s)
-                : launch_gemm<128, 1, HBA_ACT_QUICKGELU>(p, g, s);
-  set_error("hba_gemm_bf16: HBA_GEMM_CTA_GROUP=1 supports HBA_ACT_NONE / HBA_ACT_QUICKGELU only");
-  return HBA_ERR_ARG;
+  return HBA_ERR_ARG;  // (unreachable: act was checked above)
 }

@@ -1,8 +1,6 @@
 // Bandwidth-bound row-wise kernels of the CLIP-HBA towers: operand staging (fp32 -> bf16 hi/lo),
 // LayerNorm forward/backward, patch im2col, token assembly + ln_pre, text embedding, row gathers.
 // All are one-warp-per-row or grid-stride kernels with 128-bit accesses; bound: HBM.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace hba {
@@ -164,8 +162,6 @@ __global__ void __launch_bounds__(kLnsThreads, 1)
     }
     mbar_fence_init();
   }
-  pdl_wait();                // (secondary of the kernel that produces x: the barriers are set up before x exists)
-  pdl_launch_dependents();   // the GEMM that consumes y may run its prologue while the last rows are normalised
   for (int c = threadIdx.x * 4; c < cols; c += kLnsThreads * 4) {
     *reinterpret_cast<float4*>(s_gamma + c) = __ldg(reinterpret_cast<const float4*>(gamma + c));
     *reinterpret_cast<float4*>(s_beta + c) = __ldg(reinterpret_cast<const float4*>(beta + c));
@@ -459,12 +455,7 @@ extern "C" int hba_layernorm_fwd(const float* x, int64_t rows, int32_t cols, int
   HBA_REQUIRE(ldx % 4 == 0 && ld_yf % 4 == 0 && ld_yb % 4 == 0 && lo_off % 4 == 0 && ((uintptr_t)y_bf16 & 7) == 0, "hba_layernorm_fwd: leading dimensions must keep 16-byte (fp32) / 8-byte (bf16) alignment");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (row_step < 1) row_step = 1;
-  static int use_stream = -1;
-  if (use_stream < 0) {
-    const char* e = getenv("HBA_LN_STREAM");
-    use_stream = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (use_stream && rows >= 1024 && ((uintptr_t)x & 15) == 0) {
+  if (rows >= 1024 && ((uintptr_t)x & 15) == 0) {
     // streaming form: persistent CTAs, rows staged through shared memory by bulk asynchronous copies
     int stages = (int)((220 * 1024 - 2 * cols * 4 - 256) / ((size_t)kLnsRows * cols * 4));
     if (stages > kLnsMaxStages) stages = kLnsMaxStages;
@@ -473,14 +464,9 @@ extern "C" int hba_layernorm_fwd(const float* x, int64_t rows, int32_t cols, int
     HBA_CHECK(ensure_dyn_smem(layernorm_fwd_stream_kernel, smem, attr, "layernorm_fwd_stream_kernel"));
     int grid = num_sms();
     if ((int64_t)grid * kLnsRows > rows) grid = (int)((rows + kLnsRows - 1) / kLnsRows);
-    cudaError_t e = launch_pdl(layernorm_fwd_stream_kernel, dim3(grid), dim3(kLnsThreads), smem, s, x, rows, cols, ldx,
-                               row_step, gamma, beta, eps, y_f32, ld_yf, static_cast<__nv_bfloat16*>(y_bf16), ld_yb,
-                               lo_off, stages);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      set_error("layernorm_fwd_stream_kernel launch: %s", cudaGetErrorString(e));
-      return HBA_ERR_CUDA;
-    }
+    layernorm_fwd_stream_kernel<<<grid, kLnsThreads, smem, s>>>(x, rows, cols, ldx, row_step, gamma, beta, eps, y_f32,
+                                                                ld_yf, static_cast<__nv_bfloat16*>(y_bf16), ld_yb,
+                                                                lo_off, stages);
     return check_launch("hba_layernorm_fwd (stream)");
   }
   layernorm_fwd_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, s>>>(

@@ -286,7 +286,7 @@ class Engine:
         leave most of the 74 CTA pairs idle while a few SMs stream the whole weight matrix; split along K the
         matrix is pulled by ~74 pairs at once and the epilogue runs in the slice reduction (same fused epilogue).
         The workspace is per tag: the two towers run on different streams."""
-        if R > 256 or os.environ.get("HBA_SKINNY_SPLITK", "1") == "0":
+        if R > 256:
             return {}
         s = ops.auto_k_slices(R, N, K, min_kblocks=4)
         if s <= 1:
