@@ -308,6 +308,26 @@ int hba_rsa_bootstrap(const double* ref_tri, const uint32_t* ref_order, const do
                       int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Kendall's tau-a and tau-b, the RDM comparator Nili et al. 2014 recommend when either RDM has ties (tau-a does not
+ * favour models that predict tied dissimilarities).  For x [n] (model triangle) and y [n] (reference triangle),
+ * n0 = n(n-1)/2, with values equal as in numpy (-0.0 == +0.0):
+ *   n1 = sum t(t-1)/2 over the tie groups of x, n2 the same over y, n3 = pairs tied in both x and y,
+ *   S  = concordant - discordant = n0 - n1 - n2 + n3 - 2 D   (D = discordant pairs),
+ *   counts[0..3] = S, n1, n2, n3  (exact int64: outputs are bit-identical run to run),
+ *   tau[0] = tau_a = S / n0,
+ *   tau[1] = tau_b = S / sqrt(n0 - n1) / sqrt(n0 - n2) clipped to [-1, 1]  (= scipy.stats.kendalltau, variant 'b').
+ * A NaN in x or y gives counts -1 and NaN taus; so does a y_order with an entry outside [0, n) or that does not sort
+ * y.  A constant side (n1 == n0 or n2 == n0) gives NaN taus with the counts written.
+ * y_order: the stable sorted order of y (hba_rank_order_f64; any permutation that sorts y will do).  2 <= n < 2^30
+ * (the bound of hba_rank_order_f64).  n <= 2048 runs in one CTA without workspace; larger n needs
+ * hba_kendall_workspace_bytes(n) bytes, 256-byte aligned: x[y_order] sorted by the radix passes of
+ * hba_rank_order_f64, then a merge sort of the y-ranks that counts D as it merges (Knight's method, O(n log n)).
+ */
+int64_t hba_kendall_workspace_bytes(int64_t n);
+int hba_kendall_tau_f64(const double* x, const double* y, const uint32_t* y_order, int64_t n, int64_t* counts,
+                        double* tau, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Softmax cross-entropy (nn.CrossEntropyLoss at VIT:291, applied VIT:139) forward + backward:
  * logits [B, C] fp32, labels int64 -> loss (mean, device float) and d_logits = (softmax - 1hot)/B
  */

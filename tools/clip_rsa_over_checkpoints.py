@@ -11,7 +11,9 @@ the two CSV files (rows in the order train csv, then inference csv) - what RDM48
 The last stdout line is a JSON record with checkpoints/s (wall clock, max over ranks, cache fill included).
 --permutations N adds the Mantel p-value column behavioral_rsa_p_perm, --bootstrap N the stimulus-bootstrap 95 %
 interval (behavioral_rsa_ci_low / _ci_high) and the number of valid replicates (behavioral_rsa_boot_valid); --seed
-seeds both, identically for every checkpoint.  Without them the CSV has the columns of hba.rsa_scale.RESULT_COLUMNS.
+seeds both, identically for every checkpoint.  --kendall adds Kendall's tau-a and tau-b of each model RDM against the
+reference (behavioral_rsa_tau_a / _tau_b).  Without these flags the CSV has the columns of
+hba.rsa_scale.RESULT_COLUMNS.
 """
 import argparse
 import json
@@ -40,6 +42,8 @@ def main(argv=None):
     ap.add_argument("--permutations", type=int, default=0, help="Mantel permutations per checkpoint (0: none)")
     ap.add_argument("--bootstrap", type=int, default=0, help="stimulus-bootstrap replicates per checkpoint (0: none)")
     ap.add_argument("--seed", type=int, default=0, help="seed of the permutations and resamples")
+    ap.add_argument("--kendall", action="store_true",
+                    help="add Kendall's tau-a and tau-b columns (tau-a: preferred when either RDM has ties)")
     a = ap.parse_args(argv)
     import numpy as np
     import pandas as pd
@@ -90,7 +94,8 @@ def main(argv=None):
     t_setup = time.perf_counter() - t_start
     res = rsa_scale.clip_rsa_over_checkpoints(model, loaders, ref, files, device, rank=rank, world_size=world,
                                               output_csv=a.output_csv or None, log=None, root=a.checkpoints,
-                                              n_perm=a.permutations, n_boot=a.bootstrap, seed=a.seed)
+                                              n_perm=a.permutations, n_boot=a.bootstrap, seed=a.seed,
+                                              kendall=a.kendall)
     torch.cuda.synchronize()
     wall = time.perf_counter() - t_start
     if world > 1:

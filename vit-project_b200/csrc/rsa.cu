@@ -16,6 +16,7 @@
 
 #include "common.cuh"
 #include "rsa_keys.cuh"
+#include "rsa_radix.cuh"
 
 namespace hba {
 
@@ -169,11 +170,7 @@ __global__ void __launch_bounds__(1024)
 }
 
 // ------------------------------------------------------------------------------------------
-// Large n: least-significant-digit radix sort of (key, original index) pairs.
-//   control block (zeroed by one memset per call):
-//     hist[8][256]   global digit histograms, all eight from ONE pass over the keys
-//     ticket[8]      dynamic tile numbering per pass (a tile only ever waits for tiles that already run)
-//     nan_count, done  NaN detection; last-block ticket of the final reduction
+// Large n: least-significant-digit radix sort of (key, original index) pairs (control block: rsa_radix.cuh).
 //     status[8][tiles][256]  decoupled look-back words: flag (2 bits) | count (30 bits)
 //   A digit whose histogram has a single non-empty bin leaves the order unchanged: its pass returns at once
 //   (RDM entries live in [0, 2]: the top byte is constant).  Every CTA derives which buffer holds the current
@@ -185,17 +182,7 @@ constexpr int kRadixWarps = kRadixThreads / 32;
 // the latency of its shared-memory / shuffle chain (ncu: 19 % issue-active, 38 us per pass at 1.7 M keys)
 constexpr int kRadixIters = 8;                                   // per warp
 constexpr int kRadixTile = kRadixWarps * kRadixIters * 32;       // 2048 elements per CTA
-constexpr int kDigits = 8;
 constexpr unsigned int kFlagAgg = 1u << 30, kFlagIncl = 2u << 30, kCountMask = (1u << 30) - 1u;
-
-struct RadixCtl {
-  unsigned int hist[kDigits][256];
-  unsigned int ticket[kDigits];
-  unsigned int nan_count;
-  unsigned int done;
-  unsigned int pad[256 - kDigits - 2];
-};
-static_assert(sizeof(RadixCtl) == (kDigits * 256 + 256) * 4, "control block layout");
 
 // keys (from doubles, or already produced by rdm_kernel) + all eight digit histograms + NaN count
 __global__ void __launch_bounds__(256)
@@ -235,11 +222,6 @@ __global__ void __launch_bounds__(256)
   }
   nans = warp_sum(nans);
   if ((threadIdx.x & 31) == 0 && nans) atomicAdd(&ctl->nan_count, nans);
-}
-
-// true when digit d cannot change the order (one bin holds all n keys)
-__device__ __forceinline__ bool digit_is_constant(const RadixCtl* ctl, int d, unsigned int n) {
-  return __syncthreads_or(ctl->hist[d][threadIdx.x] == n) != 0;
 }
 
 // block-wide exclusive scan of one value per thread (256 threads); `scratch` holds 8 uints
@@ -384,8 +366,7 @@ __global__ void __launch_bounds__(256)
   __shared__ double scratch[32];
   __shared__ int s_last;
   const unsigned int n32 = (unsigned int)n;
-  int executed = 0;
-  for (int d = 0; d < kDigits; ++d) executed += digit_is_constant(ctl, d, n32) ? 0 : 1;
+  const int executed = radix_passes_executed(ctl, n32);
   const unsigned long long* keys = (executed & 1) ? kbuf1 : kbuf0;
   const unsigned int* vals = (executed & 1) ? vbuf1 : vbuf0;
   const bool implicit_vals = executed == 0;
@@ -443,8 +424,7 @@ __global__ void __launch_bounds__(256)
     sorted_order_kernel(const unsigned int* __restrict__ vbuf0, const unsigned int* __restrict__ vbuf1, int64_t n,
                         RadixCtl* __restrict__ ctl, unsigned int* __restrict__ order) {
   const unsigned int n32 = (unsigned int)n;
-  int executed = 0;
-  for (int d = 0; d < kDigits; ++d) executed += digit_is_constant(ctl, d, n32) ? 0 : 1;
+  const int executed = radix_passes_executed(ctl, n32);
   const unsigned int* vals = (executed & 1) ? vbuf1 : vbuf0;
   for (int64_t p = blockIdx.x * 256ll + threadIdx.x; p < n; p += (int64_t)gridDim.x * 256)
     order[p] = executed == 0 ? (unsigned int)p : vals[p];
@@ -513,18 +493,7 @@ __global__ void pearson_final_kernel(const double* __restrict__ ws, int nblocks,
 
 static inline int64_t align256(int64_t v) { return (v + 255) & ~(int64_t)255; }
 
-struct RankWorkspace {
-  unsigned long long *k0, *k1;
-  unsigned int *v0, *v1;
-  RadixCtl* ctl;
-  unsigned int* status;
-  double* partial;
-  int tiles;
-  int64_t zero_bytes;   // control block + status words: cleared at the start of every call
-  int64_t total_bytes;
-};
-
-static RankWorkspace rank_workspace_layout(void* base, int64_t n) {
+RankWorkspace rank_workspace_layout(void* base, int64_t n) {
   RankWorkspace w;
   w.tiles = (int)((n + kRadixTile - 1) / kRadixTile);
   char* p = static_cast<char*>(base);
@@ -542,9 +511,7 @@ static RankWorkspace rank_workspace_layout(void* base, int64_t n) {
   return w;
 }
 
-// sort + final pass; keys must already be in w.k0 unless x is given
-static int rank_large(const double* x, int64_t n, const RankWorkspace& w, double* ranks_out, const double* ref,
-                      double* rho, cudaStream_t s) {
+int radix_sort(const double* x, int64_t n, const RankWorkspace& w, cudaStream_t s) {
   static SmemAttr attr;
   HBA_CHECK(ensure_dyn_smem(radix_pass_kernel, kRadixPassSmem, attr, "radix_pass_kernel"));
   cudaError_t e = cudaMemsetAsync(w.ctl, 0, (size_t)w.zero_bytes, s);
@@ -562,6 +529,13 @@ static int rank_large(const double* x, int64_t n, const RankWorkspace& w, double
                                                                      w.status, w.tiles);
     HBA_CHECK(check_launch("radix_pass_kernel"));
   }
+  return HBA_OK;
+}
+
+// sort + final pass; keys must already be in w.k0 unless x is given
+static int rank_large(const double* x, int64_t n, const RankWorkspace& w, double* ranks_out, const double* ref,
+                      double* rho, cudaStream_t s) {
+  HBA_CHECK(radix_sort(x, n, w, s));
   int fb = (int)((n + 255) / 256);
   if (fb > kFinalBlocks) fb = kFinalBlocks;
   rank_final_kernel<<<fb, 256, 0, s>>>(w.k0, w.k1, w.v0, w.v1, n, w.ctl, ranks_out, ref, w.partial, rho);

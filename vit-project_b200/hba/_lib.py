@@ -73,6 +73,8 @@ SIGNATURES = {
     "hba_rsa_perm_null": (i32, [vp, vp, i32, vp, i32, vp, vp, i64, vp]),
     "hba_rsa_boot_workspace_bytes": (i64, [i32, i32]),
     "hba_rsa_bootstrap": (i32, [vp, vp, vp, vp, vp, vp, i32, vp, i32, vp, vp, vp, i64, vp]),
+    "hba_kendall_workspace_bytes": (i64, [i64]),
+    "hba_kendall_tau_f64": (i32, [vp, vp, vp, i64, vp, vp, vp, i64, vp]),
     "hba_softmax_ce_fwd_bwd": (i32, [vp, i64, vp, i32, i32, vp, vp, i64, vp, vp, vp]),
     "hba_colsum": (i32, [vp, i32, i64, i32, i64, vp, i32, vp, vp]),
     "hba_layernorm_param_grad": (i32, [vp, i64, vp, i64, i32, i64, i64, f32, vp, i32, vp, vp]),

@@ -424,6 +424,34 @@ def rsa_bootstrap(ref_tri, ref_order, tri_a, order_a, counts, rho_a, workspace, 
                                         _stream()), "hba_rsa_bootstrap", kernels)
 
 
+def kendall_workspace_bytes(n):
+    return int(_lib.load().hba_kendall_workspace_bytes(n))
+
+
+def kendall_kernels(n):
+    """Kernels one hba_kendall_tau_f64 call launches: one CTA up to n = 2048; else keys, the radix sort (histogram +
+    8 digit passes), y-ranks, tiles of 4096, one merge level per doubling of the run width up to n, final."""
+    if n <= 2048:
+        return 1
+    levels, width = 0, 4096
+    while width < n:
+        levels, width = levels + 1, 2 * width
+    return 13 + levels
+
+
+def kendall_tau_f64(x, y, y_order, counts, tau, workspace):
+    """Kendall's tau of x against y [n] f64 from exact pair counts: counts [4] int64 = (S, n1, n2, n3), tau [2] f64 =
+    (tau_a, tau_b); y_order [n] int32 (uint32 bits) is y's stable sorted order (rank_order_f64)."""
+    n = x.numel()
+    assert x.dtype == y.dtype == tau.dtype == torch.float64 and y_order.dtype == torch.int32
+    assert counts.dtype == torch.int64 and counts.numel() >= 4 and tau.numel() >= 2
+    assert x.is_contiguous() and y.is_contiguous() and y_order.is_contiguous()
+    assert y.numel() == n and y_order.numel() == n
+    check(_lib.load().hba_kendall_tau_f64(_p(x), _p(y), _p(y_order), n, _p(counts), _p(tau), _p(workspace),
+                                          workspace.numel() if workspace is not None else 0, _stream()),
+          "hba_kendall_tau_f64", kendall_kernels(n))
+
+
 def softmax_ce(logits, labels, loss, d_logits, correct, workspace):
     B, Cc = logits.shape
     check(_lib.load().hba_softmax_ce_fwd_bwd(_p(logits), logits.stride(0), _p(labels), B, Cc, _p(loss),
@@ -516,7 +544,7 @@ for _name in ("gemm", "split_bf16", "layernorm_fwd", "layernorm_bwd", "im2col_pa
               "embed_tokens", "gather_rows", "attention_fwd", "attention_bwd_row0", "dora_merge_fwd", "dora_merge_bwd",
               "cos_head_fwd", "cos_head_bwd", "cos_mse_fwd", "cos_mse_bwd", "adamw_multi", "sgd_multi", "sgd_staged",
               "rdm_f64", "rank_avg_f64", "pearson_f64", "rdm_spearman", "rank_order_f64", "rsa_perm_null",
-              "rsa_bootstrap", "softmax_ce", "colsum", "layernorm_param_grad",
+              "rsa_bootstrap", "kendall_tau_f64", "softmax_ce", "colsum", "layernorm_param_grad",
               "attention_bwd", "layernorm_bwd_fused", "attention_fwd_lse", "attention_bwd_lse", "add_rows",
               "nonfinite_flag"):
     globals()[_name] = _device_guarded(globals()[_name])

@@ -10,6 +10,9 @@ Resampling statistics (RSAEvaluator.permutation_test / .bootstrap) resample stim
 on: a Mantel permutation test for the p-value and the stimulus bootstrap of Nili et al. 2014 for confidence intervals.
 Replicates are drawn on the host (numpy.random.default_rng(seed)) and evaluated by hba_rsa_perm_null /
 hba_rsa_bootstrap, each RDM sorted once (hba_rank_order_f64).
+
+RSAEvaluator.kendall_tau compares the two RDMs with Kendall's tau-a and tau-b instead of rho (hba_kendall_tau_f64,
+against the same cached sorted order of the reference).
 """
 from __future__ import annotations
 
@@ -42,6 +45,7 @@ class RSAEvaluator:
         ops.rank_avg_f64(ref_tri, self.ref_ranks, self.rank_ws)
         self.ref_tri = ref_tri
         self._ref_order = None
+        self._kendall = None     # (workspace, counts [4] int64, tau [2] f64) of kendall_tau, allocated on first use
         self.tri = torch.empty(self.P, dtype=torch.float64, device=self.device)
         self.ranks = torch.empty(self.P, dtype=torch.float64, device=self.device)
         self.rdm = torch.empty(self.N, self.N, dtype=torch.float64, device=self.device)
@@ -83,6 +87,14 @@ class RSAEvaluator:
         ops.rdm_f64(emb, None, tri)
         ops.rank_order_f64(tri, order, ranks, self.rank_ws)
         return tri, order, ranks
+
+    def _reference_order(self):
+        """The stable sorted order [P] int32 of the reference triangle (hba_rank_order_f64), computed once."""
+        if self._ref_order is None:
+            self._ref_order = torch.empty(self.P, dtype=torch.int32, device=self.device)
+            ranks = torch.empty(self.P, dtype=torch.float64, device=self.device)
+            ops.rank_order_f64(self.ref_tri, self._ref_order, ranks, self.rank_ws)
+        return self._ref_order
 
     def _chunk(self, n, bytes_of, per_replicate_host):
         """Replicates per device call so that workspace + uploads + outputs stay within STATS_CHUNK_BYTES."""
@@ -142,10 +154,7 @@ class RSAEvaluator:
             return (float("nan"), float("nan")), reps, 0
         rng = np.random.default_rng(seed)
         with torch.cuda.device(self.device):
-            if self._ref_order is None:
-                self._ref_order = torch.empty(self.P, dtype=torch.int32, device=self.device)
-                ranks = torch.empty(self.P, dtype=torch.float64, device=self.device)
-                ops.rank_order_f64(self.ref_tri, self._ref_order, ranks, self.rank_ws)
+            ref_order = self._reference_order()
             tri_a, order_a, _ = self._model_arrays(emb)
             tri_b = order_b = None
             if paired_with is not None:
@@ -160,13 +169,34 @@ class RSAEvaluator:
                 out_a = torch.full((k,), float("nan"), dtype=torch.float64, device=self.device)
                 out_b = None if tri_b is None else torch.full((k,), float("nan"), dtype=torch.float64,
                                                               device=self.device)
-                ops.rsa_bootstrap(self.ref_tri, self._ref_order, tri_a, order_a, counts_dev, out_a, ws,
+                ops.rsa_bootstrap(self.ref_tri, ref_order, tri_a, order_a, counts_dev, out_a, ws,
                                   tri_b=tri_b, order_b=order_b, rho_b=out_b)
                 r = out_a.cpu().numpy()
                 if out_b is not None:
                     r = r - out_b.cpu().numpy()
                 reps[s:s + k] = r
         return percentile_interval(reps, alpha), reps, int(np.isfinite(reps).sum())
+
+    # ------------------------------------------------------------------ Kendall's tau
+    def kendall_tau(self, emb):
+        """Kendall's tau of emb's RDM (x) against the reference (y) over the P upper-triangle pairs, from exact pair
+        counts on the device (hba_kendall_tau_f64) -> (tau_a, tau_b).  tau_b equals scipy.stats.kendalltau; tau_a =
+        (concordant - discordant) / (P (P - 1) / 2) does not favour model RDMs that predict tied dissimilarities, which
+        is why Nili et al. 2014 recommend it whenever either RDM has ties (e.g. a categorical reference).  NaN when an
+        RDM entry is NaN or when either triangle is constant."""
+        if emb.shape[0] != self.N:
+            raise ValueError(f"expected {self.N} embeddings, got {emb.shape[0]}")
+        with torch.cuda.device(self.device):
+            emb = emb.detach().to(self.device, torch.float32).contiguous()
+            if self._kendall is None:
+                ws = torch.empty(ops.kendall_workspace_bytes(self.P), dtype=torch.uint8, device=self.device)
+                self._kendall = (ws, torch.empty(4, dtype=torch.int64, device=self.device),
+                                 torch.empty(2, dtype=torch.float64, device=self.device))
+            ws, counts, tau = self._kendall
+            ops.rdm_f64(emb, None, self.tri)
+            ops.kendall_tau_f64(self.tri, self.ref_tri, self._reference_order(), counts, tau, ws)
+            tau_a, tau_b = tau.cpu().tolist()
+        return tau_a, tau_b
 
 
 def spearman_pvalue(rho, n):

@@ -27,6 +27,8 @@ RESULT_COLUMNS = ("checkpoint", "run", "epoch", "behavioral_rsa_rho", "behaviora
 # written only when asked for (n_perm > 0 / n_boot > 0): Mantel p-value, stimulus-bootstrap 95 % interval of rho
 PERMUTATION_COLUMNS = ("behavioral_rsa_p_perm",)
 BOOTSTRAP_COLUMNS = ("behavioral_rsa_ci_low", "behavioral_rsa_ci_high", "behavioral_rsa_boot_valid")
+# written only with kendall=True: Kendall's tau-a and tau-b of the model RDM against the reference (RSAEvaluator.kendall_tau)
+KENDALL_COLUMNS = ("behavioral_rsa_tau_a", "behavioral_rsa_tau_b")
 _EPOCH = re.compile(r"epoch(\d+)_dora_params\.pth$")
 
 
@@ -67,14 +69,15 @@ def embeddings(model, loaders, device):
 
 
 def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank=0, world_size=1, output_csv=None,
-                              log=print, root=None, evaluator=None, embed_fn=None, n_perm=0, n_boot=0, seed=0):
+                              log=print, root=None, evaluator=None, embed_fn=None, n_perm=0, n_boot=0, seed=0,
+                              kendall=False):
     """-> (rows, per-rank stats) on rank 0 | None.  `model`: CLIPHBA with its adapters applied (weights of the
     checkpoints are loaded with strict=False exactly as NEW:1159 does); `loaders`: ResidentLoaders whose concatenation
     is the image set in the order of `reference_rdm`'s rows.  `evaluator` / `embed_fn` default to the libhba ones
     (hba.rsa.RSAEvaluator, `embeddings`); the world-2 `gloo` test of the sharding passes CPU stand-ins.
     n_perm > 0 adds PERMUTATION_COLUMNS (RSAEvaluator.permutation_test), n_boot > 0 adds BOOTSTRAP_COLUMNS
     (RSAEvaluator.bootstrap, 95 % percentile interval); `seed` seeds both, so every checkpoint sees the same
-    permutations and resamples."""
+    permutations and resamples.  kendall=True adds KENDALL_COLUMNS (RSAEvaluator.kendall_tau)."""
     if evaluator is None:
         from .rsa import RSAEvaluator
         evaluator = RSAEvaluator(reference_rdm, device)
@@ -103,6 +106,9 @@ def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank
         if n_boot > 0:
             (lo, hi), _, valid = evaluator.bootstrap(emb, n_boot=n_boot, seed=seed)
             rows[-1].update(behavioral_rsa_ci_low=lo, behavioral_rsa_ci_high=hi, behavioral_rsa_boot_valid=valid)
+        if kendall:
+            tau_a, tau_b = evaluator.kendall_tau(emb)
+            rows[-1].update(behavioral_rsa_tau_a=tau_a, behavioral_rsa_tau_b=tau_b)
         if log is not None:
             log(f"[rank {rank}] {rel}: rho {rho:.6f}")
     stats = {"rank": rank, "checkpoints": len(rows), "embed_s": t_emb, "rsa_tail_s": t_rsa}
@@ -121,6 +127,6 @@ def clip_rsa_over_checkpoints(model, loaders, reference_rdm, files, device, rank
         import pandas as pd
         os.makedirs(os.path.dirname(os.path.abspath(output_csv)), exist_ok=True)
         columns = (list(RESULT_COLUMNS) + (list(PERMUTATION_COLUMNS) if n_perm > 0 else [])
-                   + (list(BOOTSTRAP_COLUMNS) if n_boot > 0 else []))
+                   + (list(BOOTSTRAP_COLUMNS) if n_boot > 0 else []) + (list(KENDALL_COLUMNS) if kendall else []))
         pd.DataFrame(rows, columns=columns).to_csv(output_csv, index=False)
     return rows, stats
