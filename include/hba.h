@@ -120,12 +120,15 @@ int hba_split_bf16(const float* in, int64_t rows, int64_t cols, int64_t ld_in, v
  * LayerNorm (un-vendored CLIP ln_1/ln_2/ln_pre/ln_post/ln_final, eps 1e-5; timm eps 1e-6)
  * x [rows, ldx] fp32 -> y_f32 (optional) and y_bf16 hi/lo (optional), biased variance, fp32.
  * row_stride_sel: processes rows r*row_step (row_step > 1 selects e.g. the CLS row of each image)
+ * cols: a multiple of 128, <= 1024.  x, gamma, beta, y_f32 (float4 accesses) 16-byte aligned, y_bf16 8-byte
+ * aligned; ldx, ld_yf, ld_yb, lo_off multiples of 4.  HBA_ERR_ARG otherwise.
  */
 int hba_layernorm_fwd(const float* x, int64_t rows, int32_t cols, int64_t ldx, int64_t row_step,
                       const float* gamma, const float* beta, float eps, float* y_f32,
                       int64_t ld_yf, void* y_bf16, int64_t ld_yb, int64_t lo_off, void* stream);
 /* dx[r,:] (+)= LN backward of dy through (x, gamma); accumulate != 0 adds into dx.
- * dy, dx fp32 with leading dims ld_dy, ld_dx; x rows taken at r*row_step */
+ * dy, dx fp32 with leading dims ld_dy, ld_dx; x rows taken at r*row_step (dy, dx rows at r).
+ * cols as hba_layernorm_fwd; dy, x, gamma, dx 16-byte aligned, ld_dy, ldx, ld_dx multiples of 4. */
 int hba_layernorm_bwd(const float* dy, int64_t ld_dy, const float* x, int64_t rows, int32_t cols,
                       int64_t ldx, int64_t row_step, const float* gamma, float eps, float* dx,
                       int64_t ld_dx, int accumulate, void* stream);
@@ -134,16 +137,19 @@ int hba_layernorm_bwd(const float* dy, int64_t ld_dy, const float* x, int64_t ro
  * Patch embedding front end of the vision tower (un-vendored visual.conv1 + class/positional
  * embedding + ln_pre, reached via NEW:298).
  * im2col: image [B,3,H,W] fp32 NCHW -> patches [B*gh*gw, ld_out] bf16 hi/lo, column index
- *         = c*P*P + py*P + px (conv weight [width, 3, P, P] flattened), zero padded to ld.
+ *         = c*P*P + py*P + px (conv weight [width, 3, P, P] flattened); the hi part zero padded up to lo_off
+ *         (ld_out without lo part), the lo part up to ld_out; both need 3*P*P columns.
  * assemble: x[b,0,:] = cls + pos[0]; x[b,1+p,:] = conv[b*np+p,:] + pos[1+p]; then ln_pre
  *           (gamma == NULL: no LayerNorm, the timm ViT-B/16 layout of VIT:283).
+ *           width a multiple of 128, <= 1024; conv, cls, pos, gamma, beta, x_out 16-byte aligned.
  */
 int hba_im2col_patches(const float* image, int32_t B, int32_t H, int32_t W, int32_t P, void* out,
                        int64_t ld_out, int64_t lo_off, void* stream);
 int hba_assemble_tokens_ln(const float* conv, int32_t B, int32_t n_patches, int32_t width,
                            const float* cls, const float* pos, const float* gamma,
                            const float* beta, float eps, float* x_out, void* stream);
-/* text front end: x[s, t, :] = token_embedding[tokens[s,t]] + pos[t]  (fp32) */
+/* text front end: x[s, t, :] = token_embedding[tokens[s,t]] + pos[t]  (fp32); width % 4 == 0,
+ * table, pos, x_out 16-byte aligned */
 int hba_embed_tokens(const int64_t* tokens, int32_t S, int32_t T, int32_t width,
                      const float* table, const float* pos, float* x_out, void* stream);
 /* gather rows: out[i,:] = in[idx[i],:] (fp32), used for the EOT rows (text.argmax(-1)) */
@@ -339,9 +345,10 @@ int hba_softmax_ce_fwd_bwd(const float* logits, int64_t ld, const int64_t* label
 /* ------------------------------------------------------------------------------------------
  * Extra kernels of the fully-trained ViT-B/16 data-parallel baseline (VIT:125-165: every parameter
  * receives a gradient).
- * hba_colsum: out[c] (+)= sum_r x[r, c]  (bias gradients of every Linear / the conv);
- *   workspace >= 128 * cols floats.
- * hba_layernorm_param_grad: dgamma_dbeta[0:cols] (+)= sum_r dy * xhat, [cols:2cols] (+)= sum_r dy;
+ * hba_colsum: out[c] (+)= sum_r x[r, c]  (bias gradients of every Linear / the conv); dtype HBA_DT_F32 or
+ *   HBA_DT_BF16; workspace >= 128 * cols floats.
+ * hba_layernorm_param_grad: dgamma_dbeta[0:cols] (+)= sum_r dy * xhat, [cols:2cols] (+)= sum_r dy, x rows taken
+ *   at r*row_step; cols % 4 == 0, x 16-byte aligned and ldx % 4 == 0 (x is read as float4);
  *   workspace >= 2*rows + 256*cols floats.
  * hba_attention_bwd: full softmax-attention backward, d_out [B*T, H*64] -> d_qkv [B*T, 3*H*64]
  *   (dtypes HBA_DT_*: (bf16, bf16|f32, bf16) or (f32, f32, f32); with bf16 qkv an f32 d_out is rounded to
@@ -356,7 +363,8 @@ int hba_layernorm_param_grad(const float* dy, int64_t ld_dy, const float* x, int
 /* Fused LayerNorm backward of the trained ViT: dx (+)= LN'(dy), optional bf16 hi[/lo] copy of the
  * resulting dx (operand of the next GEMMs), dgamma_dbeta [2*cols] (+)=, and dx_colsum [cols] = column
  * sums of the resulting dx (bias gradient of the Linear feeding this residual stream); one pass over
- * HBM.  cols in {128, 256, 512, 768, 1024}; workspace >= 2 * #SM * 3 * cols floats. */
+ * HBM.  cols in {128, 256, 512, 768, 1024}; workspace >= 2 * #SM * 3 * cols floats; dy, x, gamma, dx 16-byte
+ * aligned, dx_bf16 8-byte aligned, ld_dy, ldx, ld_dx, ld_b, lo_off multiples of 4. */
 int hba_layernorm_bwd_fused(const float* dy, int64_t ld_dy, const float* x, int64_t rows,
                             int32_t cols, int64_t ldx, const float* gamma, float eps, float* dx,
                             int64_t ld_dx, int32_t accumulate, void* dx_bf16, int64_t ld_b,

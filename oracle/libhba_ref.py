@@ -250,6 +250,7 @@ class RefLib:
         _require(cols % 128 == 0 and cols <= 1024, f"cols={cols} must be a multiple of 128 and <= 1024")
         _require(ldx % 4 == 0 and ld_yf % 4 == 0 and ld_yb % 4 == 0 and lo_off % 4 == 0 and _al(y_bf16, 8),
                  "leading dimensions must keep 16-byte (fp32) / 8-byte (bf16) row alignment")
+        _require(_al(x) and _al(gamma) and _al(beta) and _al(y_f32), "x, gamma, beta and y_f32 must be 16-byte aligned")
         row_step = max(1, row_step)
         xv = self._rows(x, rows, cols, ldx, row_step)
         mu = xv.mean(1, keepdim=True)
@@ -265,6 +266,7 @@ class RefLib:
         _require(_addr(dy) and _addr(x) and _addr(gamma) and _addr(dx) and rows > 0, "bad arguments")
         _require(cols % 128 == 0 and cols <= 1024, f"cols={cols} must be a multiple of 128 and <= 1024")
         _require(ldx % 4 == 0 and ld_dy % 4 == 0 and ld_dx % 4 == 0, "leading dimensions must be multiples of 4")
+        _require(_al(dy) and _al(x) and _al(gamma) and _al(dx), "dy, x, gamma and dx must be 16-byte aligned")
         row_step = max(1, row_step)
         xv = self._rows(x, rows, cols, ldx, row_step)
         g = mat(dy, rows, cols, ld_dy, torch.float32) * flat(gamma, cols, torch.float32)
@@ -279,17 +281,27 @@ class RefLib:
     # ---------------------------------------------------------------- front ends of the towers
     def hba_im2col_patches(self, image, B, H, W, P, out, ld_out, lo_off, stream):
         _require(_addr(image) and _addr(out) and B > 0 and P > 0 and H % P == 0 and W % P == 0, "bad arguments")
-        _require((ld_out if lo_off == 0 else lo_off) >= 3 * P * P, "row too short for 3*P*P columns")
+        _require((ld_out if lo_off == 0 else lo_off) >= 3 * P * P and (lo_off == 0 or ld_out - lo_off >= 3 * P * P),
+                 "row too short for 3*P*P columns")
         img = flat(image, B * 3 * H * W, torch.float32).view(B, 3, H, W)
         gh, gw = H // P, W // P
         cols = img.view(B, 3, gh, P, gw, P).permute(0, 2, 4, 1, 3, 5).reshape(B * gh * gw, 3 * P * P)
-        write_operand(out, cols.contiguous(), ld_out, lo_off)      # (the pad columns stay as allocated: zero)
+        # zeros up to lo_off in the hi part (up to ld_out without a lo part) and up to ld_out in the lo part
+        padded = torch.zeros(B * gh * gw, lo_off if lo_off > 0 else ld_out)
+        padded[:, :3 * P * P] = cols
+        write_operand(out, padded, ld_out, 0)
+        if lo_off > 0:
+            lo = torch.zeros(B * gh * gw, ld_out - lo_off)
+            lo[:, :3 * P * P] = cols - cols.to(torch.bfloat16).float()
+            write_operand(_addr(out) + 2 * lo_off, lo, ld_out, 0)
         return self._ok("hba_im2col_patches")
 
     def hba_assemble_tokens_ln(self, conv, B, n_patches, width, cls, pos, gamma, beta, eps, x_out, stream):
         _require(_addr(conv) and _addr(cls) and _addr(pos) and _addr(x_out) and B > 0 and (not _addr(gamma)) == (not _addr(beta)),
                  "bad arguments")
         _require(width % 128 == 0 and width <= 1024, f"width={width} unsupported")
+        _require(all(_al(p) for p in (conv, cls, pos, gamma, beta, x_out)),
+                 "conv, cls, pos, gamma, beta and x_out must be 16-byte aligned")
         c = flat(conv, B * n_patches * width, torch.float32).view(B, n_patches, width)
         ps = flat(pos, (n_patches + 1) * width, torch.float32).view(n_patches + 1, width)
         x = torch.cat([flat(cls, width, torch.float32).expand(B, 1, width), c], 1) + ps
@@ -302,6 +314,7 @@ class RefLib:
     def hba_embed_tokens(self, tokens, S, T, width, table, pos, x_out, stream):
         _require(_addr(tokens) and _addr(table) and _addr(pos) and _addr(x_out) and S > 0 and T > 0 and width % 4 == 0,
                  "bad arguments")
+        _require(_al(table) and _al(pos) and _al(x_out), "table, pos and x_out must be 16-byte aligned")
         tok = flat(tokens, S * T, torch.int64).view(S, T)
         n_vocab = int(tok.max()) + 1
         tab = flat(table, n_vocab * width, torch.float32).view(n_vocab, width)
@@ -573,6 +586,8 @@ class RefLib:
         return self._ok("hba_softmax_ce_fwd_bwd")
 
     def hba_colsum(self, x, dtype, rows, cols, ld, out, accumulate, workspace, stream):
+        _require(_addr(x) and _addr(out) and _addr(workspace) and rows > 0 and cols > 0, "bad arguments")
+        _require(dtype in DT, f"unknown dtype {dtype}")
         s_ = mat(x, rows, cols, ld, DT[dtype]).float().sum(0)
         o = flat(out, cols, torch.float32)
         o.copy_(o + s_ if accumulate else s_)
@@ -586,7 +601,10 @@ class RefLib:
 
     def hba_layernorm_param_grad(self, dy, ld_dy, x, rows, cols, ldx, row_step, eps, dgamma_dbeta, accumulate,
                                  workspace, stream):
-        xhat, _ = self._ln_stats(x, rows, cols, ldx, row_step, eps)
+        _require(_addr(dy) and _addr(x) and _addr(dgamma_dbeta) and _addr(workspace) and rows > 0 and cols > 0
+                 and cols % 4 == 0, "bad arguments")
+        _require(ldx % 4 == 0 and _al(x), "x must be 16-byte aligned and ldx a multiple of 4")
+        xhat, _ = self._ln_stats(x, rows, cols, ldx, max(1, row_step), eps)
         g = mat(dy, rows, cols, ld_dy, torch.float32)
         new = torch.cat([(g * xhat).sum(0), g.sum(0)])
         o = flat(dgamma_dbeta, 2 * cols, torch.float32)
@@ -595,6 +613,13 @@ class RefLib:
 
     def hba_layernorm_bwd_fused(self, dy, ld_dy, x, rows, cols, ldx, gamma, eps, dx, ld_dx, accumulate, dx_bf16, ld_b,
                                 lo_off, dgamma_dbeta, accumulate_params, dx_colsum, workspace, stream):
+        _require(_addr(dy) and _addr(x) and _addr(gamma) and _addr(dx) and _addr(dgamma_dbeta) and _addr(workspace)
+                 and rows > 0, "bad arguments")
+        _require(ldx % 4 == 0 and ld_dy % 4 == 0 and ld_dx % 4 == 0 and ld_b % 4 == 0 and lo_off % 4 == 0,
+                 "leading dimensions must be multiples of 4")
+        _require(_al(dy) and _al(x) and _al(gamma) and _al(dx) and _al(dx_bf16, 8),
+                 "dy, x, gamma and dx must be 16-byte aligned, dx_bf16 8-byte aligned")
+        _require(cols in (128, 256, 512, 768, 1024), f"cols={cols} (supported: 128, 256, 512, 768, 1024)")
         xhat, rstd = self._ln_stats(x, rows, cols, ldx, 1, eps)
         g0 = mat(dy, rows, cols, ld_dy, torch.float32)
         g = g0 * flat(gamma, cols, torch.float32)
@@ -603,10 +628,9 @@ class RefLib:
         out.copy_(out + d if accumulate else d)
         if _addr(dx_bf16):
             write_operand(dx_bf16, out.clone(), ld_b, lo_off)
-        if _addr(dgamma_dbeta):
-            new = torch.cat([(g0 * xhat).sum(0), g0.sum(0)])
-            o = flat(dgamma_dbeta, 2 * cols, torch.float32)
-            o.copy_(o + new if accumulate_params else new)
+        new = torch.cat([(g0 * xhat).sum(0), g0.sum(0)])
+        o = flat(dgamma_dbeta, 2 * cols, torch.float32)
+        o.copy_(o + new if accumulate_params else new)
         if _addr(dx_colsum):
             flat(dx_colsum, cols, torch.float32).copy_(out.sum(0))
         return self._ok("hba_layernorm_bwd_fused")

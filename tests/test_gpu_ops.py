@@ -233,37 +233,6 @@ def test_layernorm_fwd_bwd(cols, split):
     assert rel_err(ysel, y.detach()[::5][: rows // 5]) < 1e-5
 
 
-@pytest.mark.parametrize("rows,cols", [(8224, 1024), (5082, 768), (1024, 128), (1031, 256), (3000, 1024)])
-@pytest.mark.parametrize("split", [False, True])
-def test_layernorm_fwd_streaming_form(rows, cols, split):
-    """>= 1024 rows take the persistent bulk-copy-staged kernel (layernorm_fwd_stream_kernel): same arithmetic as
-    the warp-per-row kernel, checked against torch and - bit for bit - against the warp-per-row kernel run on the
-    same rows in two halves of < 1024 rows... (which the launcher routes to the per-row kernel)."""
-    hba, ops, ref = _imports()
-    g = torch.Generator().manual_seed(rows + cols)
-    x = (torch.randn(rows, cols, generator=g) * 3 - 0.7)
-    x[5, 7] = 250.0                                   # an outlier feature, as the CLIP residual stream has
-    w, b = torch.randn(cols, generator=g), torch.randn(cols, generator=g)
-    want = torch.nn.functional.layer_norm(x, (cols,), w, b, 1e-5)
-    xd, wd, bd = x.to(DEV), w.to(DEV), b.to(DEV)
-    yf = torch.full((rows, cols), float("nan"), device=DEV)
-    yo = ops.Operand.empty(rows, cols, split, DEV)
-    ops.layernorm_fwd(xd, rows, cols, wd, bd, 1e-5, y_f32=yf, y=yo)
-    assert rel_err(yf, want) < 1e-5
-    assert rel_err(operand_value(yo), want) < (2e-5 if split else 5e-3)
-    # the per-row kernel on chunks of 1000 rows: identical bits
-    yc = torch.empty(rows, cols, device=DEV)
-    for r0 in range(0, rows, 1000):
-        n = min(1000, rows - r0)
-        ops.layernorm_fwd(xd[r0:], n, cols, wd, bd, 1e-5, y_f32=yc[r0:])
-    assert torch.equal(yc, yf)
-    # bf16-only output with a strided source (every 2nd row), as the engine never uses but the ABI allows
-    if rows >= 2048:
-        ys = torch.empty(rows // 2, cols, device=DEV)
-        ops.layernorm_fwd(xd, rows // 2, cols, wd, bd, 1e-5, row_step=2, y_f32=ys)
-        assert torch.equal(ys, yf[::2][: rows // 2])
-
-
 @pytest.mark.parametrize("split", [False, True])
 def test_patch_embed_front_end(split):
     hba, ops, ref = _imports()

@@ -51,6 +51,9 @@ int make_tma_2d_bf16(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t 
 int make_tma_3d_bf16(CUtensorMap* map, const void* ptr, uint64_t batch, uint64_t rows, uint64_t cols,
                      uint64_t ld, uint32_t box_rows, uint32_t box_cols);
 
+// pointers a kernel loads / stores as float4 (NULL counts as aligned: optional arguments are checked for presence apart)
+inline bool aligned16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+
 #define HBA_CHECK(expr)                  \
   do {                                   \
     int _rc = (expr);                    \

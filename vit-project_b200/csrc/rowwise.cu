@@ -299,7 +299,9 @@ __global__ void im2col_kernel(const float* __restrict__ image, int B, int H, int
   const int b = patch / (gh * gw), pr = (patch / gw) % gh, pc = patch % gw;
   const int kk = 3 * P * P;
   __nv_bfloat16* o = out + patch * ld_out;
-  for (int k = lane; k < ld_out && (lo_off == 0 || k < lo_off); k += 32) {
+  // hi part: columns [0, hi_end); lo part: columns lo_off + [0, lo_end) - both zero past 3*P*P, neither past ld_out
+  const int64_t hi_end = lo_off > 0 ? lo_off : ld_out, lo_end = lo_off > 0 ? ld_out - lo_off : 0;
+  for (int64_t k = lane; k < hi_end || k < lo_end; k += 32) {
     float v = 0.f;
     if (k < kk) {
       const int c = k / (P * P), py = (k / P) % P, px = k % P;
@@ -307,8 +309,8 @@ __global__ void im2col_kernel(const float* __restrict__ image, int B, int H, int
     }
     __nv_bfloat16 h, l;
     split_bf16(v, h, l);
-    o[k] = h;
-    if (lo_off > 0) o[lo_off + k] = l;
+    if (k < hi_end) o[k] = h;
+    if (k < lo_end) o[lo_off + k] = l;
   }
 }
 
@@ -453,9 +455,11 @@ extern "C" int hba_layernorm_fwd(const float* x, int64_t rows, int32_t cols, int
   HBA_REQUIRE(x && gamma && beta && (y_f32 || y_bf16) && rows > 0, "hba_layernorm_fwd: bad arguments");
   HBA_REQUIRE(cols % 128 == 0 && cols <= 128 * kLnMaxVec, "hba_layernorm_fwd: cols=%d must be a multiple of 128 and <= %d", cols, 128 * kLnMaxVec);
   HBA_REQUIRE(ldx % 4 == 0 && ld_yf % 4 == 0 && ld_yb % 4 == 0 && lo_off % 4 == 0 && ((uintptr_t)y_bf16 & 7) == 0, "hba_layernorm_fwd: leading dimensions must keep 16-byte (fp32) / 8-byte (bf16) alignment");
+  HBA_REQUIRE(aligned16(x) && aligned16(gamma) && aligned16(beta) && aligned16(y_f32),
+              "hba_layernorm_fwd: x, gamma, beta and y_f32 are read / written as float4 and must be 16-byte aligned");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (row_step < 1) row_step = 1;
-  if (rows >= 1024 && ((uintptr_t)x & 15) == 0) {
+  if (rows >= 1024) {
     // streaming form: persistent CTAs, rows staged through shared memory by bulk asynchronous copies
     int stages = (int)((220 * 1024 - 2 * cols * 4 - 256) / ((size_t)kLnsRows * cols * 4));
     if (stages > kLnsMaxStages) stages = kLnsMaxStages;
@@ -481,6 +485,8 @@ extern "C" int hba_layernorm_bwd(const float* dy, int64_t ld_dy, const float* x,
   HBA_REQUIRE(dy && x && gamma && dx && rows > 0, "hba_layernorm_bwd: bad arguments");
   HBA_REQUIRE(cols % 128 == 0 && cols <= 128 * kLnMaxVec, "hba_layernorm_bwd: cols=%d must be a multiple of 128 and <= %d", cols, 128 * kLnMaxVec);
   HBA_REQUIRE(ldx % 4 == 0 && ld_dy % 4 == 0 && ld_dx % 4 == 0, "hba_layernorm_bwd: leading dimensions must be multiples of 4");
+  HBA_REQUIRE(aligned16(dy) && aligned16(x) && aligned16(gamma) && aligned16(dx),
+              "hba_layernorm_bwd: dy, x, gamma and dx are accessed as float4 and must be 16-byte aligned");
   layernorm_bwd_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       dy, ld_dy, x, rows, cols, ldx, row_step < 1 ? 1 : row_step, gamma, eps, dx, ld_dx, accumulate);
   return check_launch("hba_layernorm_bwd");
@@ -489,7 +495,8 @@ extern "C" int hba_layernorm_bwd(const float* dy, int64_t ld_dy, const float* x,
 extern "C" int hba_im2col_patches(const float* image, int32_t B, int32_t H, int32_t W, int32_t P,
                                   void* out, int64_t ld_out, int64_t lo_off, void* stream) {
   HBA_REQUIRE(image && out && B > 0 && P > 0 && H % P == 0 && W % P == 0, "hba_im2col_patches: bad arguments");
-  HBA_REQUIRE((lo_off == 0 ? ld_out : lo_off) >= 3 * P * P, "hba_im2col_patches: row too short for 3*P*P columns");
+  HBA_REQUIRE((lo_off == 0 ? ld_out : lo_off) >= 3 * P * P && (lo_off == 0 || ld_out - lo_off >= 3 * P * P),
+              "hba_im2col_patches: row too short for 3*P*P columns");
   const int64_t patches = (int64_t)B * (H / P) * (W / P);
   im2col_kernel<<<(unsigned)((patches + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       image, B, H, W, P, static_cast<__nv_bfloat16*>(out), ld_out, lo_off);
@@ -502,6 +509,8 @@ extern "C" int hba_assemble_tokens_ln(const float* conv, int32_t B, int32_t n_pa
                                       float* x_out, void* stream) {
   HBA_REQUIRE(conv && cls && pos && x_out && B > 0 && (!gamma == !beta), "hba_assemble_tokens_ln: bad arguments");
   HBA_REQUIRE(width % 128 == 0 && width <= 128 * kLnMaxVec, "hba_assemble_tokens_ln: width=%d unsupported", width);
+  HBA_REQUIRE(aligned16(conv) && aligned16(cls) && aligned16(pos) && aligned16(gamma) && aligned16(beta) && aligned16(x_out),
+              "hba_assemble_tokens_ln: conv, cls, pos, gamma, beta and x_out are accessed as float4 and must be 16-byte aligned");
   const int64_t rows = (int64_t)B * (n_patches + 1);
   assemble_tokens_ln_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       conv, B, n_patches, width, cls, pos, gamma, beta, eps, x_out);
@@ -511,6 +520,8 @@ extern "C" int hba_assemble_tokens_ln(const float* conv, int32_t B, int32_t n_pa
 extern "C" int hba_embed_tokens(const int64_t* tokens, int32_t S, int32_t T, int32_t width,
                                 const float* table, const float* pos, float* x_out, void* stream) {
   HBA_REQUIRE(tokens && table && pos && x_out && S > 0 && T > 0 && width % 4 == 0, "hba_embed_tokens: bad arguments");
+  HBA_REQUIRE(aligned16(table) && aligned16(pos) && aligned16(x_out),
+              "hba_embed_tokens: table, pos and x_out are accessed as float4 and must be 16-byte aligned");
   const int64_t rows = (int64_t)S * T;
   embed_tokens_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       tokens, S, T, width, table, pos, x_out);

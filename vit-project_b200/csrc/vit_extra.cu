@@ -440,6 +440,8 @@ extern "C" int hba_layernorm_param_grad(const float* dy, int64_t ld_dy, const fl
                                         void* stream) {
   HBA_REQUIRE(dy && x && dgamma_dbeta && workspace && rows > 0 && cols > 0 && cols % 4 == 0,
               "hba_layernorm_param_grad: bad arguments");
+  HBA_REQUIRE(ldx % 4 == 0 && aligned16(x),
+              "hba_layernorm_param_grad: x rows are read as float4: x must be 16-byte aligned and ldx a multiple of 4");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   float* stats = workspace;                 // [rows, 2]
   float* partial = workspace + 2 * rows;    // [chunks, 2*cols]
@@ -478,6 +480,8 @@ extern "C" int hba_layernorm_bwd_fused(const float* dy, int64_t ld_dy, const flo
   HBA_REQUIRE(dy && x && gamma && dx && dgamma_dbeta && workspace && rows > 0, "hba_layernorm_bwd_fused: bad arguments");
   HBA_REQUIRE(ldx % 4 == 0 && ld_dy % 4 == 0 && ld_dx % 4 == 0 && ld_b % 4 == 0 && lo_off % 4 == 0,
               "hba_layernorm_bwd_fused: leading dimensions must be multiples of 4");
+  HBA_REQUIRE(aligned16(dy) && aligned16(x) && aligned16(gamma) && aligned16(dx) && ((uintptr_t)dx_bf16 & 7) == 0,
+              "hba_layernorm_bwd_fused: dy, x, gamma and dx must be 16-byte aligned (float4), dx_bf16 8-byte aligned");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   int blocks = 2 * num_sms();
   if ((int64_t)blocks * 8 > rows) blocks = (int)((rows + 7) / 8);
